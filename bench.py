@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the pterotactyl reconstruction hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): Chamfer pairs/s at 10k x 10k points.  One "step" = Chamfer forward + backward
 (both directions, mean reduction, gradients w.r.t. both clouds) over a batch of 256 cloud pairs per GPU
@@ -18,6 +18,11 @@ One JSON line on stdout (rank 0).  Besides the base contract it carries
 
 `--impl reference` times the reference arm: the CPU restatement of the reference's PyTorch3D path
 (oracle port; PyTorch3D itself is not vendored/installable here) on all host threads, bounded sample.
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32: the per-pair
+Chamfer values and, at a fixed sample of (pair, point) positions, both nearest-neighbour index arrays and both gradient
+clouds.  The inputs depend only on the arguments, so two builds can be compared output for output: the Chamfer values
+and indices exactly, the gradients to a few ulps (the backward scatters them with float atomics, as PyTorch3D's does).
 """
 import argparse
 import json
@@ -31,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it
 # NCCL_DEBUG is left as the launcher set it: whatever NCCL prints goes to stderr (run_ours dup2()s fd 1 onto fd 2
 # while the job runs), stdout carries exactly one JSON line.
 
@@ -38,17 +44,40 @@ P = 10000           # points per cloud
 B_PER_GPU = 256     # cloud pairs per GPU per step
 NSETS = 4           # rotating input sets: 4 x 61 MB = 246 MB > 126 MB L2
 FLOP_PER_EVAL = 8   # algorithmic: 3 sub + 3 mul + 2 add per (query, target) distance (SURVEY.md 8d)
+DUMP_SAMPLE = 1 << 20  # (pair, point) positions of the per-point outputs --dump-outputs keeps: 34 MB of 82 MB
 
 
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (float32)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs:
+        if a.impl != "ours":
+            ap.error("--dump-outputs applies to the GPU path (--impl ours)")
+        os.makedirs(a.dump_outputs, exist_ok=True)  # an unusable DIR fails here, before any GPU work
+    return a
+
+
+def dump_outputs(torch, d, cham, idx_x, idx_y, grad_x, grad_y):
+    """What one Chamfer fwd+bwd step hands its caller, as float32 .npy files in `d`: the (B,) Chamfer values in full;
+    the (B, P) indices and (B, P, 3) gradients at DUMP_SAMPLE (pair, point) positions drawn once with seed 0, in
+    ascending flat order, the same for every run (indices < 2^24 are exact in float32)."""
+    n = idx_x.numel()
+    pos = np.sort(np.random.default_rng(0).choice(n, size=min(DUMP_SAMPLE, n), replace=False))
+    sel = torch.from_numpy(pos).to(idx_x.device)
+    out = {"cham": cham, "idx_x": idx_x.reshape(-1)[sel], "idx_y": idx_y.reshape(-1)[sel],
+           "grad_x": grad_x.reshape(-1, 3)[sel], "grad_y": grad_y.reshape(-1, 3)[sel]}
+    for name, t in out.items():
+        np.save(os.path.join(d, name + ".npy"), t.float().cpu().numpy())
 
 
 # --------------------------------------------------------------------------------- clocks sampler
@@ -333,6 +362,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         total_ms = float(t.item())
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:  # before the pruned-scan leg below reuses these buffers
+        dump_outputs(torch, args.dump_outputs, cham, idx_x, idx_y, gx, gy)
     pairs_per_s = world * B * K / (total_ms * 1e-3)
     rescued = C.c_int64(0)  # queries of the last timed forward that the filter handed to the exact rescue scan
     _lib.check(L.ptk_chamfer_rescued(p(ws), B, P, P, C.byref(rescued), sp), "ptk_chamfer_rescued")

@@ -92,18 +92,22 @@ def test_shard_bounds_cover_everything():
 def test_install_patches_reference_module():
     fake = types.SimpleNamespace()
     fake_model = types.SimpleNamespace(GCN=None, GCN_layer=None)
-    ptk_b200.install(fake, [fake_model])
-    assert fake.chamfer_distance is ptk_b200.utils.chamfer_distance
-    assert fake.batch_sample is ptk_b200.utils.batch_sample
-    assert fake_model.GCN is ptk_b200.GCN and fake_model.GCN_layer is ptk_b200.GCN_layer
-    assert not hasattr(fake_model, "Encoder") and not hasattr(fake_model, "Graph_Model")
-    # the autoencoder / DDQN modules: their GCN consumers and the Positional_Encoder copies are replaced too
-    ae = types.SimpleNamespace(GCN_layer=None, Encoder=None, AutoEncoder=None, Positional_Encoder=None)
-    ddqn = types.SimpleNamespace(GCN_layer=None, Graph_Model=None, Positional_Encoder=None, Encoder=None)
-    ptk_b200.install(fake, [ae, ddqn])
-    assert ae.Encoder is ptk_b200.model.Encoder and ae.Positional_Encoder is ptk_b200.Positional_Encoder
-    assert ddqn.Graph_Model is ptk_b200.model.Graph_Model and ddqn.GCN_layer is ptk_b200.GCN_layer
-    assert ddqn.Encoder is None  # an unrelated class called Encoder (no AutoEncoder beside it) is left alone
+    try:
+        ptk_b200.install(fake, [fake_model])
+        assert fake.chamfer_distance is ptk_b200.utils.chamfer_distance
+        assert fake.batch_sample is ptk_b200.utils.batch_sample
+        assert fake_model.GCN is ptk_b200.GCN and fake_model.GCN_layer is ptk_b200.GCN_layer
+        assert not hasattr(fake_model, "Encoder") and not hasattr(fake_model, "Graph_Model")
+        # the autoencoder / DDQN modules: their GCN consumers and the Positional_Encoder copies are replaced too
+        ae = types.SimpleNamespace(GCN_layer=None, Encoder=None, AutoEncoder=None, Positional_Encoder=None)
+        ddqn = types.SimpleNamespace(GCN_layer=None, Graph_Model=None, Positional_Encoder=None, Encoder=None)
+        ptk_b200.install(fake, [ae, ddqn])
+        assert ae.Encoder is ptk_b200.model.Encoder and ae.Positional_Encoder is ptk_b200.Positional_Encoder
+        assert ddqn.Graph_Model is ptk_b200.model.Graph_Model and ddqn.GCN_layer is ptk_b200.GCN_layer
+        assert ddqn.Encoder is None  # an unrelated class called Encoder (no AutoEncoder beside it) is left alone
+    finally:
+        ptk_b200.uninstall()  # install() also switched ptk_b200.utils.face_draw; later tests expect the default
+    assert ptk_b200.utils.face_draw == "uniform"
 
 
 def test_encoder_mirrors_state_dict_layout():
