@@ -41,7 +41,9 @@ namespace ptk {
 
 // library configuration of the kernel template (tuned with tools/chamfer_tune.cu)
 constexpr int CH_THREADS = 128;
-constexpr int CH_CHUNK = 16;
+constexpr int CH_CHUNK = 16;   // exact scan; filter scan on clouds the recheck cannot read with vector loads
+constexpr int CH_CHUNK_F = 64; // filter scan: one bookkeeping step per 64 targets (DESIGN.md K1)
+constexpr int CH_WIDE_MIN_SPLIT = 2048;  // fewer targets per split: 16-target chunks (see launch_nn)
 constexpr int CH_MINB = 3;   // exact scan
 constexpr int CH_MINB_F = 4; // filter scan
 constexpr int CH_TT_F = 1024; // targets per TMA tile (double buffered: 2 x 4 x 4 KB)
@@ -258,10 +260,10 @@ __global__ void chamfer_bwd_scatter_kernel(const float *__restrict__ x, const fl
 struct NNPlan {
     int R;          // queries per thread
     int n_split;    // CTAs along the target range
-    int split_len;  // targets per split (multiple of CH_CHUNK)
+    int split_len;  // targets per split (multiple of the scan's chunk, so every split starts on a chunk boundary)
 };
 
-static NNPlan plan_nn(int64_t B, int64_t Pq_max, int64_t Pt_max, int ndir, int minb) {
+static NNPlan plan_nn(int64_t B, int64_t Pq_max, int64_t Pt_max, int ndir, int minb, int64_t chunk) {
     // With >= 4 waves of CTAs (minb resident per SM) from the query blocks alone, the target range is not split.
     // Otherwise prefer R = 8 queries per thread (fewest shared-memory loads per evaluation) and get the CTA count
     // from splitting the target range; fall back to fewer queries per thread for tiny clouds.
@@ -280,7 +282,7 @@ static NNPlan plan_nn(int64_t B, int64_t Pq_max, int64_t Pt_max, int ndir, int m
     // gives ns = sqrt(Pt * slots / (512 * base)); within ~3 % of the measured optimum for P = 4k..100k, B = 1..64.
     const double slots = (double)sm_count() * minb;
     int64_t ns = base >= want ? 1 : (int64_t)(sqrt((double)Pt_max * slots / (512.0 * (double)base)) + 0.5);
-    auto split_len = [&](int64_t n) { return ceil_div(ceil_div(Pt_max, n), (int64_t)CH_CHUNK) * CH_CHUNK; };
+    auto split_len = [&](int64_t n) { return ceil_div(ceil_div(Pt_max, n), chunk) * chunk; };
     if (getenv("PTK_CH_NSPLIT")) ns = atoi(getenv("PTK_CH_NSPLIT"));  // tuning tools only (read per call)
     if (ns < 1) ns = 1;
     if (ns > max_split) ns = max_split;
@@ -372,7 +374,7 @@ static int launch_nn_pruned(const float *x, const float *y, int64_t B, int64_t P
                    (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, keys_x,
                    keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
     PTK_CHECK_LAUNCH();
-    const NNPlan p = plan_nn(B, Pq, Pt, ndir, CH_MINB);
+    const NNPlan p = plan_nn(B, Pq, Pt, ndir, CH_MINB, CH_CHUNK);
     dim3 rgrid((unsigned)ceil_div(Pq, (int64_t)CH_THREADS * 8), (unsigned)p.n_split, (unsigned)(B * ndir));
     launch_pdl(chamfer_nn_exact2_kernel<8, CH_CHUNK, CH_THREADS, CH_MINB>, rgrid, dim3(CH_THREADS), 0, st, x, y, iP1, iP2,
                p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
@@ -398,7 +400,19 @@ static int launch_nn(const float *x, const float *y, int64_t B, int64_t P1, int6
     const int64_t Pq = dir_only == 0 ? P1 : (dir_only == 1 ? P2 : (P1 > P2 ? P1 : P2));
     const int64_t Pt = dir_only == 0 ? P2 : (dir_only == 1 ? P1 : (P1 > P2 ? P1 : P2));
     const bool filter = algo == PTK_CHAMFER_FILTER;
-    NNPlan p = plan_nn(B, Pq, Pt, ndir, filter ? CH_MINB_F : CH_MINB);
+    // The filter's exact recheck reads each query's recorded chunk with per-thread vector loads, which needs every cloud
+    // of the batch 16-byte aligned.  With 4-byte loads a 64-target recheck costs more than the wider chunks save
+    // (DESIGN.md K1), so such batches keep 16-target chunks.
+    // The recheck is paid once per query and split, so its share grows as the splits shrink: 64-target chunks also
+    // need splits of at least CH_WIDE_MIN_SPLIT targets (fitted on tools/chamfer_layout_bench.py and
+    // tools/chamfer_sweep.py: +5 % at 10k targets per split, -4 % at 900).
+    auto vec_ok = [&](const float *p, int64_t P) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0 && (B == 1 || P % 4 == 0); };
+    bool wide = filter && vec_ok(x, P1) && vec_ok(y, P2);
+    NNPlan p = plan_nn(B, Pq, Pt, ndir, filter ? CH_MINB_F : CH_MINB, wide ? CH_CHUNK_F : CH_CHUNK);
+    if (wide && p.split_len < CH_WIDE_MIN_SPLIT) {
+        wide = false;
+        p = plan_nn(B, Pq, Pt, ndir, CH_MINB_F, CH_CHUNK);
+    }
     u64 *keys_x = dir_only == 1 ? nullptr : w.keys_x;
     u64 *keys_y = dir_only == 0 ? nullptr : w.keys_y;
     if (p.n_split > 1 && !filter) {  // (the filter path initialises keys and flags in chamfer_prep_kernel)
@@ -417,14 +431,14 @@ static int launch_nn(const float *x, const float *y, int64_t B, int64_t P1, int6
         launch_pdl(chamfer_prep_kernel, dim3((unsigned)ceil_div(Pp, 256), (unsigned)(2 * B)), dim3(256), 0, st, x, y, iP1, iP2,
                    w.aux, w.soa_x, w.soa_y, keys_x, keys_y, w.flag_x, w.flag_y, p.n_split > 1 ? 1 : 0);
         PTK_CHECK_LAUNCH();
-#define PTK_FILTER(RR)                                                                                          \
-    launch_pdl(chamfer_nn_filter_tma_kernel<RR, CH_CHUNK, CH_THREADS, CH_MINB_F, CH_TT_F>, grid, dim3(CH_THREADS), 0, st, \
+#define PTK_FILTER(RR, CC)                                                                                      \
+    launch_pdl(chamfer_nn_filter_tma_kernel<RR, CC, CH_THREADS, CH_MINB_F, CH_TT_F>, grid, dim3(CH_THREADS), 0, st,      \
                x, y, iP1, iP2, p.split_len, p.n_split, w.aux, w.soa_x, w.soa_y, w.keys_x, w.keys_y, dir_only, w.rescue_x, \
                w.rescue_y, w.count, w.flag_x, w.flag_y)
         switch (p.R) {
-            case 8: PTK_FILTER(8); break;
-            case 4: PTK_FILTER(4); break;
-            default: PTK_FILTER(2); break;
+            case 8: if (wide) PTK_FILTER(8, CH_CHUNK_F); else PTK_FILTER(8, CH_CHUNK); break;
+            case 4: if (wide) PTK_FILTER(4, CH_CHUNK_F); else PTK_FILTER(4, CH_CHUNK); break;
+            default: if (wide) PTK_FILTER(2, CH_CHUNK_F); else PTK_FILTER(2, CH_CHUNK); break;
         }
 #undef PTK_FILTER
         PTK_CHECK_LAUNCH();

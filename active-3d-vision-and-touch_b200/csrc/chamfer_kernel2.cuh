@@ -12,8 +12,8 @@
 // can be:
 //   * clouds are translated to the centre c of their joint bounding box (shrinks R; the exact
 //     arithmetic keeps using the untranslated coordinates);
-//   * per query the scan keeps the smallest chunk minimum `best` (chunk = 16 consecutive targets),
-//     the chunk that produced it, and the smallest chunk minimum of any OTHER chunk, `second`;
+//   * per query the scan keeps the smallest chunk minimum `best` (chunk = CHUNK consecutive targets, 64 in
+//     the library's TMA scan), the chunk that produced it, and the smallest chunk minimum of any OTHER chunk, `second`;
 //   * afterwards the recorded chunk is re-evaluated with the exact arithmetic (first minimum wins);
 //   * if second > best + thr no target outside that chunk can beat or tie it (thr bounds every
 //     rounding error involved, see PairAux below), so the result is final.  Otherwise the
@@ -68,6 +68,9 @@ __device__ __forceinline__ u64 mul2(u64 a, u64 b) {
 //                                         <= 25.1 u M^2 + 26.1 u bd          (2 M sqrt(bd) <= M^2/4 + 4 bd).
 // The kernels use thr_q = 32 u M^2 + 32 u bd: the spare 7 u M^2 covers the rounding of `best + thr_q` itself
 // (|best| <= 4 M^2) and second-order terms.  aux.thr = 32 u M^2 = 2^-19 M^2, rounded up.
+// The chunk width does not enter: the claim compares single targets t and b*, e* is the exact arg-min of whatever
+// range is rechecked, and `second` is a minimum over single targets outside it.  A wider chunk only moves near-ties
+// inside the rechecked range, where the exact arithmetic settles them.
 // Non-finite input, M^2 > 1e30 or M^2 < 1e-30 (squares would overflow / lose relative accuracy to underflow)
 // set thr = +inf: every query then takes the exact path.
 struct PairAux {
@@ -471,15 +474,14 @@ chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restric
         const int chunk0 = tile / CHUNK;
         mbar_wait_parity((it & 1) ? bar1 : bar0, (uint32_t)((it >> 1) & 1));
         const float *sx = sbuf[it & 1][0], *sy = sbuf[it & 1][1], *sz = sbuf[it & 1][2], *st = sbuf[it & 1][3];
-        // 16-target bodies; the per-chunk bookkeeping runs after every CHUNK/16-th body (uniform branch)
-        float m[R];
+        // One fully unrolled body per chunk: the chunk minimum starts from the chunk's first values (no +inf operand,
+        // no reset), and the bookkeeping is straight-line code the scheduler can slot between the FFMA2s of the other
+        // queries.  Per query and 64 targets: 96 FFMA2, 31 FMNMX3 + 1 FMNMX for the minimum, 5 bookkeeping instructions.
+        for (int c = 0; c < nchunks; ++c) {
+            float m[R];
 #pragma unroll
-        for (int r = 0; r < R; ++r) m[r] = INF;
-        const int nbodies = nchunks * (CHUNK / 16);
-        for (int sb = 0; sb < nbodies; ++sb) {
-#pragma unroll
-            for (int g4 = 0; g4 < 4; ++g4) {
-                const int o = sb * 16 + g4 * 4;
+            for (int g4 = 0; g4 < CHUNK / 4; ++g4) {
+                const int o = c * CHUNK + g4 * 4;
                 const ulonglong2 tx = *reinterpret_cast<const ulonglong2 *>(&sx[o]);
                 const ulonglong2 ty = *reinterpret_cast<const ulonglong2 *>(&sy[o]);
                 const ulonglong2 tz = *reinterpret_cast<const ulonglong2 *>(&sz[o]);
@@ -496,25 +498,35 @@ chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restric
                     float a0, a1, a2, a3;
                     unpack2(a, a0, a1);
                     unpack2(c2, a2, a3);
-                    m[r] = min3f(m[r], a0, a1);
-                    m[r] = min3f(m[r], a2, a3);
+                    if (g4 == 0) {
+                        m[r] = fminf(min3f(a0, a1, a2), a3);
+                    } else {
+                        m[r] = min3f(m[r], a0, a1);
+                        m[r] = min3f(m[r], a2, a3);
+                    }
                 }
             }
-            if (CHUNK == 16 || (sb & (CHUNK / 16 - 1)) == CHUNK / 16 - 1) {
-                const int cid = chunk0 + sb / (CHUNK / 16);
+            const int cid = chunk0 + c;
 #pragma unroll
-                for (int r = 0; r < R; ++r) {
-                    sec[r] = fminf(sec[r], fmaxf(m[r], best[r]));
-                    bchunk[r] = m[r] < best[r] ? cid : bchunk[r];
-                    best[r] = fminf(best[r], m[r]);
-                    m[r] = INF;
-                }
+            for (int r = 0; r < R; ++r) {
+                sec[r] = fminf(sec[r], fmaxf(m[r], best[r]));
+                bchunk[r] = m[r] < best[r] ? cid : bchunk[r];
+                best[r] = fminf(best[r], m[r]);
             }
         }
         __syncthreads();  // every warp is done with this buffer
         if (tid == 0 && it + 2 < ntiles) issue(it + 2);
     }
 
+    // Exact recheck of the recorded chunk.  It needs the untranslated coordinates, so it reads the caller's AoS cloud,
+    // not the translated SoA copy.  Each thread reads its own chunk, so every load of a warp touches 32 different
+    // cache lines: with 4-byte loads the recheck of 64-target chunks cost more L1 bandwidth than the wider chunks
+    // saved.  Whole chunks are therefore read with 256-bit loads (3 per 8 targets) when the cloud is 32-byte aligned,
+    // with float4 loads (3 per 4 targets) when it is 16-byte aligned; a chunk then starts on such a boundary because
+    // CHUNK * 12 is a multiple of 32.
+    static_assert(CHUNK % 8 == 0, "vector recheck reads whole groups of 8 targets");
+    const bool t_aligned = (reinterpret_cast<uintptr_t>(T) & 15) == 0;
+    const bool t_aligned32 = (reinterpret_cast<uintptr_t>(T) & 31) == 0;
     int *__restrict__ rescue = dir == 0 ? rescue_x + (size_t)b * P1 : rescue_y + (size_t)b * P2;
     unsigned int *__restrict__ rflag = dir == 0 ? rescue_flag_x + (size_t)b * P1 : rescue_flag_y + (size_t)b * P2;
 #pragma unroll
@@ -526,12 +538,39 @@ chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restric
         const int j1 = min(j0 + CHUNK, t_end);
         float bd = INF;
         int arg = j0;
-        for (int j = j0; j < j1; ++j) {
-            const float d = sqdist(qx, qy, qz, T[(size_t)j * 3], T[(size_t)j * 3 + 1], T[(size_t)j * 3 + 2]);
+        auto consider = [&](float tx, float ty, float tz, int j) {
+            const float d = sqdist(qx, qy, qz, tx, ty, tz);
             if (d < bd) {
                 bd = d;
                 arg = j;
             }
+        };
+        if (t_aligned32 && j1 - j0 == CHUNK) {
+            const float *tp = T + (size_t)j0 * 3;
+#pragma unroll 2
+            for (int k = 0; k < CHUNK / 8; ++k) {
+                float v[24];
+#pragma unroll
+                for (int h = 0; h < 3; ++h)
+                    asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
+                        : "=f"(v[8 * h]), "=f"(v[8 * h + 1]), "=f"(v[8 * h + 2]), "=f"(v[8 * h + 3]), "=f"(v[8 * h + 4]),
+                          "=f"(v[8 * h + 5]), "=f"(v[8 * h + 6]), "=f"(v[8 * h + 7])
+                        : "l"(tp + 24 * k + 8 * h));
+#pragma unroll
+                for (int i = 0; i < 8; ++i) consider(v[3 * i], v[3 * i + 1], v[3 * i + 2], j0 + 8 * k + i);
+            }
+        } else if (t_aligned && j1 - j0 == CHUNK) {
+            const float4 *__restrict__ t4 = reinterpret_cast<const float4 *>(T + (size_t)j0 * 3);
+#pragma unroll 4
+            for (int k = 0; k < CHUNK / 4; ++k) {
+                const float4 u = __ldg(t4 + 3 * k), v = __ldg(t4 + 3 * k + 1), w = __ldg(t4 + 3 * k + 2);
+                consider(u.x, u.y, u.z, j0 + 4 * k);
+                consider(u.w, v.x, v.y, j0 + 4 * k + 1);
+                consider(v.z, v.w, w.x, j0 + 4 * k + 2);
+                consider(w.y, w.z, w.w, j0 + 4 * k + 3);
+            }
+        } else {
+            for (int j = j0; j < j1; ++j) consider(T[(size_t)j * 3], T[(size_t)j * 3 + 1], T[(size_t)j * 3 + 2], j);
         }
         const u64 key = ((u64)__float_as_uint(bd) << 32) | (unsigned int)arg;
         if (n_split > 1)
@@ -544,6 +583,7 @@ chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restric
         }
     }
 }
+
 
 // The defining arithmetic with packed FP32x2 instructions (two targets per instruction): same
 // results as chamfer_nn_kernel bit for bit, half the FP32-pipe issue slots.

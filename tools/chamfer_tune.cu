@@ -240,9 +240,12 @@ int main(int argc, char **argv) {
     unsigned int *d_amb;
     CK(cudaMalloc(&aux, sizeof(PairAux) * B)); CK(cudaMalloc(&d_amb, 4));
     V(8, 16, 128, 3);
-    T(8, 16, 128, 4, 1024);
-    T(8, 32, 128, 4, 1024);
-    T(8, 64, 128, 4, 1024);
-    T(8, 32, 128, 3, 1024);
+    // chunk widths of the TMA filter scan, interleaved so that clock and neighbour drift hit every width alike
+    const int rounds = getenv("TUNE_ROUNDS") ? atoi(getenv("TUNE_ROUNDS")) : 1;
+    for (int i = 0; i < rounds; ++i) {
+        T(8, 16, 128, 4, 1024);
+        T(8, 32, 128, 4, 1024);
+        T(8, 64, 128, 4, 1024);
+    }
     return 0;
 }
