@@ -9,6 +9,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libptk_b200.so")
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "ptk.h")
 
 CHAMFER_FILTER, CHAMFER_EXACT, CHAMFER_PRUNED, CHAMFER_AUTO = 0, 1, 2, 3
+REDUCE_MEAN, REDUCE_SUM = 0, 1
 PTK_OK, PTK_ERR_SHAPE, PTK_ERR_ALIGN, PTK_ERR_ARCH, PTK_ERR_CUDA, PTK_ERR_WORKSPACE = 0, -1, -2, -3, -4, -5
 
 _vp, _i64, _i32, _sz = C.c_void_p, C.c_int64, C.c_int32, C.c_size_t
@@ -35,6 +36,10 @@ SIGNATURES = {
     "ptk_knn1_fwd": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_chamfer_fwd": (C.c_int, [_vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ptk_chamfer_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp]),
+    "ptk_chamfer_fwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _sz,
+                                          _vp]),
+    "ptk_chamfer_bwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp]),
+    "ptk_knn1_fwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_sample_workspace_bytes": (_sz, [_i64, _i64]),
     "ptk_sample_fwd": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_sample_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp]),

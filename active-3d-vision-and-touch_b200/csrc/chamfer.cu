@@ -32,6 +32,8 @@
 //     PTK_CHAMFER_EXACT (the 6-op scan on packed FP32x2, kept selectable for checks).
 //   * PTK_CHAMFER_PRUNED (chamfer_pruned.cuh): the same results from a cell-sorted copy of both clouds and a box
 //     hierarchy -- a few hundred evaluations per query instead of P; PTK_CHAMFER_AUTO picks it for large clouds.
+//   * ragged batches (ptk_*_lengths): one code path -- every kernel bounds its queries and targets by the pair's
+//     device-side lengths (pair_len(), NULL = full) and keeps the padded strides; the homogeneous calls pass NULL.
 #include <atomic>
 
 #include "chamfer_kernel2.cuh"
@@ -124,43 +126,61 @@ static ChamferWs carve(void *workspace, int64_t B, int64_t P1, int64_t P2) {
     return w;
 }
 
-// Unpack keys -> (dist, idx) and reduce the per-cloud means in a fixed order.
+// Unpack keys -> (dist, idx) and reduce the per-cloud sums in a fixed order.
 // grid = (B, nsplit), block = 512.  cham may be NULL (plain knn).  nsplit = fin_splits(P1, P2) is a function of the cloud
 // sizes only (1 up to 16k points): CTA (b, s) handles slice s of both clouds of pair b; with nsplit > 1 it writes its two
 // partial sums to `partial` and chamfer_finalize_sum_kernel adds them in slice order -- deterministic, and a pair's value
-// does not depend on the batch it is computed in.
+// does not depend on the batch it is computed in.  In a ragged batch each pair is sliced by fin_splits of its OWN lengths
+// (CTAs past that count only zero-fill padding), so its value is also that of a homogeneous call on the sliced pair.
+// Padded queries (i >= len) and queries whose target cloud is empty get dist = 0, idx = 0 (PyTorch3D's zero fill).
 constexpr int FIN_SLICE = 16384;
-static int fin_splits(int64_t P1, int64_t P2) {
+__host__ __device__ inline int fin_splits(int64_t P1, int64_t P2) {
     const int64_t n = ceil_div(P1 > P2 ? P1 : P2, (int64_t)FIN_SLICE);
     return (int)(n < 1 ? 1 : (n > 64 ? 64 : n));
+}
+
+// cham[b] from the two sums: mean = sum_x / max(lx, 1) + sum_y / max(ly, 1), sum = sum_x + sum_y
+__device__ __forceinline__ float chamfer_reduce(float sx, float sy, int L1, int L2, int mean) {
+    return mean ? sx / (float)max(L1, 1) + sy / (float)max(L2, 1) : sx + sy;
 }
 
 __global__ void __launch_bounds__(512)
 chamfer_finalize_kernel(const unsigned long long *__restrict__ keys_x,
                         const unsigned long long *__restrict__ keys_y, int P1, int P2,
+                        const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
                         float *__restrict__ dist_x, int32_t *__restrict__ idx_x,
                         float *__restrict__ dist_y, int32_t *__restrict__ idx_y,
                         float *__restrict__ cham, float *__restrict__ partial) {
     pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
     const int b = blockIdx.x, sp = blockIdx.y, nsp = gridDim.y;
     const int tid = threadIdx.x;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    const int nv = fin_splits(L1, L2);  // == nsp without lengths
     __shared__ float red[16];
     float sum[2] = {0.f, 0.f};
     for (int dir = 0; dir < 2; ++dir) {
         const unsigned long long *keys = dir == 0 ? keys_x : keys_y;
         if (keys == nullptr) continue;
         const int P = dir == 0 ? P1 : P2;
-        const int len = (int)(((long long)P + nsp - 1) / nsp), i0 = sp * len, i1 = min(P, i0 + len);
+        const int L = (dir == 0 ? L2 : L1) == 0 ? 0 : (dir == 0 ? L1 : L2);  // queries with a key; no target: none
         float *dist = dir == 0 ? dist_x : dist_y;
         int32_t *idx = dir == 0 ? idx_x : idx_y;
         float acc = 0.f;
+        if (sp < nv) {
+            const int len = (int)(((long long)L + nv - 1) / nv), i0 = sp * len, i1 = min(L, i0 + len);
 #pragma unroll 8
-        for (int i = i0 + tid; i < i1; i += 512) {
-            unsigned long long k = keys[(size_t)b * P + i];
-            float d = __uint_as_float((unsigned int)(k >> 32));
-            if (dist) dist[(size_t)b * P + i] = d;
-            if (idx) idx[(size_t)b * P + i] = (int32_t)(unsigned int)(k & 0xffffffffull);
-            acc += d;
+            for (int i = i0 + tid; i < i1; i += 512) {
+                unsigned long long k = keys[(size_t)b * P + i];
+                float d = __uint_as_float((unsigned int)(k >> 32));
+                if (dist) dist[(size_t)b * P + i] = d;
+                if (idx) idx[(size_t)b * P + i] = (int32_t)(unsigned int)(k & 0xffffffffull);
+                acc += d;
+            }
+        }
+        const int plen = (P - L + nsp - 1) / nsp, p0 = L + sp * plen, p1 = min(P, p0 + plen);
+        for (int i = p0 + tid; i < p1; i += 512) {
+            if (dist) dist[(size_t)b * P + i] = 0.f;
+            if (idx) idx[(size_t)b * P + i] = 0;
         }
         acc = warp_sum(acc);
         __syncthreads();
@@ -174,81 +194,100 @@ chamfer_finalize_kernel(const unsigned long long *__restrict__ keys_x,
     }
     if (tid == 0 && cham) {
         if (nsp == 1) {
-            cham[b] = sum[0] / (float)P1 + sum[1] / (float)P2;
-        } else {
+            cham[b] = chamfer_reduce(sum[0], sum[1], L1, L2, mean);
+        } else if (sp < nv) {
             partial[((size_t)b * nsp + sp) * 2 + 0] = sum[0];
             partial[((size_t)b * nsp + sp) * 2 + 1] = sum[1];
         }
     }
 }
 
-// grid = ceil(B / 128), block = 128: cham[b] = (sum of the slices' partials, in slice order) / P
+// grid = ceil(B / 128), block = 128: cham[b] from the sums of the pair's slice partials, in slice order (a single
+// partial p gives 0 + p = p: the value of an unsliced pair)
 __global__ void __launch_bounds__(128)
-chamfer_finalize_sum_kernel(const float *__restrict__ partial, int B, int nsp, int P1, int P2, float *__restrict__ cham) {
+chamfer_finalize_sum_kernel(const float *__restrict__ partial, int B, int nsp, int P1, int P2,
+                            const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
+                            float *__restrict__ cham) {
     pdl_wait();
     const int b = blockIdx.x * 128 + threadIdx.x;
     if (b >= B) return;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    const int nv = fin_splits(L1, L2);
     float sx = 0.f, sy = 0.f;
-    for (int s = 0; s < nsp; ++s) {
+    for (int s = 0; s < nv; ++s) {
         sx += partial[((size_t)b * nsp + s) * 2 + 0];
         sy += partial[((size_t)b * nsp + s) * 2 + 1];
     }
-    cham[b] = sx / (float)P1 + sy / (float)P2;
+    cham[b] = chamfer_reduce(sx, sy, L1, L2, mean);
 }
 
-// Backward, phase A (plain stores): the "own point" terms.
-//   grad_x[b,i] = 2 * (g[b]/P1) * (x_i - y[idx_x[i]]);  grad_y[b,j] = 2 * (g[b]/P2) * (y_j - x[idx_y[j]])
+// Backward, phase A (plain stores): the "own point" terms, s_x = 2 g[b] / max(lx, 1) (mean) or 2 g[b] (sum).
+//   grad_x[b,i] = s_x * (x_i - y[idx_x[i]]);  grad_y[b,j] = s_y * (y_j - x[idx_y[j]])
+// Padded points (i >= len) and points whose target cloud is empty get 0: every row is written.
 __global__ void chamfer_bwd_direct_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                           const int32_t *__restrict__ idx_x,
                                           const int32_t *__restrict__ idx_y,
                                           const float *__restrict__ grad_cham, int P1, int P2,
+                                          const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
                                           float *__restrict__ grad_x, float *__restrict__ grad_y) {
     pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
     const int b = blockIdx.y;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const float g = grad_cham[b];
     const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
     if (grad_x && i < P1) {
-        const int j = idx_x[(size_t)b * P1 + i];
-        const float s = 2.0f * (g / (float)P1);
         float *o = grad_x + ((size_t)b * P1 + i) * 3;
-        o[0] = s * (xb[i * 3 + 0] - yb[j * 3 + 0]);
-        o[1] = s * (xb[i * 3 + 1] - yb[j * 3 + 1]);
-        o[2] = s * (xb[i * 3 + 2] - yb[j * 3 + 2]);
+        if (i < L1 && L2 > 0) {
+            const int j = idx_x[(size_t)b * P1 + i];
+            const float s = mean ? 2.0f * (g / (float)L1) : 2.0f * g;
+            o[0] = s * (xb[i * 3 + 0] - yb[j * 3 + 0]);
+            o[1] = s * (xb[i * 3 + 1] - yb[j * 3 + 1]);
+            o[2] = s * (xb[i * 3 + 2] - yb[j * 3 + 2]);
+        } else {
+            o[0] = o[1] = o[2] = 0.f;
+        }
     }
     if (grad_y && i < P2) {
-        const int j = idx_y[(size_t)b * P2 + i];
-        const float s = 2.0f * (g / (float)P2);
         float *o = grad_y + ((size_t)b * P2 + i) * 3;
-        o[0] = s * (yb[i * 3 + 0] - xb[j * 3 + 0]);
-        o[1] = s * (yb[i * 3 + 1] - xb[j * 3 + 1]);
-        o[2] = s * (yb[i * 3 + 2] - xb[j * 3 + 2]);
+        if (i < L2 && L1 > 0) {
+            const int j = idx_y[(size_t)b * P2 + i];
+            const float s = mean ? 2.0f * (g / (float)L2) : 2.0f * g;
+            o[0] = s * (yb[i * 3 + 0] - xb[j * 3 + 0]);
+            o[1] = s * (yb[i * 3 + 1] - xb[j * 3 + 1]);
+            o[2] = s * (yb[i * 3 + 2] - xb[j * 3 + 2]);
+        } else {
+            o[0] = o[1] = o[2] = 0.f;
+        }
     }
 }
 
-// Backward, phase B (scatter): the "I am somebody's nearest neighbour" terms, RED.ADD.F32.
-//   grad_y[b, idx_x[i]] -= 2 (g/P1) (x_i - y[idx_x[i]]);  grad_x[b, idx_y[j]] -= 2 (g/P2) (y_j - x[idx_y[j]])
+// Backward, phase B (scatter): the "I am somebody's nearest neighbour" terms, RED.ADD.F32, from valid queries with a
+// non-empty target cloud only.
+//   grad_y[b, idx_x[i]] -= s_x (x_i - y[idx_x[i]]);  grad_x[b, idx_y[j]] -= s_y (y_j - x[idx_y[j]])
 __global__ void chamfer_bwd_scatter_kernel(const float *__restrict__ x, const float *__restrict__ y,
                                            const int32_t *__restrict__ idx_x,
                                            const int32_t *__restrict__ idx_y,
                                            const float *__restrict__ grad_cham, int P1, int P2,
+                                           const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
                                            float *__restrict__ grad_x, float *__restrict__ grad_y) {
     pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
     const int b = blockIdx.y;
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const float g = grad_cham[b];
     const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
-    if (grad_y && i < P1) {
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    if (grad_y && i < L1 && L2 > 0) {
         const int j = idx_x[(size_t)b * P1 + i];
-        const float s = 2.0f * (g / (float)P1);
+        const float s = mean ? 2.0f * (g / (float)L1) : 2.0f * g;
         float *o = grad_y + ((size_t)b * P2 + j) * 3;
         atomicAdd(o + 0, -(s * (xb[i * 3 + 0] - yb[j * 3 + 0])));
         atomicAdd(o + 1, -(s * (xb[i * 3 + 1] - yb[j * 3 + 1])));
         atomicAdd(o + 2, -(s * (xb[i * 3 + 2] - yb[j * 3 + 2])));
     }
-    if (grad_x && i < P2) {
+    if (grad_x && i < L2 && L1 > 0) {
         const int j = idx_y[(size_t)b * P2 + i];
-        const float s = 2.0f * (g / (float)P2);
+        const float s = mean ? 2.0f * (g / (float)L2) : 2.0f * g;
         float *o = grad_x + ((size_t)b * P1 + j) * 3;
         atomicAdd(o + 0, -(s * (yb[i * 3 + 0] - xb[j * 3 + 0])));
         atomicAdd(o + 1, -(s * (yb[i * 3 + 1] - xb[j * 3 + 1])));
@@ -296,8 +335,8 @@ static unsigned long long g_pr_optin = 0ull;  // cudaFuncAttributeMaxDynamicShar
 
 // PTK_CHAMFER_PRUNED: sort both clouds into cells (one CTA per cloud), walk the box hierarchy (one warp per 32 sorted
 // queries), re-scan the queued queries (exact ties across leaves, non-finite clouds) with the exact kernel.
-static int launch_nn_pruned(const float *x, const float *y, int64_t B, int64_t P1, int64_t P2, const ChamferWs &w,
-                            int dir_only, cudaStream_t st) {
+static int launch_nn_pruned(const float *x, const float *y, const int64_t *lx, const int64_t *ly, int64_t B, int64_t P1,
+                            int64_t P2, const ChamferWs &w, int dir_only, cudaStream_t st) {
     const int ndir = dir_only >= 0 ? 1 : 2;
     const int64_t Pq = dir_only == 0 ? P1 : (dir_only == 1 ? P2 : (P1 > P2 ? P1 : P2));
     const int64_t Pt = dir_only == 0 ? P2 : (dir_only == 1 ? P1 : (P1 > P2 ? P1 : P2));
@@ -314,28 +353,28 @@ static int launch_nn_pruned(const float *x, const float *y, int64_t B, int64_t P
         launch_pdl(pr_wide_init_kernel, dim3((unsigned)(NC / 1024), (unsigned)(2 * B)), dim3(1024), 0, st, w.wide, w.ghist, NC,
                    w.count);
         PTK_CHECK_LAUNCH();
-        launch_pdl(pr_wide_bbox_kernel, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, w.wide);
+        launch_pdl(pr_wide_bbox_kernel, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, lx, ly, w.wide);
         PTK_CHECK_LAUNCH();
         if (fine) {
-            launch_pdl(pr_wide_hist_scatter_kernel<5, false>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2,
+            launch_pdl(pr_wide_hist_scatter_kernel<5, false>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, lx, ly,
                        (const PrWide *)w.wide, w.ghist, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.bad);
             PTK_CHECK_LAUNCH();
             launch_pdl(pr_wide_scan_kernel<5>, dim3((unsigned)(2 * B)), dim3(1024), 0, st, w.ghist);
             PTK_CHECK_LAUNCH();
-            launch_pdl(pr_wide_hist_scatter_kernel<5, true>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2,
+            launch_pdl(pr_wide_hist_scatter_kernel<5, true>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, lx, ly,
                        (const PrWide *)w.wide, w.ghist, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.bad);
         } else {
-            launch_pdl(pr_wide_hist_scatter_kernel<4, false>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2,
+            launch_pdl(pr_wide_hist_scatter_kernel<4, false>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, lx, ly,
                        (const PrWide *)w.wide, w.ghist, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.bad);
             PTK_CHECK_LAUNCH();
             launch_pdl(pr_wide_scan_kernel<4>, dim3((unsigned)(2 * B)), dim3(1024), 0, st, w.ghist);
             PTK_CHECK_LAUNCH();
-            launch_pdl(pr_wide_hist_scatter_kernel<4, true>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2,
+            launch_pdl(pr_wide_hist_scatter_kernel<4, true>, sgrid, dim3(PRW_THREADS), 0, st, x, y, iP1, iP2, lx, ly,
                        (const PrWide *)w.wide, w.ghist, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.bad);
         }
         PTK_CHECK_LAUNCH();
         launch_pdl(pr_wide_leaf_kernel, dim3((unsigned)ceil_div((int64_t)soa_padded((int)Pm) / PR_CHUNK, (int64_t)16), (unsigned)(2 * B)),
-                   dim3(256), 0, st, iP1, iP2, (const float4 *)w.stage_x, (const float4 *)w.stage_y, w.soa_x, w.soa_y, w.box_x,
+                   dim3(256), 0, st, iP1, iP2, lx, ly, (const float4 *)w.stage_x, (const float4 *)w.stage_y, w.soa_x, w.soa_y, w.box_x,
                    w.box_y);
         PTK_CHECK_LAUNCH();
         launch_pdl(pr_wide_inner_kernel, dim3((unsigned)(2 * B)), dim3(1024), 0, st, iP1, iP2, w.box_x, w.box_y);
@@ -348,13 +387,13 @@ static int launch_nn_pruned(const float *x, const float *y, int64_t B, int64_t P
             if (dev < 64) g_pr_optin |= 1ull << dev;
         }
         launch_pdl(chamfer_pruned_sort_kernel<5>, dim3((unsigned)(2 * B)), dim3(PR_SORT_THREADS), 4 * 32768, st, x, y, iP1,
-                   iP2, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.box_x, w.box_y, w.bad, w.count, 0);
+                   iP2, lx, ly, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.box_x, w.box_y, w.bad, w.count, 0);
     } else {
         // <= 32768 points: 16 KB histogram + up to 64 KB of 16-bit cell ranks (the 48 KB default limit covers 16k points)
         const size_t smem = 4 * 4096 + 2 * (size_t)((P1 > P2 ? P1 : P2) + 8);
         int keep = smem <= 48 * 1024 ? 1 : 0;
         launch_pdl(chamfer_pruned_sort_kernel<4>, dim3((unsigned)(2 * B)), dim3(PR_SORT_THREADS), keep ? smem : 4 * 4096, st, x,
-                   y, iP1, iP2, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.box_x, w.box_y, w.bad, w.count, keep);
+                   y, iP1, iP2, lx, ly, w.soa_x, w.soa_y, w.stage_x, w.stage_y, w.box_x, w.box_y, w.bad, w.count, keep);
     }
     PTK_CHECK_LAUNCH();
     u64 *keys_x = dir_only == 1 ? nullptr : w.keys_x;
@@ -367,17 +406,17 @@ static int launch_nn_pruned(const float *x, const float *y, int64_t B, int64_t P
     dim3 qgrid((unsigned)ceil_div(Pq, (int64_t)PR_QUERY_WARPS * 32 * R), (unsigned)(B * ndir));
     if (R == 2)
         launch_pdl(chamfer_pruned_query_kernel<2>, qgrid, dim3(PR_QUERY_WARPS * 32), 0, st, (const float *)w.soa_x,
-                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, keys_x,
+                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, lx, ly, keys_x,
                    keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
     else
         launch_pdl(chamfer_pruned_query_kernel<1>, qgrid, dim3(PR_QUERY_WARPS * 32), 0, st, (const float *)w.soa_x,
-                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, keys_x,
+                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, lx, ly, keys_x,
                    keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
     PTK_CHECK_LAUNCH();
     const NNPlan p = plan_nn(B, Pq, Pt, ndir, CH_MINB, CH_CHUNK);
     dim3 rgrid((unsigned)ceil_div(Pq, (int64_t)CH_THREADS * 8), (unsigned)p.n_split, (unsigned)(B * ndir));
     launch_pdl(chamfer_nn_exact2_kernel<8, CH_CHUNK, CH_THREADS, CH_MINB>, rgrid, dim3(CH_THREADS), 0, st, x, y, iP1, iP2,
-               p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
+               lx, ly, p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }
@@ -392,10 +431,12 @@ static int resolve_algo(int64_t P1, int64_t P2) {
     return algo;
 }
 
-static int launch_nn(const float *x, const float *y, int64_t B, int64_t P1, int64_t P2, const ChamferWs &w,
-                     int dir_only, cudaStream_t st) {
+// lx / ly: per-pair lengths (NULL: every cloud is full).  Plans, grids and the choice of the scan come from the padded
+// sizes; the kernels bound their queries and targets by the lengths.
+static int launch_nn(const float *x, const float *y, const int64_t *lx, const int64_t *ly, int64_t B, int64_t P1,
+                     int64_t P2, const ChamferWs &w, int dir_only, cudaStream_t st) {
     const int algo = resolve_algo(P1, P2);
-    if (algo == PTK_CHAMFER_PRUNED) return launch_nn_pruned(x, y, B, P1, P2, w, dir_only, st);
+    if (algo == PTK_CHAMFER_PRUNED) return launch_nn_pruned(x, y, lx, ly, B, P1, P2, w, dir_only, st);
     const int ndir = dir_only >= 0 ? 1 : 2;
     const int64_t Pq = dir_only == 0 ? P1 : (dir_only == 1 ? P2 : (P1 > P2 ? P1 : P2));
     const int64_t Pt = dir_only == 0 ? P2 : (dir_only == 1 ? P1 : (P1 > P2 ? P1 : P2));
@@ -425,15 +466,15 @@ static int launch_nn(const float *x, const float *y, int64_t B, int64_t P1, int6
                 "chamfer: batch %lld too large for one launch (max 32767 clouds)", (long long)B);
     const int iP1 = (int)P1, iP2 = (int)P2;
     if (filter) {
-        launch_pdl(chamfer_bounds_kernel, dim3((unsigned)B), dim3(1024), 0, st, x, y, iP1, iP2, w.aux, w.count);
+        launch_pdl(chamfer_bounds_kernel, dim3((unsigned)B), dim3(1024), 0, st, x, y, iP1, iP2, lx, ly, w.aux, w.count);
         PTK_CHECK_LAUNCH();
         const int Pp = soa_padded(iP1 > iP2 ? iP1 : iP2);
         launch_pdl(chamfer_prep_kernel, dim3((unsigned)ceil_div(Pp, 256), (unsigned)(2 * B)), dim3(256), 0, st, x, y, iP1, iP2,
-                   w.aux, w.soa_x, w.soa_y, keys_x, keys_y, w.flag_x, w.flag_y, p.n_split > 1 ? 1 : 0);
+                   lx, ly, w.aux, w.soa_x, w.soa_y, keys_x, keys_y, w.flag_x, w.flag_y, p.n_split > 1 ? 1 : 0);
         PTK_CHECK_LAUNCH();
 #define PTK_FILTER(RR, CC)                                                                                      \
     launch_pdl(chamfer_nn_filter_tma_kernel<RR, CC, CH_THREADS, CH_MINB_F, CH_TT_F>, grid, dim3(CH_THREADS), 0, st,      \
-               x, y, iP1, iP2, p.split_len, p.n_split, w.aux, w.soa_x, w.soa_y, w.keys_x, w.keys_y, dir_only, w.rescue_x, \
+               x, y, iP1, iP2, lx, ly, p.split_len, p.n_split, w.aux, w.soa_x, w.soa_y, w.keys_x, w.keys_y, dir_only, w.rescue_x, \
                w.rescue_y, w.count, w.flag_x, w.flag_y)
         switch (p.R) {
             case 8: if (wide) PTK_FILTER(8, CH_CHUNK_F); else PTK_FILTER(8, CH_CHUNK); break;
@@ -445,13 +486,13 @@ static int launch_nn(const float *x, const float *y, int64_t B, int64_t P1, int6
         // rescue pass over the queued (ambiguous) queries; CTAs beyond the list length exit at once
         dim3 rgrid((unsigned)ceil_div(Pq, (int64_t)CH_THREADS * 8), (unsigned)p.n_split, (unsigned)(B * ndir));
         launch_pdl(chamfer_nn_exact2_kernel<8, CH_CHUNK, CH_THREADS, CH_MINB>, rgrid, dim3(CH_THREADS), 0, st, x, y, iP1, iP2,
-                   p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
+                   lx, ly, p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
         PTK_CHECK_LAUNCH();
         return PTK_OK;
     }
 #define PTK_EXACT(RR)                                                                            \
     launch_pdl(chamfer_nn_exact2_kernel<RR, CH_CHUNK, CH_THREADS, CH_MINB>, grid, dim3(CH_THREADS), 0, st, x, y, iP1, iP2, \
-               p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, nullptr, nullptr, nullptr)
+               lx, ly, p.split_len, p.n_split, w.keys_x, w.keys_y, dir_only, nullptr, nullptr, nullptr)
     switch (p.R) {
         case 8: PTK_EXACT(8); break;
         case 4: PTK_EXACT(4); break;
@@ -523,10 +564,8 @@ static int check_clouds(const void *x, const void *y, int64_t B, int64_t P1, int
     return PTK_OK;
 }
 
-extern "C" int ptk_knn1_fwd(const float *p1, const float *p2, int64_t B, int64_t P1, int64_t P2,
-                            float *dist, int32_t *idx, void *workspace, size_t workspace_bytes,
-                            ptk_stream_t stream) {
-    PTK_NVTX("ptk_knn1_fwd");
+static int knn1_fwd(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, int64_t B, int64_t P1,
+                    int64_t P2, float *dist, int32_t *idx, void *workspace, size_t workspace_bytes, ptk_stream_t stream) {
     int rc = check_clouds(p1, p2, B, P1, P2);
     if (rc) return rc;
     PTK_REQUIRE(workspace && workspace_bytes >= chamfer_ws_bytes(B, P1, P2), PTK_ERR_WORKSPACE,
@@ -534,20 +573,40 @@ extern "C" int ptk_knn1_fwd(const float *p1, const float *p2, int64_t B, int64_t
     PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN, "knn1: workspace must be 16-byte aligned");
     cudaStream_t st = as_stream(stream);
     const ChamferWs w = carve(workspace, B, P1, P2);
-    rc = launch_nn(p1, p2, B, P1, P2, w, 0, st);
+    rc = launch_nn(p1, p2, len1, len2, B, P1, P2, w, 0, st);
     if (rc) return rc;
     launch_pdl(chamfer_finalize_kernel, dim3((unsigned)B, (unsigned)fin_splits(P1, P2)), dim3(512), 0, st, w.keys_x, nullptr,
-               (int)P1, (int)P2, dist, idx, nullptr, nullptr, nullptr, nullptr);
+               (int)P1, (int)P2, len1, len2, 1, dist, idx, nullptr, nullptr, nullptr, nullptr);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }
 
-extern "C" int ptk_chamfer_fwd(const float *x, const float *y, int64_t B, int64_t P1, int64_t P2,
-                               float *dist_x, int32_t *idx_x, float *dist_y, int32_t *idx_y,
-                               float *cham, void *workspace, size_t workspace_bytes,
-                               ptk_stream_t stream) {
-    PTK_NVTX("ptk_chamfer_fwd");
+extern "C" int ptk_knn1_fwd(const float *p1, const float *p2, int64_t B, int64_t P1, int64_t P2,
+                            float *dist, int32_t *idx, void *workspace, size_t workspace_bytes,
+                            ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_fwd");
+    return knn1_fwd(p1, p2, nullptr, nullptr, B, P1, P2, dist, idx, workspace, workspace_bytes, stream);
+}
+
+extern "C" int ptk_knn1_fwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, int64_t B,
+                                    int64_t P1, int64_t P2, float *dist, int32_t *idx, void *workspace,
+                                    size_t workspace_bytes, ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_fwd_lengths");
+    return knn1_fwd(p1, p2, len1, len2, B, P1, P2, dist, idx, workspace, workspace_bytes, stream);
+}
+
+static int check_reduction(int reduction) {
+    PTK_REQUIRE(reduction == PTK_REDUCE_MEAN || reduction == PTK_REDUCE_SUM, PTK_ERR_SHAPE,
+                "chamfer: unknown point reduction %d", reduction);
+    return PTK_OK;
+}
+
+static int chamfer_fwd(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y, int64_t B, int64_t P1,
+                       int64_t P2, int reduction, float *dist_x, int32_t *idx_x, float *dist_y, int32_t *idx_y, float *cham,
+                       void *workspace, size_t workspace_bytes, ptk_stream_t stream) {
     int rc = check_clouds(x, y, B, P1, P2);
+    if (rc) return rc;
+    rc = check_reduction(reduction);
     if (rc) return rc;
     PTK_REQUIRE(idx_x && idx_y && cham, PTK_ERR_SHAPE, "chamfer_fwd: idx_x, idx_y and cham are required");
     PTK_REQUIRE(workspace && workspace_bytes >= ptk_chamfer_workspace_bytes(B, P1, P2),
@@ -557,18 +616,60 @@ extern "C" int ptk_chamfer_fwd(const float *x, const float *y, int64_t B, int64_
                 "chamfer_fwd: workspace must be 16-byte aligned");
     cudaStream_t st = as_stream(stream);
     const ChamferWs w = carve(workspace, B, P1, P2);
-    rc = launch_nn(x, y, B, P1, P2, w, -1, st);
+    rc = launch_nn(x, y, len_x, len_y, B, P1, P2, w, -1, st);
     if (rc) return rc;
     const int nsp = fin_splits(P1, P2);
+    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
     // partial sums of the slices: the rescue flags are dead once the scan is over (flag_x holds B * P1 >= 2 * B * nsp words)
     float *partial = reinterpret_cast<float *>(w.flag_x);
     launch_pdl(chamfer_finalize_kernel, dim3((unsigned)B, (unsigned)nsp), dim3(512), 0, st, w.keys_x, w.keys_y, (int)P1, (int)P2,
-               dist_x, idx_x, dist_y, idx_y, cham, partial);
+               len_x, len_y, mean, dist_x, idx_x, dist_y, idx_y, cham, partial);
     if (nsp > 1) {
         PTK_CHECK_LAUNCH();
         launch_pdl(chamfer_finalize_sum_kernel, dim3((unsigned)ceil_div(B, (int64_t)128)), dim3(128), 0, st, (const float *)partial,
-                   (int)B, nsp, (int)P1, (int)P2, cham);
+                   (int)B, nsp, (int)P1, (int)P2, len_x, len_y, mean, cham);
     }
+    PTK_CHECK_LAUNCH();
+    return PTK_OK;
+}
+
+extern "C" int ptk_chamfer_fwd(const float *x, const float *y, int64_t B, int64_t P1, int64_t P2,
+                               float *dist_x, int32_t *idx_x, float *dist_y, int32_t *idx_y,
+                               float *cham, void *workspace, size_t workspace_bytes,
+                               ptk_stream_t stream) {
+    PTK_NVTX("ptk_chamfer_fwd");
+    return chamfer_fwd(x, y, nullptr, nullptr, B, P1, P2, PTK_REDUCE_MEAN, dist_x, idx_x, dist_y, idx_y, cham, workspace,
+                       workspace_bytes, stream);
+}
+
+extern "C" int ptk_chamfer_fwd_lengths(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y, int64_t B,
+                                       int64_t P1, int64_t P2, int reduction, float *dist_x, int32_t *idx_x, float *dist_y,
+                                       int32_t *idx_y, float *cham, void *workspace, size_t workspace_bytes,
+                                       ptk_stream_t stream) {
+    PTK_NVTX("ptk_chamfer_fwd_lengths");
+    return chamfer_fwd(x, y, len_x, len_y, B, P1, P2, reduction, dist_x, idx_x, dist_y, idx_y, cham, workspace,
+                       workspace_bytes, stream);
+}
+
+static int chamfer_bwd(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y, const int32_t *idx_x,
+                       const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1, int64_t P2, int reduction,
+                       float *grad_x, float *grad_y, ptk_stream_t stream) {
+    int rc = check_clouds(x, y, B, P1, P2);
+    if (rc) return rc;
+    rc = check_reduction(reduction);
+    if (rc) return rc;
+    PTK_REQUIRE(idx_x && idx_y && grad_cham, PTK_ERR_SHAPE, "chamfer_bwd: null index / grad pointer");
+    if (!grad_x && !grad_y) return PTK_OK;
+    cudaStream_t st = as_stream(stream);
+    const int64_t Pm = P1 > P2 ? P1 : P2;
+    dim3 grid((unsigned)ceil_div(Pm, 256), (unsigned)B);
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "chamfer_bwd: batch too large");
+    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
+    launch_pdl(chamfer_bwd_direct_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, len_x, len_y,
+               mean, grad_x, grad_y);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(chamfer_bwd_scatter_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, len_x, len_y,
+               mean, grad_x, grad_y);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }
@@ -577,19 +678,13 @@ extern "C" int ptk_chamfer_bwd(const float *x, const float *y, const int32_t *id
                                const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1,
                                int64_t P2, float *grad_x, float *grad_y, ptk_stream_t stream) {
     PTK_NVTX("ptk_chamfer_bwd");
-    int rc = check_clouds(x, y, B, P1, P2);
-    if (rc) return rc;
-    PTK_REQUIRE(idx_x && idx_y && grad_cham, PTK_ERR_SHAPE, "chamfer_bwd: null index / grad pointer");
-    if (!grad_x && !grad_y) return PTK_OK;
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    dim3 grid((unsigned)ceil_div(Pm, 256), (unsigned)B);
-    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "chamfer_bwd: batch too large");
-    launch_pdl(chamfer_bwd_direct_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, grad_x,
-               grad_y);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_bwd_scatter_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, grad_x,
-               grad_y);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
+    return chamfer_bwd(x, y, nullptr, nullptr, idx_x, idx_y, grad_cham, B, P1, P2, PTK_REDUCE_MEAN, grad_x, grad_y, stream);
+}
+
+extern "C" int ptk_chamfer_bwd_lengths(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y,
+                                       const int32_t *idx_x, const int32_t *idx_y, const float *grad_cham, int64_t B,
+                                       int64_t P1, int64_t P2, int reduction, float *grad_x, float *grad_y,
+                                       ptk_stream_t stream) {
+    PTK_NVTX("ptk_chamfer_bwd_lengths");
+    return chamfer_bwd(x, y, len_x, len_y, idx_x, idx_y, grad_cham, B, P1, P2, reduction, grad_x, grad_y, stream);
 }

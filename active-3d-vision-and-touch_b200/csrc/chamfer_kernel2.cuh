@@ -78,12 +78,23 @@ struct PairAux {
 };
 constexpr float FILTER_THR_BD = 1.9073486e-6f;  // 32 u = 2^-19
 
+// Ragged batches: the points of cloud b that exist, len[b] clamped to [0, P] (P when the caller passed no lengths).
+// Row strides stay those of the padded (B, P, 3) tensor; only the counts of queries and targets become per pair, so
+// padding points are never read into a result, a bound or the filter's certificate.
+__device__ __forceinline__ int pair_len(const int64_t *__restrict__ len, int b, int P) {
+    if (len == nullptr) return P;
+    const long long v = len[b];
+    return v < 0 ? 0 : (v > P ? P : (int)v);
+}
+
 __global__ void __launch_bounds__(1024)
 chamfer_bounds_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                      const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
                       PairAux *__restrict__ aux, unsigned int *__restrict__ rescue_count) {
     pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
     const int b = blockIdx.x;
     const int tid = threadIdx.x;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
     const float PINF = __int_as_float(0x7f800000), NINF = __int_as_float(0xff800000);
     __shared__ float sred[7][32];
     __shared__ float sctr[3];
@@ -96,7 +107,7 @@ chamfer_bounds_kernel(const float *__restrict__ x, const float *__restrict__ y, 
     bool bad = false;
     for (int s = 0; s < 2; ++s) {
         const float *p = s == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
-        const int n = (s == 0 ? P1 : P2) * 3;
+        const int n = (s == 0 ? L1 : L2) * 3;
         // eight loads in flight per thread: at small batches this single CTA per pair is latency-bound
         for (int e0 = tid; e0 < n; e0 += 8 * 1024) {
             float v[8];
@@ -138,7 +149,7 @@ chamfer_bounds_kernel(const float *__restrict__ x, const float *__restrict__ y, 
             l = fminf(l, sred[tid][w]);
             h = fmaxf(h, sred[3 + tid][w]);
         }
-        sctr[tid] = 0.5f * l + 0.5f * h;
+        sctr[tid] = l <= h ? 0.5f * l + 0.5f * h : 0.f;  // no finite point (both clouds empty): not NaN
     }
     __syncthreads();
     const float cx = sctr[0], cy = sctr[1], cz = sctr[2];
@@ -147,7 +158,7 @@ chamfer_bounds_kernel(const float *__restrict__ x, const float *__restrict__ y, 
     float m2 = 0.f;
     for (int s = 0; s < 2; ++s) {
         const float *p = s == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
-        const int n = s == 0 ? P1 : P2;
+        const int n = s == 0 ? L1 : L2;
 #pragma unroll 4
         for (int i = tid; i < n; i += 1024) {
             const float dx = __fsub_rn(p[i * 3 + 0], cx), dy = __fsub_rn(p[i * 3 + 1], cy), dz = __fsub_rn(p[i * 3 + 2], cz);
@@ -349,6 +360,7 @@ __host__ __device__ inline int soa_padded(int P) { return (P + SOA_PAD - 1) / SO
 // grid (ceil(Ppad_max / 256), 2 * B): blockIdx.y = 2 * b + cloud
 __global__ void __launch_bounds__(256)
 chamfer_prep_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                    const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
                     const PairAux *__restrict__ aux, float *__restrict__ soa_x, float *__restrict__ soa_y,
                     u64 *__restrict__ keys_x, u64 *__restrict__ keys_y, unsigned int *__restrict__ flag_x,
                     unsigned int *__restrict__ flag_y, int init_keys) {
@@ -361,8 +373,10 @@ chamfer_prep_kernel(const float *__restrict__ x, const float *__restrict__ y, in
     const float *src = (cloud == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3);
     float *dst = (cloud == 0 ? soa_x + (size_t)b * 4 * Pp : soa_y + (size_t)b * 4 * Pp);
     const PairAux ax = aux[b];
+    // points past the cloud's length are padding like those past P: the scan's tiles round up to whole chunks and
+    // read up to a chunk past the length
     float tx = 0.f, ty = 0.f, tz = 0.f, tt = __int_as_float(0x7f800000);
-    if (i < P) {
+    if (i < pair_len(cloud == 0 ? len_x : len_y, b, P)) {
         tx = __fsub_rn(src[i * 3 + 0], ax.cx);
         ty = __fsub_rn(src[i * 3 + 1], ax.cy);
         tz = __fsub_rn(src[i * 3 + 2], ax.cz);
@@ -398,6 +412,7 @@ __device__ __forceinline__ void mbar_wait_parity(uint32_t bar, uint32_t parity) 
 template <int R, int CHUNK, int THREADS, int MINB, int TT>
 __global__ void __launch_bounds__(THREADS, MINB)
 chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                             const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
                              int split_len, int n_split, const PairAux *__restrict__ aux,
                              const float *__restrict__ soa_x, const float *__restrict__ soa_y,
                              u64 *__restrict__ keys_x, u64 *__restrict__ keys_y, int dir_only,
@@ -409,8 +424,10 @@ chamfer_nn_filter_tma_kernel(const float *__restrict__ x, const float *__restric
     const int z = blockIdx.z;
     const int b = dir_only >= 0 ? z : (z >> 1);
     const int dir = dir_only >= 0 ? dir_only : (z & 1);
-    const int NQ = dir == 0 ? P1 : P2;
-    const int NT = dir == 0 ? P2 : P1;
+    // NQ / NT: this pair's lengths (the SoA and AoS strides below keep using P1 / P2).  The exits below come before any
+    // query load, so NQ >= 1 and NT >= 1 past them; a chunk that straddles NT fails `j1 - j0 == CHUNK` in the recheck.
+    const int NQ = pair_len(dir == 0 ? len_x : len_y, b, dir == 0 ? P1 : P2);
+    const int NT = pair_len(dir == 0 ? len_y : len_x, b, dir == 0 ? P2 : P1);
     const int P1p = soa_padded(P1), P2p = soa_padded(P2);
     const int NQp = dir == 0 ? P1p : P2p, NTp = dir == 0 ? P2p : P1p;
     const float *__restrict__ Q = dir == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
@@ -706,6 +723,7 @@ __device__ __forceinline__ void exact2_body(const float *__restrict__ Q, const f
 template <int R, int CHUNK, int THREADS, int MINB>
 __global__ void __launch_bounds__(THREADS, MINB)
 chamfer_nn_exact2_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                         const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
                          int split_len, int n_split, u64 *__restrict__ keys_x,
                          u64 *__restrict__ keys_y, int dir_only, const int *__restrict__ rescue_x,
                          const int *__restrict__ rescue_y, const unsigned int *__restrict__ rescue_count) {
@@ -713,8 +731,8 @@ chamfer_nn_exact2_kernel(const float *__restrict__ x, const float *__restrict__ 
     const int z = blockIdx.z;
     const int b = dir_only >= 0 ? z : (z >> 1);
     const int dir = dir_only >= 0 ? dir_only : (z & 1);
-    const int NQ = dir == 0 ? P1 : P2;
-    const int NT = dir == 0 ? P2 : P1;
+    const int NQ = pair_len(dir == 0 ? len_x : len_y, b, dir == 0 ? P1 : P2);  // this pair's lengths, as in the filter
+    const int NT = pair_len(dir == 0 ? len_y : len_x, b, dir == 0 ? P2 : P1);
     const float *__restrict__ Q = dir == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
     const float *__restrict__ T = dir == 0 ? y + (size_t)b * P2 * 3 : x + (size_t)b * P1 * 3;
     u64 *__restrict__ keys = dir == 0 ? keys_x + (size_t)b * P1 : keys_y + (size_t)b * P2;

@@ -91,7 +91,8 @@ __device__ __forceinline__ unsigned pr_cell_rank(int cx, int cy, int cz) {
 // + 2 * max(P1, P2) bytes when keep_codes.
 template <int BITS>
 __global__ void __launch_bounds__(PR_SORT_THREADS)
-chamfer_pruned_sort_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2, float *soa_x,
+chamfer_pruned_sort_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                           const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, float *soa_x,
                            float *soa_y, float4 *stage_x, float4 *stage_y, PrBox *box_x, PrBox *box_y,
                            int *__restrict__ bad_flags, unsigned int *__restrict__ rescue_count, int keep_codes) {
     constexpr int G = 1 << BITS, NC = G * G * G, PER = NC / PR_SORT_THREADS;
@@ -106,13 +107,17 @@ chamfer_pruned_sort_kernel(const float *__restrict__ x, const float *__restrict_
     (void)t_phase;
     const int b = blockIdx.x >> 1, cloud = blockIdx.x & 1;
     const int tid = threadIdx.x;
-    const int P = cloud == 0 ? P1 : P2;
-    const int Pp = soa_padded(P);
+    // Pc sizes the layout (padded cloud); only the cloud's first P points exist and are sorted.  Leaves past them hold
+    // padding only: their box is empty (lo = +inf, hi = -inf), its lower bound +inf, and so is that of an inner box
+    // over such leaves -- never below a live query's best once one leaf has been scanned.
+    const int Pc = cloud == 0 ? P1 : P2;
+    const int P = pair_len(cloud == 0 ? len_x : len_y, b, Pc);
+    const int Pp = soa_padded(Pc);
     const float *__restrict__ src = cloud == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
     float *out = cloud == 0 ? soa_x + (size_t)b * 4 * Pp : soa_y + (size_t)b * 4 * Pp;
     float4 *stage = cloud == 0 ? stage_x + (size_t)b * Pp : stage_y + (size_t)b * Pp;
-    PrBox *box0 = (cloud == 0 ? box_x : box_y) + (size_t)b * pr_boxes(P);
-    const int nb0 = pr_nb0(P), nb1 = pr_nb1(P), nb2 = pr_nb2(P);
+    PrBox *box0 = (cloud == 0 ? box_x : box_y) + (size_t)b * pr_boxes(Pc);
+    const int nb0 = pr_nb0(Pc), nb1 = pr_nb1(Pc), nb2 = pr_nb2(Pc);
     PrBox *box1 = box0 + nb0, *box2 = box1 + nb1;
     const float PINF = __int_as_float(0x7f800000), NINF = __int_as_float(0xff800000);
     if (tid == 0) sbad = 0;
@@ -364,10 +369,11 @@ pr_wide_init_kernel(PrWide *__restrict__ st, unsigned int *__restrict__ ghist, i
 
 // grid (ceil(Pmax / PRW_SLICE), 2 * B), block 256
 __global__ void __launch_bounds__(PRW_THREADS)
-pr_wide_bbox_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2, PrWide *__restrict__ st) {
+pr_wide_bbox_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                    const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, PrWide *__restrict__ st) {
     pdl_wait();
     const int cl = blockIdx.y, b = cl >> 1, cloud = cl & 1;
-    const int P = cloud == 0 ? P1 : P2;
+    const int P = pair_len(cloud == 0 ? len_x : len_y, b, cloud == 0 ? P1 : P2);  // valid points only
     const int e0 = blockIdx.x * PRW_SLICE * 3, e1 = min(P * 3, e0 + PRW_SLICE * 3);
     if (e0 >= e1) return;
     const float *__restrict__ src = cloud == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
@@ -426,12 +432,14 @@ __device__ __forceinline__ unsigned pr_wide_cell(const float (&org)[3], const fl
 template <int BITS, bool SCATTER>
 __global__ void __launch_bounds__(PRW_THREADS)
 pr_wide_hist_scatter_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,
+                            const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
                             const PrWide *__restrict__ st, unsigned int *__restrict__ ghist, float *soa_x, float *soa_y,
                             float4 *__restrict__ stage_x, float4 *__restrict__ stage_y, int *__restrict__ bad_flags) {
     pdl_wait();
     constexpr int NC = 1 << (3 * BITS);
     const int cl = blockIdx.y, b = cl >> 1, cloud = cl & 1;
-    const int P = cloud == 0 ? P1 : P2, Pp = soa_padded(P);
+    const int Pc = cloud == 0 ? P1 : P2, Pp = soa_padded(Pc);  // layout; P: the points that exist
+    const int P = pair_len(cloud == 0 ? len_x : len_y, b, Pc);
     const int i0 = blockIdx.x * PRW_SLICE + threadIdx.x;
     if (blockIdx.x * PRW_SLICE >= P) return;
     const float *__restrict__ src = cloud == 0 ? x + (size_t)b * P1 * 3 : y + (size_t)b * P2 * 3;
@@ -523,16 +531,18 @@ pr_wide_scan_kernel(unsigned int *__restrict__ ghist) {
 // grid (ceil(leaves / 16), 2 * B), block 256: a half-warp per leaf -- transpose the staged points into the leaf layout,
 // reduce the leaf box (the same pass as in chamfer_pruned_sort_kernel)
 __global__ void __launch_bounds__(256)
-pr_wide_leaf_kernel(int P1, int P2, const float4 *__restrict__ stage_x, const float4 *__restrict__ stage_y, float *soa_x,
-                    float *soa_y, PrBox *box_x, PrBox *box_y) {
+pr_wide_leaf_kernel(int P1, int P2, const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
+                    const float4 *__restrict__ stage_x, const float4 *__restrict__ stage_y, float *soa_x, float *soa_y,
+                    PrBox *box_x, PrBox *box_y) {
     pdl_wait();
     const int cl = blockIdx.y, b = cl >> 1, cloud = cl & 1;
-    const int P = cloud == 0 ? P1 : P2, Pp = soa_padded(P);
+    const int Pc = cloud == 0 ? P1 : P2, Pp = soa_padded(Pc);  // layout; P: the points that exist
+    const int P = pair_len(cloud == 0 ? len_x : len_y, b, Pc);
     const int c = blockIdx.x * 16 + (threadIdx.x >> 4), l16 = threadIdx.x & 15, lane = threadIdx.x & 31;
     if (c >= Pp / PR_CHUNK) return;  // uniform per half-warp
     const float4 *__restrict__ stage = cloud == 0 ? stage_x + (size_t)b * Pp : stage_y + (size_t)b * Pp;
     float *o = (cloud == 0 ? soa_x + (size_t)b * 4 * Pp : soa_y + (size_t)b * 4 * Pp) + (size_t)c * 64;
-    PrBox *box0 = (cloud == 0 ? box_x : box_y) + (size_t)b * pr_boxes(P);
+    PrBox *box0 = (cloud == 0 ? box_x : box_y) + (size_t)b * pr_boxes(Pc);
     const float PINF = __int_as_float(0x7f800000), NINF = __int_as_float(0xff800000);
     const bool live = c * PR_CHUNK + l16 < P;
     float4 pt = make_float4(PINF, PINF, PINF, __int_as_float(0x7fffffff));
@@ -550,7 +560,7 @@ pr_wide_leaf_kernel(int P1, int P2, const float4 *__restrict__ stage_x, const fl
             l[k] = fminf(l[k], __shfl_xor_sync(hmask, l[k], off));
             h[k] = fmaxf(h[k], __shfl_xor_sync(hmask, h[k], off));
         }
-    if (l16 == 0 && c < pr_nb0(P)) {
+    if (l16 == 0 && c < pr_nb0(Pc)) {
         box0[c].lo = make_float4(l[0], l[1], l[2], 0.f);
         box0[c].hi = make_float4(h[0], h[1], h[2], 0.f);
     }
@@ -624,7 +634,8 @@ template <int R>
 __global__ void __launch_bounds__(PR_QUERY_WARPS * 32)
 chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__restrict__ soa_y,
                             const PrBox *__restrict__ box_x, const PrBox *__restrict__ box_y,
-                            const int *__restrict__ bad_flags, int P1, int P2, u64 *__restrict__ keys_x,
+                            const int *__restrict__ bad_flags, int P1, int P2, const int64_t *__restrict__ len_x,
+                            const int64_t *__restrict__ len_y, u64 *__restrict__ keys_x,
                             u64 *__restrict__ keys_y, int dir_only, int *__restrict__ rescue_x,
                             int *__restrict__ rescue_y, unsigned int *__restrict__ rescue_count) {
     pdl_wait();
@@ -632,16 +643,19 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
     const int z = blockIdx.y;
     const int b = dir_only >= 0 ? z : (z >> 1);
     const int dir = dir_only >= 0 ? dir_only : (z & 1);
-    const int NQ = dir == 0 ? P1 : P2, NT = dir == 0 ? P2 : P1;
+    // NQ / NT: this pair's lengths; the layout of the sorted clouds and boxes is that of the padded sizes
+    const int NQ = pair_len(dir == 0 ? len_x : len_y, b, dir == 0 ? P1 : P2);
+    const int NT = pair_len(dir == 0 ? len_y : len_x, b, dir == 0 ? P2 : P1);
     const int lane = threadIdx.x & 31;
     const int base = (blockIdx.x * PR_QUERY_WARPS + (threadIdx.x >> 5)) * 32 * R;  // first sorted position of the warp
-    if (base >= NQ) return;  // whole warp
+    if (base >= NQ || NT == 0) return;  // whole warp (no target: chamfer_finalize_kernel writes the zero result)
     const int P1p = soa_padded(P1), P2p = soa_padded(P2);
     const int NQp = dir == 0 ? P1p : P2p;
     const float *__restrict__ QS = dir == 0 ? soa_x + (size_t)b * 4 * P1p : soa_y + (size_t)b * 4 * P2p;
     const float *__restrict__ TS = dir == 0 ? soa_y + (size_t)b * 4 * P2p : soa_x + (size_t)b * 4 * P1p;
     const PrBox *__restrict__ b0 = dir == 0 ? box_y + (size_t)b * pr_boxes(P2) : box_x + (size_t)b * pr_boxes(P1);
-    const int nb0 = pr_nb0(NT), nb1 = pr_nb1(NT), nb2 = pr_nb2(NT);
+    const int NTc = dir == 0 ? P2 : P1;
+    const int nb0 = pr_nb0(NTc), nb1 = pr_nb1(NTc), nb2 = pr_nb2(NTc);
     const PrBox *__restrict__ b1 = b0 + nb0, *__restrict__ b2 = b1 + nb1;
     u64 *__restrict__ keys = dir == 0 ? keys_x + (size_t)b * P1 : keys_y + (size_t)b * P2;
     int *__restrict__ list = dir == 0 ? rescue_x + (size_t)b * P1 : rescue_y + (size_t)b * P2;
@@ -679,7 +693,7 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
         for (int r = 0; r < R; ++r) qx2[r] = pack2(qx[r], qx[r]), qy2[r] = pack2(qy[r], qy[r]), qz2[r] = pack2(qz[r], qz[r]);
         unsigned wbest = 0x7f800000u;  // bit pattern of the largest `best` among the warp's live queries
         int scans = 0;
-        const int scan_cap = max(64, nb0 >> 3);
+        const int scan_cap = max(64, pr_nb0(NT) >> 3);
         bool bail = false;
 
         int st1 = 0, st2 = 0, st3 = 0, stA = 0, stB = 0, stL = 0;

@@ -46,13 +46,37 @@ def set_chamfer_algo(name):
     _lib.check(_lib.lib().ptk_chamfer_set_algo(algo), "ptk_chamfer_set_algo")
 
 
-def chamfer_rescued(x, y):
+_REDUCTIONS = {"mean": _lib.REDUCE_MEAN, "sum": _lib.REDUCE_SUM}
+
+
+def _lengths(lengths, B, device, name):
+    """Per-cloud lengths as a contiguous int64 (B,) device tensor, or None.  No host synchronisation: the values are
+    clamped to [0, P] by the kernels."""
+    if lengths is None:
+        return None
+    if not torch.is_tensor(lengths) or lengths.dtype not in (torch.int32, torch.int64):
+        raise ValueError(f"{name} must be an int32 or int64 tensor")
+    if lengths.shape != (B,):
+        raise ValueError(f"{name} must have shape ({B},), got {tuple(lengths.shape)}")
+    return lengths.to(device=device, dtype=torch.int64, non_blocking=True).contiguous()
+
+
+def _check_pair(x, y):
+    if x.dim() != 3 or y.dim() != 3 or x.shape[2] != 3 or y.shape[2] != 3:
+        raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(x.shape)} and {tuple(y.shape)}")
+    if x.shape[0] != y.shape[0]:
+        raise ValueError("y must have the same batch dimension as x")
+
+
+def chamfer_rescued(x, y, x_lengths=None, y_lengths=None):
     """Diagnostics: run the forward NN scan on (x, y) and return how many of the B*(P1+P2) queries the
-    filter could not decide (near or exact ties across chunks) and handed to the exact rescue scan."""
+    filter could not decide (near or exact ties across chunks) and handed to the exact rescue scan.
+    x_lengths / y_lengths: a ragged batch, as in chamfer()."""
     _need_cuda(x, y)
     x, y = _f32c(x), _f32c(y)
     B, P1, _ = x.shape
     P2 = y.shape[1]
+    lx, ly = _lengths(x_lengths, B, x.device, "x_lengths"), _lengths(y_lengths, B, x.device, "y_lengths")
     L = _lib.lib()
     idx_x = torch.empty(B, P1, dtype=torch.int32, device=x.device)
     idx_y = torch.empty(B, P2, dtype=torch.int32, device=x.device)
@@ -60,23 +84,22 @@ def chamfer_rescued(x, y):
     ws = _ws(L.ptk_chamfer_workspace_bytes(B, P1, P2), x.device)
     n = C.c_int64(0)
     with torch.cuda.device(x.device):
-        _lib.check(L.ptk_chamfer_fwd(_p(x), _p(y), B, P1, P2, None, _p(idx_x), None, _p(idx_y), _p(cham),
-                                     _p(ws), ws.numel(), _stream()), "ptk_chamfer_fwd")
+        _lib.check(L.ptk_chamfer_fwd_lengths(_p(x), _p(y), _p(lx), _p(ly), B, P1, P2, _lib.REDUCE_MEAN, None, _p(idx_x),
+                                             None, _p(idx_y), _p(cham), _p(ws), ws.numel(), _stream()),
+                   "ptk_chamfer_fwd_lengths")
         _lib.check(L.ptk_chamfer_rescued(_p(ws), B, P1, P2, C.byref(n), _stream()), "ptk_chamfer_rescued")
     return int(n.value)
 
 
 class _Chamfer(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, x, y):
+    def forward(ctx, x, y, lx, ly, reduction):
         _need_cuda(x, y)
         x, y = _f32c(x), _f32c(y)
-        if x.dim() != 3 or y.dim() != 3 or x.shape[2] != 3 or y.shape[2] != 3:
-            raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(x.shape)} and {tuple(y.shape)}")
-        if x.shape[0] != y.shape[0]:
-            raise ValueError("y must have the same batch dimension as x")
+        _check_pair(x, y)
         B, P1, _ = x.shape
         P2 = y.shape[1]
+        lx, ly = _lengths(lx, B, x.device, "x_lengths"), _lengths(ly, B, x.device, "y_lengths")
         L = _lib.lib()
         idx_x = torch.empty(B, P1, dtype=torch.int32, device=x.device)
         idx_y = torch.empty(B, P2, dtype=torch.int32, device=x.device)
@@ -84,46 +107,57 @@ class _Chamfer(torch.autograd.Function):
         nb = L.ptk_chamfer_workspace_bytes(B, P1, P2)
         ws = _ws(nb, x.device)
         with torch.cuda.device(x.device):
-            _lib.check(L.ptk_chamfer_fwd(_p(x), _p(y), B, P1, P2, None, _p(idx_x), None, _p(idx_y), _p(cham),
-                                         _p(ws), ws.numel(), _stream()), "ptk_chamfer_fwd")
-        ctx.save_for_backward(x, y, idx_x, idx_y)
+            _lib.check(L.ptk_chamfer_fwd_lengths(_p(x), _p(y), _p(lx), _p(ly), B, P1, P2, reduction, None, _p(idx_x),
+                                                 None, _p(idx_y), _p(cham), _p(ws), ws.numel(), _stream()),
+                       "ptk_chamfer_fwd_lengths")
+        ctx.save_for_backward(x, y, idx_x, idx_y, lx, ly)
+        ctx.reduction = reduction
         ctx.mark_non_differentiable(idx_x, idx_y)
         return cham, idx_x, idx_y
 
     @staticmethod
     def backward(ctx, g, _gi, _gj):
-        x, y, idx_x, idx_y = ctx.saved_tensors
+        x, y, idx_x, idx_y, lx, ly = ctx.saved_tensors
         B, P1, _ = x.shape
         P2 = y.shape[1]
         g = _f32c(g)
         gx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         gy = torch.empty_like(y) if ctx.needs_input_grad[1] else None
         with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().ptk_chamfer_bwd(_p(x), _p(y), _p(idx_x), _p(idx_y), _p(g), B, P1, P2, _p(gx),
-                                                  _p(gy), _stream()), "ptk_chamfer_bwd")
-        return gx, gy
+            _lib.check(_lib.lib().ptk_chamfer_bwd_lengths(_p(x), _p(y), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B,
+                                                          P1, P2, ctx.reduction, _p(gx), _p(gy), _stream()),
+                       "ptk_chamfer_bwd_lengths")
+        return gx, gy, None, None, None
 
 
-def chamfer(x, y):
-    """cham (B,), idx_x (B,P1) int32, idx_y (B,P2) int32.  Differentiable w.r.t. x and y."""
-    return _Chamfer.apply(x, y)
+def chamfer(x, y, x_lengths=None, y_lengths=None, point_reduction="mean"):
+    """cham (B,), idx_x (B,P1) int32, idx_y (B,P2) int32.  Differentiable w.r.t. x and y.
+
+    x_lengths / y_lengths (B,) int32 or int64, on any device: only x[b, :x_lengths[b]] and y[b, :y_lengths[b]] exist
+    (ragged batch, values clamped to [0, P]).  Padded rows get idx 0 and zero gradient; cham[b] is
+    sum_x / max(lx, 1) + sum_y / max(ly, 1) for point_reduction="mean", sum_x + sum_y for "sum" (include/ptk.h)."""
+    if point_reduction not in _REDUCTIONS:
+        raise ValueError('point_reduction must be one of ["mean", "sum"]')
+    return _Chamfer.apply(x, y, x_lengths, y_lengths, _REDUCTIONS[point_reduction])
 
 
-def knn1(p1, p2):
-    """dists (B,P1) f32, idx (B,P1) int32 -- forward only."""
+def knn1(p1, p2, lengths1=None, lengths2=None):
+    """dists (B,P1) f32, idx (B,P1) int32 -- forward only.  lengths1 / lengths2 as in chamfer(): padded queries and
+    queries whose target cloud is empty get dist 0, idx 0."""
     _need_cuda(p1, p2)
     p1, p2 = _f32c(p1), _f32c(p2)
     if p1.dim() != 3 or p2.dim() != 3 or p1.shape[2] != 3 or p2.shape[2] != 3 or p1.shape[0] != p2.shape[0]:
         raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(p1.shape)} and {tuple(p2.shape)}")
     B, P1, _ = p1.shape
     P2 = p2.shape[1]
+    l1, l2 = _lengths(lengths1, B, p1.device, "lengths1"), _lengths(lengths2, B, p1.device, "lengths2")
     L = _lib.lib()
     dist = torch.empty(B, P1, dtype=torch.float32, device=p1.device)
     idx = torch.empty(B, P1, dtype=torch.int32, device=p1.device)
     ws = _ws(L.ptk_chamfer_workspace_bytes(B, P1, P2), p1.device)
     with torch.cuda.device(p1.device):
-        _lib.check(L.ptk_knn1_fwd(_p(p1), _p(p2), B, P1, P2, _p(dist), _p(idx), _p(ws), ws.numel(), _stream()),
-                   "ptk_knn1_fwd")
+        _lib.check(L.ptk_knn1_fwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), B, P1, P2, _p(dist), _p(idx), _p(ws),
+                                          ws.numel(), _stream()), "ptk_knn1_fwd_lengths")
     return dist, idx
 
 

@@ -98,6 +98,37 @@ int ptk_chamfer_bwd(const float *x, const float *y, const int32_t *idx_x, const 
                     const float *grad_cham, int64_t B, int64_t P1, int64_t P2, float *grad_x,
                     float *grad_y, ptk_stream_t stream);
 
+/* Ragged batches: clouds of different sizes padded to (B,P1,3) / (B,P2,3), as PyTorch3D batches them.
+ *   len_x / len_y (resp. len1 / len2) are DEVICE int64 arrays of B lengths; NULL means every cloud is full.  Each
+ *   value is clamped to [0, P] on the device; the host never reads them, so a call needs no synchronisation and can
+ *   be captured in a CUDA graph with the lengths changed in place between replays.  For pair b only x[b, :lx] and
+ *   y[b, :ly] exist: padding is never read into a result, whatever it holds.
+ *   - valid queries: dist / idx bit-identical to a homogeneous call on the sliced pair (same arithmetic, same
+ *     lowest-index tie rule), and so is cham[b];
+ *   - padded queries (i >= len) and valid queries whose target cloud is empty: dist = 0, idx = 0 (PyTorch3D's zero
+ *     fill);
+ *   - reduction PTK_REDUCE_MEAN: cham[b] = sum_x / max(lx, 1) + sum_y / max(ly, 1).  An empty cloud contributes 0
+ *     (the divisor is clamped to 1, as current PyTorch3D releases clamp their lengths; 0.5.0's behaviour for a zero
+ *     length is not pinned here).  PTK_REDUCE_SUM: cham[b] = sum_x + sum_y.  Any other value is PTK_ERR_SHAPE;
+ *   - backward: the valid points of pair b get the gradient of its own term (scale 1 / max(len, 1) for mean, 1 for
+ *     sum); padded points get exactly 0 and queries with an empty target cloud contribute nothing.  grad_* are
+ *     fully overwritten.
+ * The workspace is ptk_chamfer_workspace_bytes(B, P1, P2) and ptk_chamfer_rescued works after these calls.  The
+ * homogeneous entry points above are these calls with NULL lengths and PTK_REDUCE_MEAN.
+ * Replace pytorch3d.loss.chamfer_distance(x, y, x_lengths, y_lengths, point_reduction=...) and
+ * pytorch3d.ops.knn_points(p1, p2, lengths1, lengths2, K=1) of PyTorch3D 0.5.0. */
+#define PTK_REDUCE_MEAN 0
+#define PTK_REDUCE_SUM 1
+int ptk_chamfer_fwd_lengths(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y, int64_t B,
+                            int64_t P1, int64_t P2, int reduction, float *dist_x, int32_t *idx_x, float *dist_y,
+                            int32_t *idx_y, float *cham, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+int ptk_chamfer_bwd_lengths(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y,
+                            const int32_t *idx_x, const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1,
+                            int64_t P2, int reduction, float *grad_x, float *grad_y, ptk_stream_t stream);
+int ptk_knn1_fwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, int64_t B,
+                         int64_t P1, int64_t P2, float *dist, int32_t *idx, void *workspace, size_t workspace_bytes,
+                         ptk_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Area-weighted surface sampling.  Replaces the body of utils.batch_sample
  * (pterotactyl/utility/utils.py:152-187): pytorch3d mesh_face_areas_normals (utils.py:164), the NaN

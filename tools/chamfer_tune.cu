@@ -81,7 +81,7 @@ void run_exact2(const char *name, const float *x, const float *y, int B, int P, 
     int split_len = ((P + CHUNK - 1) / CHUNK) * CHUNK;
     cudaEvent_t a, b;
     CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b));
-    auto launch = [&]() { chamfer_nn_exact2_kernel<R, CHUNK, THREADS, MINB><<<grid, THREADS>>>(x, y, P, P, split_len, 1, kx, ky, -1, nullptr, nullptr, nullptr); };
+    auto launch = [&]() { chamfer_nn_exact2_kernel<R, CHUNK, THREADS, MINB><<<grid, THREADS>>>(x, y, P, P, nullptr, nullptr, split_len, 1, kx, ky, -1, nullptr, nullptr, nullptr); };
     launch(); launch();
     CK(cudaDeviceSynchronize());
     CK(cudaEventRecord(a));
@@ -120,9 +120,9 @@ void run_filter(const char *name, const float *x, const float *y, int B, int P, 
     if (!rescue) { CK(cudaMalloc(&rescue, 8 * (size_t)B * P)); CK(cudaMalloc(&rcount, 8 * (size_t)B)); }
     dim3 rgrid((P + 128 * 8 - 1) / (128 * 8), 1, B * 2);
     auto launch = [&](unsigned int *) {
-        chamfer_bounds_kernel<<<B, 1024>>>(x, y, P, P, aux, rcount);
+        chamfer_bounds_kernel<<<B, 1024>>>(x, y, P, P, nullptr, nullptr, aux, rcount);
         chamfer_nn_filter_kernel<R, CHUNK, THREADS, MINB, TT, PK><<<grid, THREADS>>>(x, y, P, P, split_len, 1, aux, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount, nullptr, nullptr);
-        chamfer_nn_exact2_kernel<8, 16, 128, 3><<<rgrid, 128>>>(x, y, P, P, split_len, 1, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount);
+        chamfer_nn_exact2_kernel<8, 16, 128, 3><<<rgrid, 128>>>(x, y, P, P, nullptr, nullptr, split_len, 1, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount);
     };
     launch(nullptr);
     CK(cudaDeviceSynchronize());
@@ -173,10 +173,10 @@ void run_tma(const char *name, const float *x, const float *y, int B, int P, uns
     dim3 rgrid((P + 128 * 8 - 1) / (128 * 8), 1, B * 2);
     dim3 pgrid((Pp + 255) / 256, 2 * B);
     auto launch = [&]() {
-        chamfer_bounds_kernel<<<B, 1024>>>(x, y, P, P, aux, rcount);
-        chamfer_prep_kernel<<<pgrid, 256>>>(x, y, P, P, aux, soa_x, soa_y, nullptr, nullptr, nullptr, nullptr, 0);
-        chamfer_nn_filter_tma_kernel<R, CHUNK, THREADS, MINB, TT><<<grid, THREADS>>>(x, y, P, P, split_len, 1, aux, soa_x, soa_y, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount, nullptr, nullptr);
-        chamfer_nn_exact2_kernel<8, 16, 128, 3><<<rgrid, 128>>>(x, y, P, P, split_len, 1, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount);
+        chamfer_bounds_kernel<<<B, 1024>>>(x, y, P, P, nullptr, nullptr, aux, rcount);
+        chamfer_prep_kernel<<<pgrid, 256>>>(x, y, P, P, nullptr, nullptr, aux, soa_x, soa_y, nullptr, nullptr, nullptr, nullptr, 0);
+        chamfer_nn_filter_tma_kernel<R, CHUNK, THREADS, MINB, TT><<<grid, THREADS>>>(x, y, P, P, nullptr, nullptr, split_len, 1, aux, soa_x, soa_y, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount, nullptr, nullptr);
+        chamfer_nn_exact2_kernel<8, 16, 128, 3><<<rgrid, 128>>>(x, y, P, P, nullptr, nullptr, split_len, 1, kx, ky, -1, rescue, rescue + (size_t)B * P, rcount);
     };
     launch();
     CK(cudaDeviceSynchronize());
