@@ -40,9 +40,13 @@ SIGNATURES = {
                                           _vp]),
     "ptk_chamfer_bwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp]),
     "ptk_knn1_fwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
+    "ptk_chamfer_bwd_det_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "ptk_chamfer_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _sz, _vp]),
     "ptk_sample_workspace_bytes": (_sz, [_i64, _i64]),
     "ptk_sample_fwd": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_sample_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp]),
+    "ptk_sample_bwd_det_workspace_bytes": (_sz, [_i64, _i64]),
+    "ptk_sample_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _sz, _vp]),
     "ptk_face_areas_normals": (C.c_int, [_vp, _i64, _vp, _i64, _vp, _vp, _vp]),
     "ptk_mesh_face_areas": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp]),
     "ptk_gcn_aggregate": (C.c_int, [_vp, _vp, _vp, _vp, _i32, _i64, _vp, _i64, _i64, _i64, _vp, C.c_int, _vp, _vp]),
@@ -82,6 +86,9 @@ SIGNATURES = {
                                        _vp, _sz, _vp]),
     "ptk_mesh_chamfer_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp, _vp,
                                        _vp, _sz, _vp]),
+    "ptk_mesh_chamfer_bwd_det_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64, _i64]),
+    "ptk_mesh_chamfer_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _vp,
+                                           _vp, _vp, _sz, _vp]),
     "ptk_host_ctx_create": (_vp, [C.c_int]),
     "ptk_host_ctx_destroy": (None, [_vp]),
     "ptk_host_chamfer": (C.c_int, [_vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),

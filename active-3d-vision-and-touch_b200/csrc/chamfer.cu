@@ -38,6 +38,7 @@
 
 #include "chamfer_kernel2.cuh"
 #include "chamfer_pruned.cuh"
+#include "det_accum.cuh"
 
 namespace ptk {
 
@@ -292,6 +293,121 @@ __global__ void chamfer_bwd_scatter_kernel(const float *__restrict__ x, const fl
         atomicAdd(o + 0, -(s * (yb[i * 3 + 0] - xb[j * 3 + 0])));
         atomicAdd(o + 1, -(s * (yb[i * 3 + 1] - xb[j * 3 + 1])));
         atomicAdd(o + 2, -(s * (yb[i * 3 + 2] - xb[j * 3 + 2])));
+    }
+}
+
+// Deterministic backward (ptk_chamfer_bwd_det, scheme in det_accum.cuh): three kernels, grid = (ceil(max(P1,P2) / 256), B).
+// Thread i owns x-query i and y-query i.  A valid query's own term is s * (q - t[idx]) per component, with s and the
+// arithmetic of chamfer_bwd_direct_kernel; it goes to the query's row and, negated, to its nearest neighbour's row.
+// M_b and the scatter into one cloud always take the terms of both directions, so each gradient has the same bits
+// whether or not the other one is requested.  A row of x receives at most ly + 1 terms, a row of y lx + 1.
+constexpr int CD_THREADS = 256;
+
+// the three components of query i's own term (dir 0: x-query against y, dir 1: y-query against x); false: no term
+__device__ __forceinline__ bool chamfer_own_term(const float *__restrict__ qb, const float *__restrict__ tb,
+                                                 const int32_t *__restrict__ idx, float g, int i, int Lq, int Lt,
+                                                 int mean, int &j, float t[3]) {
+    if (i >= Lq || Lt <= 0) return false;
+    j = idx[i];
+    const float s = mean ? 2.0f * (g / (float)Lq) : 2.0f * g;
+    t[0] = s * (qb[i * 3 + 0] - tb[j * 3 + 0]);
+    t[1] = s * (qb[i * 3 + 1] - tb[j * 3 + 1]);
+    t[2] = s * (qb[i * 3 + 2] - tb[j * 3 + 2]);
+    return true;
+}
+
+// phase 1: M_b (atomicMax into mbits[b], zeroed by the caller); zero the accumulators and the outputs of every row
+__global__ void __launch_bounds__(CD_THREADS)
+chamfer_bwd_det_terms_kernel(const float *__restrict__ x, const float *__restrict__ y, const int32_t *__restrict__ idx_x,
+                             const int32_t *__restrict__ idx_y, const float *__restrict__ grad_cham, int P1, int P2,
+                             const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
+                             float *__restrict__ grad_x, float *__restrict__ grad_y, unsigned long long *__restrict__ acc_x,
+                             unsigned long long *__restrict__ acc_y, unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const float g = grad_cham[b];
+    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    float m = 0.0f, t[3];
+    int j;
+    if (chamfer_own_term(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, t))
+        m = fmaxf(m, fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2]))));
+    if (chamfer_own_term(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, t))
+        m = fmaxf(m, fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2]))));
+    if (grad_x && i < P1) {
+        const size_t r = ((size_t)b * P1 + i) * 3;
+        acc_x[r + 0] = acc_x[r + 1] = acc_x[r + 2] = 0ull;
+        grad_x[r + 0] = grad_x[r + 1] = grad_x[r + 2] = 0.0f;
+    }
+    if (grad_y && i < P2) {
+        const size_t r = ((size_t)b * P2 + i) * 3;
+        acc_y[r + 0] = acc_y[r + 1] = acc_y[r + 2] = 0ull;
+        grad_y[r + 0] = grad_y[r + 1] = grad_y[r + 2] = 0.0f;
+    }
+    det_block_max<CD_THREADS>(m, mbits + b);
+}
+
+// the own term of one query into its row (acc_q / out_q) and, negated, into its neighbour's row (acc_t / out_t)
+__device__ __forceinline__ void chamfer_det_add(const float t[3], double scale, unsigned long long *acc_q, float *out_q,
+                                                unsigned long long *acc_t, float *out_t) {
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        if (isfinite(t[d])) {
+            const unsigned long long q = det_quantise(t[d], scale);
+            if (acc_q) atomicAdd(acc_q + d, q);
+            if (acc_t) atomicAdd(acc_t + d, 0ull - q);
+        } else {
+            if (out_q) atomicAdd(out_q + d, t[d]);
+            if (out_t) atomicAdd(out_t + d, -t[d]);
+        }
+    }
+}
+
+// phase 2: quantise and add (64-bit reductions; non-finite terms into the outputs)
+__global__ void __launch_bounds__(CD_THREADS)
+chamfer_bwd_det_reduce_kernel(const float *__restrict__ x, const float *__restrict__ y, const int32_t *__restrict__ idx_x,
+                              const int32_t *__restrict__ idx_y, const float *__restrict__ grad_cham, int P1, int P2,
+                              const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
+                              float *__restrict__ grad_x, float *__restrict__ grad_y,
+                              unsigned long long *__restrict__ acc_x, unsigned long long *__restrict__ acc_y,
+                              const unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const float g = grad_cham[b];
+    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)max(L1, L2) + 1));
+    const size_t bx = (size_t)b * P1 * 3, by = (size_t)b * P2 * 3;
+    float t[3];
+    int j;
+    if (chamfer_own_term(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, t))
+        chamfer_det_add(t, scale, acc_x ? acc_x + bx + (size_t)i * 3 : nullptr, grad_x ? grad_x + bx + (size_t)i * 3 : nullptr,
+                        acc_y ? acc_y + by + (size_t)j * 3 : nullptr, grad_y ? grad_y + by + (size_t)j * 3 : nullptr);
+    if (chamfer_own_term(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, t))
+        chamfer_det_add(t, scale, acc_y ? acc_y + by + (size_t)i * 3 : nullptr, grad_y ? grad_y + by + (size_t)i * 3 : nullptr,
+                        acc_x ? acc_x + bx + (size_t)j * 3 : nullptr, grad_x ? grad_x + bx + (size_t)j * 3 : nullptr);
+}
+
+// phase 3: grad = fp32(acc) * 2^-e_b, unless the row's output already holds a non-finite sum
+__global__ void __launch_bounds__(CD_THREADS)
+chamfer_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
+                               const unsigned int *__restrict__ mbits, const unsigned long long *__restrict__ acc_x,
+                               const unsigned long long *__restrict__ acc_y, float *__restrict__ grad_x,
+                               float *__restrict__ grad_y) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
+    const int e = det_exponent(mbits[b], (long long)max(L1, L2) + 1);
+    if (grad_x && i < P1) {
+        const size_t r = ((size_t)b * P1 + i) * 3;
+        for (int d = 0; d < 3; ++d) det_convert(grad_x + r + d, acc_x + r + d, e);
+    }
+    if (grad_y && i < P2) {
+        const size_t r = ((size_t)b * P2 + i) * 3;
+        for (int d = 0; d < 3; ++d) det_convert(grad_y + r + d, acc_y + r + d, e);
     }
 }
 
@@ -687,4 +803,51 @@ extern "C" int ptk_chamfer_bwd_lengths(const float *x, const float *y, const int
                                        ptk_stream_t stream) {
     PTK_NVTX("ptk_chamfer_bwd_lengths");
     return chamfer_bwd(x, y, len_x, len_y, idx_x, idx_y, grad_cham, B, P1, P2, reduction, grad_x, grad_y, stream);
+}
+
+// det workspace: [M_b bits B, padded to 256 bytes][acc_x B*P1*3 int64][acc_y B*P2*3 int64]
+static size_t det_align(size_t b) { return (b + 255) & ~(size_t)255; }
+
+extern "C" size_t ptk_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
+    if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;
+    return det_align(4 * (size_t)B) + det_align(24 * (size_t)B * P1) + 24 * (size_t)B * P2;
+}
+
+extern "C" int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y,
+                                   const int32_t *idx_x, const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1,
+                                   int64_t P2, int reduction, float *grad_x, float *grad_y, void *workspace,
+                                   size_t workspace_bytes, ptk_stream_t stream) {
+    PTK_NVTX("ptk_chamfer_bwd_det");
+    int rc = check_clouds(x, y, B, P1, P2);
+    if (rc) return rc;
+    rc = check_reduction(reduction);
+    if (rc) return rc;
+    PTK_REQUIRE(idx_x && idx_y && grad_cham, PTK_ERR_SHAPE, "chamfer_bwd_det: null index / grad pointer");
+    if (!grad_x && !grad_y) return PTK_OK;
+    const size_t need = ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2);
+    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "chamfer_bwd_det: workspace too small (%zu < %zu)",
+                workspace_bytes, need);
+    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
+                "chamfer_bwd_det: workspace must be 16-byte aligned");
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "chamfer_bwd_det: batch too large");
+    char *p = reinterpret_cast<char *>(workspace);
+    auto *mbits = reinterpret_cast<unsigned int *>(p);
+    auto *acc_x = grad_x ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B)) : nullptr;
+    auto *acc_y = grad_y ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B) + det_align(24 * (size_t)B * P1))
+                         : nullptr;
+    cudaStream_t st = as_stream(stream);
+    const int64_t Pm = P1 > P2 ? P1 : P2;
+    const dim3 grid((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B);
+    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
+    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
+    launch_pdl(chamfer_bwd_det_terms_kernel, grid, dim3(CD_THREADS), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2,
+               len_x, len_y, mean, grad_x, grad_y, acc_x, acc_y, mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(chamfer_bwd_det_reduce_kernel, grid, dim3(CD_THREADS), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2,
+               len_x, len_y, mean, grad_x, grad_y, acc_x, acc_y, (const unsigned int *)mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(chamfer_bwd_det_convert_kernel, grid, dim3(CD_THREADS), 0, st, (int)P1, (int)P2, len_x, len_y,
+               (const unsigned int *)mbits, (const unsigned long long *)acc_x, (const unsigned long long *)acc_y, grad_x, grad_y);
+    PTK_CHECK_LAUNCH();
+    return PTK_OK;
 }

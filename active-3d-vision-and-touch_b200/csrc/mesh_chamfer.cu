@@ -6,7 +6,8 @@
 // (ptk_chamfer_bwd -> ptk_sample_bwd) accumulated into one vertex gradient (and, for the autoencoder, one gradient of
 // the second cloud, autoencoder/train.py:145-150).  The kernels are the ones behind the separate entry points (same
 // results); what goes away is the host frame between them: one autograd node instead of 2 x repeat + 2, no
-// intermediate torch tensors.  The host-buffer twin is ptk_host_mesh_chamfer (host_api.cu).
+// intermediate torch tensors.  The host-buffer twin is ptk_host_mesh_chamfer (host_api.cu).  ptk_mesh_chamfer_bwd_det
+// runs the same loop on the deterministic backward pieces (ptk_chamfer_bwd_det -> ptk_sample_bwd_det).
 #include "ptk_common.cuh"
 
 namespace ptk {
@@ -89,19 +90,23 @@ extern "C" int ptk_mesh_chamfer_fwd(const float *verts, int64_t B, int64_t V, co
     return PTK_OK;
 }
 
-extern "C" int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int32_t *face_idx, const int32_t *idx_x,
-                                    const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd,
-                                    int64_t B, int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat,
-                                    float *grad_verts, float *grad_gt, void *workspace, size_t workspace_bytes,
-                                    ptk_stream_t stream) {
-    PTK_NVTX("ptk_mesh_chamfer_bwd");
-    PTK_REQUIRE(gt && pts && face_idx && idx_x && idx_y && uv && faces && grad_cd, PTK_ERR_SHAPE, "mesh_chamfer_bwd: null pointer");
-    PTK_REQUIRE(B > 0 && V > 0 && F > 0 && P2 > 0 && S > 0 && repeat > 0, PTK_ERR_SHAPE, "mesh_chamfer_bwd: empty input");
+// det: the deterministic pieces (ptk_chamfer_bwd_det, ptk_sample_bwd_det), whose workspaces follow the default layout
+static int mesh_chamfer_bwd(const float *gt, const float *pts, const int32_t *face_idx, const int32_t *idx_x,
+                            const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd, int64_t B,
+                            int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat, float *grad_verts, float *grad_gt,
+                            void *workspace, size_t workspace_bytes, bool det, ptk_stream_t stream) {
+    const char *name = det ? "mesh_chamfer_bwd_det" : "mesh_chamfer_bwd";
+    PTK_REQUIRE(gt && pts && face_idx && idx_x && idx_y && uv && faces && grad_cd, PTK_ERR_SHAPE, "%s: null pointer", name);
+    PTK_REQUIRE(B > 0 && V > 0 && F > 0 && P2 > 0 && S > 0 && repeat > 0, PTK_ERR_SHAPE, "%s: empty input", name);
     if (!grad_verts && !grad_gt) return PTK_OK;
-    PTK_REQUIRE(workspace && workspace_bytes >= ptk_mesh_chamfer_workspace_bytes(B, V, F, S, P2), PTK_ERR_WORKSPACE,
-                "mesh_chamfer_bwd: workspace too small");
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, PTK_ERR_ALIGN, "mesh_chamfer_bwd: workspace must be 256-byte aligned");
+    const size_t need = det ? ptk_mesh_chamfer_bwd_det_workspace_bytes(B, V, F, S, P2) : ptk_mesh_chamfer_workspace_bytes(B, V, F, S, P2);
+    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "%s: workspace too small", name);
+    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, PTK_ERR_ALIGN, "%s: workspace must be 256-byte aligned", name);
     const McWs w = mc_carve(workspace, B, V, F, S, P2);
+    char *det_c = reinterpret_cast<char *>(workspace) + w.total;
+    const size_t det_c_bytes = ptk_chamfer_bwd_det_workspace_bytes(B, S, P2);
+    char *det_s = det_c + mc_align(det_c_bytes);
+    const size_t det_s_bytes = ptk_sample_bwd_det_workspace_bytes(B, V);
     cudaStream_t st = as_stream(stream);
     const size_t ns = (size_t)B * S, ny = (size_t)B * P2;
     const long long nv = (long long)B * V * 3, ng = (long long)ny * 3;
@@ -110,8 +115,11 @@ extern "C" int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int
     PTK_CHECK_LAUNCH();
     for (int64_t r = 0; r < repeat; ++r) {
         float *gy_dst = grad_gt ? (r == 0 ? grad_gt : w.gy) : nullptr;
-        int rc = ptk_chamfer_bwd(pts + r * ns * 3, gt, idx_x + r * ns, idx_y + r * ny, w.gc, B, S, P2,
-                                 grad_verts ? w.gx : nullptr, gy_dst, stream);
+        float *gx_dst = grad_verts ? w.gx : nullptr;
+        int rc = det ? ptk_chamfer_bwd_det(pts + r * ns * 3, gt, nullptr, nullptr, idx_x + r * ns, idx_y + r * ny, w.gc, B, S,
+                                           P2, PTK_REDUCE_MEAN, gx_dst, gy_dst, det_c, det_c_bytes, stream)
+                     : ptk_chamfer_bwd(pts + r * ns * 3, gt, idx_x + r * ns, idx_y + r * ny, w.gc, B, S, P2, gx_dst, gy_dst,
+                                       stream);
         if (rc) return rc;
         if (grad_gt && r > 0) {
             launch_pdl(mc_accumulate_kernel, dim3((unsigned)ceil_div(ng, 256)), dim3(256), 0, st, grad_gt, (const float *)w.gy, ng, 0, 1.0f);
@@ -119,7 +127,9 @@ extern "C" int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int
         }
         if (grad_verts) {
             float *gv_dst = r == 0 ? grad_verts : w.gv;
-            rc = ptk_sample_bwd(w.gx, face_idx + r * ns, uv + r * 2 * ns, faces, B, V, F, S, gv_dst, stream);
+            rc = det ? ptk_sample_bwd_det(w.gx, face_idx + r * ns, uv + r * 2 * ns, faces, B, V, F, S, gv_dst, det_s, det_s_bytes,
+                                          stream)
+                     : ptk_sample_bwd(w.gx, face_idx + r * ns, uv + r * 2 * ns, faces, B, V, F, S, gv_dst, stream);
             if (rc) return rc;
             if (r > 0) {
                 launch_pdl(mc_accumulate_kernel, dim3((unsigned)ceil_div(nv, 256)), dim3(256), 0, st, grad_verts, (const float *)w.gv, nv, 0, 1.0f);
@@ -128,4 +138,31 @@ extern "C" int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int
         }
     }
     return PTK_OK;
+}
+
+extern "C" int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int32_t *face_idx, const int32_t *idx_x,
+                                    const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd,
+                                    int64_t B, int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat,
+                                    float *grad_verts, float *grad_gt, void *workspace, size_t workspace_bytes,
+                                    ptk_stream_t stream) {
+    PTK_NVTX("ptk_mesh_chamfer_bwd");
+    return mesh_chamfer_bwd(gt, pts, face_idx, idx_x, idx_y, uv, faces, grad_cd, B, V, F, S, P2, repeat, grad_verts, grad_gt,
+                            workspace, workspace_bytes, false, stream);
+}
+
+// the default workspace followed by those of ptk_chamfer_bwd_det (B, S, P2) and ptk_sample_bwd_det (B, V)
+extern "C" size_t ptk_mesh_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t V, int64_t F, int64_t S, int64_t P2) {
+    if (B <= 0 || V <= 0 || F <= 0 || S <= 0 || P2 <= 0) return 0;
+    return mc_carve(nullptr, B, V, F, S, P2).total + mc_align(ptk_chamfer_bwd_det_workspace_bytes(B, S, P2)) +
+           mc_align(ptk_sample_bwd_det_workspace_bytes(B, V));
+}
+
+extern "C" int ptk_mesh_chamfer_bwd_det(const float *gt, const float *pts, const int32_t *face_idx, const int32_t *idx_x,
+                                        const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd,
+                                        int64_t B, int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat,
+                                        float *grad_verts, float *grad_gt, void *workspace, size_t workspace_bytes,
+                                        ptk_stream_t stream) {
+    PTK_NVTX("ptk_mesh_chamfer_bwd_det");
+    return mesh_chamfer_bwd(gt, pts, face_idx, idx_x, idx_y, uv, faces, grad_cd, B, V, F, S, P2, repeat, grad_verts, grad_gt,
+                            workspace, workspace_bytes, true, stream);
 }

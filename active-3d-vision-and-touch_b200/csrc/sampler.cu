@@ -11,7 +11,7 @@
 //                           individually rounded ops in the reference's order.
 // The arithmetic is defined in oracle/ptk_oracle.c (orc_face_cumweights / orc_sample_fwd); this file
 // must match it bit for bit.
-#include "ptk_common.cuh"
+#include "det_accum.cuh"
 
 namespace ptk {
 
@@ -207,6 +207,110 @@ sample_bwd_kernel(const float *__restrict__ grad_pts, const int32_t *__restrict_
     }
 }
 
+// Deterministic backward (ptk_sample_bwd_det, scheme in det_accum.cuh).  The terms are c = w_k * g_d with the
+// arithmetic of sample_bwd_kernel; a vertex receives at most 3 S of them (a degenerate face may list it twice).
+// phase 1, grid = (ceil(max(S, V) / SP_THREADS), B): M_b (atomicMax into mbits[b], zeroed by the caller); zero the
+// accumulators and grad_verts
+__device__ __forceinline__ void sample_det_weights(const float *__restrict__ uu, const float *__restrict__ vv, size_t o,
+                                                   float w[3]) {
+    const float rt = __fsqrt_rn(uu[o]);
+    const float v = vv[o];
+    w[0] = __fsub_rn(1.0f, rt);
+    w[1] = __fmul_rn(rt, __fsub_rn(1.0f, v));
+    w[2] = __fmul_rn(rt, v);
+}
+
+__global__ void __launch_bounds__(SP_THREADS)
+sample_bwd_det_terms_kernel(const float *__restrict__ grad_pts, const float *__restrict__ uu, const float *__restrict__ vv,
+                            int V, int S, float *__restrict__ grad_verts, unsigned long long *__restrict__ acc,
+                            unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * SP_THREADS + threadIdx.x;
+    float m = 0.0f;
+    if (i < S) {
+        const size_t o = (size_t)b * S + i;
+        float w[3];
+        sample_det_weights(uu, vv, o, w);
+#pragma unroll
+        for (int k = 0; k < 3; ++k)
+#pragma unroll
+            for (int d = 0; d < 3; ++d) m = fmaxf(m, det_abs_finite(__fmul_rn(w[k], grad_pts[o * 3 + d])));
+    }
+    if (i < V) {
+        const size_t r = ((size_t)b * V + i) * 3;
+        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
+        grad_verts[r + 0] = grad_verts[r + 1] = grad_verts[r + 2] = 0.0f;
+    }
+    det_block_max<SP_THREADS>(m, mbits + b);
+}
+
+// phase 2, grid = (ceil(S / samples_per_cta), B): quantise and add.  Meshes of up to SBD_SMEM_VERTS vertices are
+// accumulated in shared memory first (exact as well), then one global 64-bit reduction per touched component.
+constexpr int SBD_SMEM_VERTS = 2048;  // 2048 * 3 int64 = 48 KB
+
+__global__ void __launch_bounds__(SP_THREADS)
+sample_bwd_det_reduce_kernel(const float *__restrict__ grad_pts, const int32_t *__restrict__ face_idx,
+                             const float *__restrict__ uu, const float *__restrict__ vv, const int32_t *__restrict__ faces,
+                             int V, int S, int samples_per_cta, float *__restrict__ grad_verts,
+                             unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int tid = threadIdx.x;
+    __shared__ unsigned long long s_acc[SBD_SMEM_VERTS * 3];
+    const bool in_smem = V <= SBD_SMEM_VERTS;
+    if (in_smem) {
+        for (int k = tid; k < V * 3; k += SP_THREADS) s_acc[k] = 0ull;
+        __syncthreads();
+    }
+    const double scale = ldexp(1.0, det_exponent(mbits[b], 3LL * S + 1));
+    float *gv = grad_verts + (size_t)b * V * 3;
+    unsigned long long *av = acc + (size_t)b * V * 3;
+    const int s_begin = blockIdx.x * samples_per_cta;
+    const int s_end = min(S, s_begin + samples_per_cta);
+    for (int s = s_begin + tid; s < s_end; s += SP_THREADS) {
+        const size_t o = (size_t)b * S + s;
+        const int f = face_idx[o];
+        float w[3];
+        sample_det_weights(uu, vv, o, w);
+        const float g[3] = {grad_pts[o * 3 + 0], grad_pts[o * 3 + 1], grad_pts[o * 3 + 2]};
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const int vi = faces[f * 3 + k];
+#pragma unroll
+            for (int d = 0; d < 3; ++d) {
+                const float c = __fmul_rn(w[k], g[d]);
+                if (!isfinite(c))
+                    atomicAdd(&gv[(size_t)vi * 3 + d], c);
+                else if (in_smem)
+                    atomicAdd(&s_acc[vi * 3 + d], det_quantise(c, scale));
+                else
+                    atomicAdd(&av[(size_t)vi * 3 + d], det_quantise(c, scale));
+            }
+        }
+    }
+    if (in_smem) {
+        __syncthreads();
+        for (int k = tid; k < V * 3; k += SP_THREADS) {
+            const unsigned long long a = s_acc[k];
+            if (a != 0ull) atomicAdd(&av[k], a);
+        }
+    }
+}
+
+// phase 3, grid = (ceil(V / SP_THREADS), B)
+__global__ void __launch_bounds__(SP_THREADS)
+sample_bwd_det_convert_kernel(int V, int S, const unsigned int *__restrict__ mbits,
+                              const unsigned long long *__restrict__ acc, float *__restrict__ grad_verts) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * SP_THREADS + threadIdx.x;
+    if (i >= V) return;
+    const int e = det_exponent(mbits[b], 3LL * S + 1);
+    const size_t r = ((size_t)b * V + i) * 3;
+    for (int d = 0; d < 3; ++d) det_convert(grad_verts + r + d, acc + r + d, e);
+}
+
 // pytorch3d.ops.mesh_face_areas_normals drop-in (packed verts (V,3), int64 faces (F,3)): areas (F) and
 // unit normals (F,3) with the 1e-6 clamp of PyTorch3D's face_areas_normals kernel.
 __global__ void face_areas_normals_kernel(const float *__restrict__ verts, const long long *__restrict__ faces,
@@ -314,6 +418,44 @@ extern "C" int ptk_sample_bwd(const float *grad_pts, const int32_t *face_idx, co
     dim3 grid((unsigned)ceil_div(S, per_cta), (unsigned)B);
     launch_pdl(sample_bwd_kernel, grid, dim3(SP_THREADS), 0, st, grad_pts, face_idx, uv, uv + (size_t)B * S, faces, (int)V,
                (int)S, per_cta, grad_verts);
+    PTK_CHECK_LAUNCH();
+    return PTK_OK;
+}
+
+// det workspace: [M_b bits B, padded to 256 bytes][acc B*V*3 int64]
+static size_t sbd_mbits_bytes(int64_t B) { return (4 * (size_t)B + 255) & ~(size_t)255; }
+
+extern "C" size_t ptk_sample_bwd_det_workspace_bytes(int64_t B, int64_t V) {
+    if (B <= 0 || V <= 0) return 0;
+    return sbd_mbits_bytes(B) + 24 * (size_t)B * (size_t)V;
+}
+
+extern "C" int ptk_sample_bwd_det(const float *grad_pts, const int32_t *face_idx, const float *uv, const int32_t *faces,
+                                  int64_t B, int64_t V, int64_t F, int64_t S, float *grad_verts, void *workspace,
+                                  size_t workspace_bytes, ptk_stream_t stream) {
+    PTK_NVTX("ptk_sample_bwd_det");
+    PTK_REQUIRE(grad_pts && face_idx && uv && faces && grad_verts, PTK_ERR_SHAPE, "sample_bwd_det: null pointer");
+    PTK_REQUIRE(B > 0 && V > 0 && F > 0 && S > 0 && B <= 65535 && V < (1 << 28) && S < (1 << 28), PTK_ERR_SHAPE,
+                "sample_bwd_det: bad sizes");
+    const size_t need = ptk_sample_bwd_det_workspace_bytes(B, V);
+    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "sample_bwd_det: workspace too small (%zu < %zu)",
+                workspace_bytes, need);
+    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
+                "sample_bwd_det: workspace must be 16-byte aligned");
+    auto *mbits = reinterpret_cast<unsigned int *>(workspace);
+    auto *acc = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(workspace) + sbd_mbits_bytes(B));
+    cudaStream_t st = as_stream(stream);
+    const float *uu = uv, *vv = uv + (size_t)B * S;
+    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
+    launch_pdl(sample_bwd_det_terms_kernel, dim3((unsigned)ceil_div(S > V ? S : V, SP_THREADS), (unsigned)B), dim3(SP_THREADS),
+               0, st, grad_pts, uu, vv, (int)V, (int)S, grad_verts, acc, mbits);
+    PTK_CHECK_LAUNCH();
+    const int per_cta = 2048;
+    launch_pdl(sample_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(S, per_cta), (unsigned)B), dim3(SP_THREADS), 0, st,
+               grad_pts, face_idx, uu, vv, faces, (int)V, (int)S, per_cta, grad_verts, acc, (const unsigned int *)mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(sample_bwd_det_convert_kernel, dim3((unsigned)ceil_div(V, SP_THREADS), (unsigned)B), dim3(SP_THREADS), 0, st,
+               (int)V, (int)S, (const unsigned int *)mbits, (const unsigned long long *)acc, grad_verts);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }

@@ -36,6 +36,13 @@ def _ws(nbytes, device):
     return torch.empty(max(int(nbytes), 16), dtype=torch.uint8, device=device)
 
 
+def _deterministic():
+    """torch.use_deterministic_algorithms(True) selects the deterministic backward kernels (ptk_*_bwd_det: exact
+    fixed-point sums instead of fp32 atomics, include/ptk.h).  Read when the backward runs -- for a captured CUDA graph,
+    at capture."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
 # ------------------------------------------------------------------------------------- Chamfer / KNN
 def set_chamfer_algo(name):
     """'filter' (3-FFMA expansion filter + exact recheck), 'exact' (6-op scan), 'pruned' (cell-sorted clouds + box
@@ -123,10 +130,17 @@ class _Chamfer(torch.autograd.Function):
         g = _f32c(g)
         gx = torch.empty_like(x) if ctx.needs_input_grad[0] else None
         gy = torch.empty_like(y) if ctx.needs_input_grad[1] else None
+        L = _lib.lib()
         with torch.cuda.device(x.device):
-            _lib.check(_lib.lib().ptk_chamfer_bwd_lengths(_p(x), _p(y), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B,
-                                                          P1, P2, ctx.reduction, _p(gx), _p(gy), _stream()),
-                       "ptk_chamfer_bwd_lengths")
+            if _deterministic():
+                ws = _ws(L.ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2), x.device)
+                _lib.check(L.ptk_chamfer_bwd_det(_p(x), _p(y), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B, P1, P2,
+                                                 ctx.reduction, _p(gx), _p(gy), _p(ws), ws.numel(), _stream()),
+                           "ptk_chamfer_bwd_det")
+            else:
+                _lib.check(L.ptk_chamfer_bwd_lengths(_p(x), _p(y), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B, P1, P2,
+                                                     ctx.reduction, _p(gx), _p(gy), _stream()),
+                           "ptk_chamfer_bwd_lengths")
         return gx, gy, None, None, None
 
 
@@ -363,9 +377,15 @@ class _Sample(torch.autograd.Function):
         B, V, F, S = ctx.dims
         gpts = _f32c(gpts)
         gv = torch.empty(B, V, 3, dtype=torch.float32, device=gpts.device)
+        L = _lib.lib()
         with torch.cuda.device(gpts.device):
-            _lib.check(_lib.lib().ptk_sample_bwd(_p(gpts), _p(fidx), _p(uv), _p(faces_i32), B, V, F, S, _p(gv),
-                                                 _stream()), "ptk_sample_bwd")
+            if _deterministic():
+                ws = _ws(L.ptk_sample_bwd_det_workspace_bytes(B, V), gpts.device)
+                _lib.check(L.ptk_sample_bwd_det(_p(gpts), _p(fidx), _p(uv), _p(faces_i32), B, V, F, S, _p(gv), _p(ws),
+                                                ws.numel(), _stream()), "ptk_sample_bwd_det")
+            else:
+                _lib.check(L.ptk_sample_bwd(_p(gpts), _p(fidx), _p(uv), _p(faces_i32), B, V, F, S, _p(gv), _stream()),
+                           "ptk_sample_bwd")
         return gv, None, None, None, None
 
 
@@ -426,11 +446,15 @@ class _MeshChamfer(torch.autograd.Function):
         gv = torch.empty(B, V, 3, dtype=torch.float32, device=dev) if ctx.needs_input_grad[0] else None
         gg = torch.empty(B, P2, 3, dtype=torch.float32, device=dev) if ctx.needs_input_grad[1] else None
         L = _lib.lib()
-        ws = _ws(L.ptk_mesh_chamfer_workspace_bytes(B, V, F, S, P2), dev)
+        if _deterministic():
+            bwd, name = L.ptk_mesh_chamfer_bwd_det, "ptk_mesh_chamfer_bwd_det"
+            ws = _ws(L.ptk_mesh_chamfer_bwd_det_workspace_bytes(B, V, F, S, P2), dev)
+        else:
+            bwd, name = L.ptk_mesh_chamfer_bwd, "ptk_mesh_chamfer_bwd"
+            ws = _ws(L.ptk_mesh_chamfer_workspace_bytes(B, V, F, S, P2), dev)
         with torch.cuda.device(dev):
-            _lib.check(L.ptk_mesh_chamfer_bwd(_p(gt), _p(pts), _p(fidx), _p(idx_x), _p(idx_y), _p(uv), _p(faces_i32), _p(g),
-                                              B, V, F, S, P2, R, _p(gv), _p(gg), _p(ws), ws.numel(), _stream()),
-                       "ptk_mesh_chamfer_bwd")
+            _lib.check(bwd(_p(gt), _p(pts), _p(fidx), _p(idx_x), _p(idx_y), _p(uv), _p(faces_i32), _p(g), B, V, F, S, P2, R,
+                           _p(gv), _p(gg), _p(ws), ws.numel(), _stream()), name)
         return gv, gg, None, None, None, None
 
 

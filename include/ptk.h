@@ -129,6 +129,28 @@ int ptk_knn1_fwd_lengths(const float *p1, const float *p2, const int64_t *len1, 
                          int64_t P1, int64_t P2, float *dist, int32_t *idx, void *workspace, size_t workspace_bytes,
                          ptk_stream_t stream);
 
+/* Deterministic backward: the gradient of ptk_chamfer_bwd_lengths (same arguments, lengths and reductions), with
+ * bits that depend on neither the scheduling nor the batch the pair is computed in.  (The default backward scatters
+ * with fp32 atomics: its low bits vary from run to run.)  Per pair b:
+ *   - terms: a valid query's own term is s * (q - t[idx]) per component (s = 2 g[b] / max(len, 1) for mean, 2 g[b]
+ *     for sum), with the default kernels' fp32 operations; it goes to the query's row and, negated, to its nearest
+ *     neighbour's row.  Both directions always take part, so grad_y has the same bits with or without grad_x;
+ *   - scale: M_b = the largest finite |term| of both directions, e_b = 62 - ceil(log2 M_b) - ceil(log2(max(lx, ly) + 1));
+ *   - rounding: each finite term is quantised to round_half_even(term * 2^e_b) (int64), a row's quantised terms are
+ *     summed exactly (no overflow: a row holds at most max(lx, ly) + 1 terms) and the gradient is
+ *     ldexpf((float)sum, -e_b): one round-to-nearest-even of the exact quantised sum;
+ *   - non-finite terms (NaN / Inf input, overflow of the product) are added to their rows outside the integer sum: a
+ *     row with any is NaN if one is NaN or both infinities occur, otherwise that infinity;
+ *   - zero rows: padded rows, rows of a pair whose other cloud is empty and every row of a pair with M_b = 0 are +0.
+ * grad_x / grad_y (either may be NULL) are fully overwritten.  workspace: 16-byte aligned,
+ * ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2) (0 for an empty shape).  PTK_ERR_SHAPE for a null cloud / index /
+ * grad_cham pointer or an unknown reduction, PTK_ERR_WORKSPACE for a missing or too small workspace.  Three kernels
+ * and a memset, no host synchronisation, capture-safe. */
+size_t ptk_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2);
+int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y, const int32_t *idx_x,
+                        const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1, int64_t P2, int reduction,
+                        float *grad_x, float *grad_y, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Area-weighted surface sampling.  Replaces the body of utils.batch_sample
  * (pterotactyl/utility/utils.py:152-187): pytorch3d mesh_face_areas_normals (utils.py:164), the NaN
@@ -150,6 +172,16 @@ int ptk_sample_fwd(const float *verts, int64_t B, int64_t V, const int32_t *face
 int ptk_sample_bwd(const float *grad_pts, const int32_t *face_idx, const float *uv,
                    const int32_t *faces, int64_t B, int64_t V, int64_t F, int64_t S,
                    float *grad_verts, ptk_stream_t stream);
+/* Deterministic ptk_sample_bwd, the scheme of ptk_chamfer_bwd_det per mesh b: the terms are c = w_k * grad_pts[b,s,d]
+ * (the default kernel's fp32 operations), M_b = the largest finite |c|, e_b = 62 - ceil(log2 M_b) - ceil(log2(3 S + 1))
+ * (a vertex receives at most 3 S terms: a degenerate face may list it twice), exact int64 sums of
+ * round_half_even(c * 2^e_b), grad = ldexpf((float)sum, -e_b); non-finite terms as in ptk_chamfer_bwd_det; vertices
+ * no sample touches (and every vertex when M_b = 0) are +0.  grad_verts is fully overwritten.  workspace: 16-byte
+ * aligned, ptk_sample_bwd_det_workspace_bytes(B, V) (0 for an empty shape). */
+size_t ptk_sample_bwd_det_workspace_bytes(int64_t B, int64_t V);
+int ptk_sample_bwd_det(const float *grad_pts, const int32_t *face_idx, const float *uv, const int32_t *faces, int64_t B,
+                       int64_t V, int64_t F, int64_t S, float *grad_verts, void *workspace, size_t workspace_bytes,
+                       ptk_stream_t stream);
 
 /* Face areas of a batch of meshes sharing one face list: verts (B,V,3), faces (F,3) int32 -> areas (B,F); what
  * utils.batch_sample computes at utils.py:163-164 before normalising (NaN areas are left for the caller's guards). */
@@ -401,6 +433,14 @@ int ptk_mesh_chamfer_bwd(const float *gt, const float *pts, const int32_t *face_
                          const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd, int64_t B,
                          int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat, float *grad_verts,
                          float *grad_gt, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+/* The same backward on the deterministic pieces: repeat x (ptk_chamfer_bwd_det -> ptk_sample_bwd_det), accumulated in
+ * repeat order as above, so the result is bit-identical to that composition.  workspace: 256-byte aligned,
+ * ptk_mesh_chamfer_bwd_det_workspace_bytes (0 for an empty shape). */
+size_t ptk_mesh_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t V, int64_t F, int64_t S, int64_t P2);
+int ptk_mesh_chamfer_bwd_det(const float *gt, const float *pts, const int32_t *face_idx, const int32_t *idx_x,
+                             const int32_t *idx_y, const float *uv, const int32_t *faces, const float *grad_cd, int64_t B,
+                             int64_t V, int64_t F, int64_t S, int64_t P2, int64_t repeat, float *grad_verts,
+                             float *grad_gt, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Host-buffer entry points (end-to-end path: H2D + kernels + D2H inside the call).
