@@ -272,6 +272,10 @@ int ptk_relu_mask(const float *g, const float *act, int64_t n, float *out, ptk_s
  * csrc/gemm_tf32x3.cu); otherwise on exact-FP32 FFMA kernels (csrc/gcn_linear.cu).
  *   wgrad : gW (K,N) = X^T . gH  (overwrites gW; the sum over the M rows is split across CTAs and
  *           reduced in a fixed order through the workspace => deterministic)
+ * Finite range of the tensor-core paths: operands must satisfy |x| < 2^128 - 2^116 (FLT_MAX is 2^128 - 2^104).
+ * From there on, and for +-Inf and NaN, the TF32 split rounds x to +-Inf and its low part becomes NaN, so every
+ * output that x reaches is NaN -- where an fp32 loop would give +-Inf (or a finite value).  The FFMA paths follow
+ * IEEE fp32.
  * ---------------------------------------------------------------------------------------------- */
 /* Workspace of fwd and dgrad: the split weights, the packed ReLU mask and one partial output tile + flag per
  * persistent CTA (the tensor-core kernel deals its k-blocks out evenly; a tile shared by two CTAs is combined

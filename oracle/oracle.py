@@ -144,6 +144,23 @@ def gcn_linear(X, W):
     return H
 
 
+def gemm_fma_seq(A, B, rows=None, b_transposed=False):
+    """C = A[rows] . B as a scalar FP32 loop: per output acc = fmaf(A[i,k], B[k,j], acc) for k = 0..K-1 from 0.0f.
+    B is (K, N), or (N, K) read as its transpose without a copy when b_transposed (the dgrad's W)."""
+    A, B = _f32(A), _f32(B)
+    M, K = A.shape
+    N = B.shape[0] if b_transposed else B.shape[1]
+    assert B.shape == ((N, K) if b_transposed else (K, N))
+    idx = None if rows is None else np.ascontiguousarray(rows, np.int64)
+    if idx is not None:
+        assert idx.ndim == 1 and (idx.size == 0 or (idx.min() >= 0 and idx.max() < M))
+    n_rows = M if idx is None else idx.size
+    C_ = np.empty((n_rows, N), np.float32)
+    lib().orc_gemm_fma_seq(_p(A), C.c_int64(K), _p(B), C.c_int64(K if b_transposed else N), C.c_int(int(b_transposed)),
+                           _p(idx), C.c_int64(n_rows), C.c_int64(K), C.c_int64(N), _p(C_))
+    return C_
+
+
 def gcn_aggregate_fwd(rowptr, col, H, L, bias, relu):
     H = _f32(H)
     B, Nv, Cc = H.shape
