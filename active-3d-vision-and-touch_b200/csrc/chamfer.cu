@@ -411,6 +411,142 @@ chamfer_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len_x
     }
 }
 
+// 1-NN backward (ptk_knn1_bwd_lengths, ptk_knn1_bwd_det): the gradient of dist[b,i] = |p1_i - p2_j|^2, j = idx[b,i],
+// under a per-query upstream gradient g[b,i].  A valid query's term is s * (p1_i - p2_j) per component, s = 2 g[b,i]
+// (the fp32 operations of PyTorch3D's knn_points_backward and of chamfer_own_term); it is the whole gradient of p1 row i
+// and goes, negated, to p2 row j.  Padded queries and queries with an empty target cloud have no term (g is not read).
+__device__ __forceinline__ bool knn1_term(const float *__restrict__ p1b, const float *__restrict__ p2b,
+                                          const int32_t *__restrict__ idx, const float *__restrict__ g, int i, int L1,
+                                          int L2, int &j, float t[3]) {
+    if (i >= L1 || L2 <= 0) return false;
+    j = idx[i];
+    const float s = 2.0f * g[i];
+    t[0] = s * (p1b[i * 3 + 0] - p2b[j * 3 + 0]);
+    t[1] = s * (p1b[i * 3 + 1] - p2b[j * 3 + 1]);
+    t[2] = s * (p1b[i * 3 + 2] - p2b[j * 3 + 2]);
+    return true;
+}
+
+// phase A, grid = (ceil(max(P1,P2) / 256), B): grad_p1 rows (the term, or 0), grad_p2 rows zeroed for phase B
+__global__ void __launch_bounds__(CD_THREADS)
+knn1_bwd_direct_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
+                       const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
+                       const int64_t *__restrict__ len2, float *__restrict__ grad_p1, float *__restrict__ grad_p2) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
+    if (grad_p1 && i < P1) {
+        float *o = grad_p1 + ((size_t)b * P1 + i) * 3;
+        float t[3];
+        int j;
+        if (knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i,
+                      L1, L2, j, t)) {
+            o[0] = t[0];
+            o[1] = t[1];
+            o[2] = t[2];
+        } else {
+            o[0] = o[1] = o[2] = 0.0f;
+        }
+    }
+    if (grad_p2 && i < P2) {
+        float *o = grad_p2 + ((size_t)b * P2 + i) * 3;
+        o[0] = o[1] = o[2] = 0.0f;
+    }
+}
+
+// phase B, grid = (ceil(P1 / 256), B): grad_p2[b, j] -= term, RED.ADD.F32
+__global__ void __launch_bounds__(CD_THREADS)
+knn1_bwd_scatter_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
+                        const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
+                        const int64_t *__restrict__ len2, float *__restrict__ grad_p2) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
+    float t[3];
+    int j;
+    if (knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i, L1,
+                  L2, j, t)) {
+        float *o = grad_p2 + ((size_t)b * P2 + j) * 3;
+        atomicAdd(o + 0, -t[0]);
+        atomicAdd(o + 1, -t[1]);
+        atomicAdd(o + 2, -t[2]);
+    }
+}
+
+// Deterministic form (scheme in det_accum.cuh): a p1 row holds one term, so grad_p1 is phase A's plain store; only
+// grad_p2 goes through the integer sum.  M_b = the largest finite |term| of pair b, e_b from n = l1 + 1 (a p2 row
+// receives at most l1 terms).
+// phase 1, grid = (ceil(max(P1,P2) / 256), B): M_b (atomicMax into mbits[b], zeroed by the caller), grad_p1 as in phase A,
+// accumulators and outputs of every p2 row zeroed
+__global__ void __launch_bounds__(CD_THREADS)
+knn1_bwd_det_terms_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
+                          const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
+                          const int64_t *__restrict__ len2, float *__restrict__ grad_p1, float *__restrict__ grad_p2,
+                          unsigned long long *__restrict__ acc, unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
+    float m = 0.0f, t[3];
+    int j;
+    const bool term = knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1,
+                                grad_dist + (size_t)b * P1, i, L1, L2, j, t);
+    if (term) m = fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2])));
+    if (grad_p1 && i < P1) {
+        float *o = grad_p1 + ((size_t)b * P1 + i) * 3;
+        o[0] = term ? t[0] : 0.0f;
+        o[1] = term ? t[1] : 0.0f;
+        o[2] = term ? t[2] : 0.0f;
+    }
+    if (i < P2) {
+        const size_t r = ((size_t)b * P2 + i) * 3;
+        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
+        grad_p2[r + 0] = grad_p2[r + 1] = grad_p2[r + 2] = 0.0f;
+    }
+    det_block_max<CD_THREADS>(m, mbits + b);
+}
+
+// phase 2, grid = (ceil(P1 / 256), B): quantise and add into the neighbour's row (non-finite terms into grad_p2)
+__global__ void __launch_bounds__(CD_THREADS)
+knn1_bwd_det_reduce_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
+                           const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
+                           const int64_t *__restrict__ len2, float *__restrict__ grad_p2,
+                           unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
+    float t[3];
+    int j;
+    if (!knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i,
+                   L1, L2, j, t))
+        return;
+    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)L1 + 1));
+    const size_t r = ((size_t)b * P2 + j) * 3;
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+        if (isfinite(t[d]))
+            atomicAdd(acc + r + d, 0ull - det_quantise(t[d], scale));
+        else
+            atomicAdd(grad_p2 + r + d, -t[d]);
+    }
+}
+
+// phase 3, grid = (ceil(P2 / 256), B): grad_p2 = fp32(acc) * 2^-e_b, unless the row already holds a non-finite sum
+__global__ void __launch_bounds__(CD_THREADS)
+knn1_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len1, const unsigned int *__restrict__ mbits,
+                            const unsigned long long *__restrict__ acc, float *__restrict__ grad_p2) {
+    pdl_wait();
+    const int b = blockIdx.y;
+    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
+    if (i >= P2) return;
+    const int e = det_exponent(mbits[b], (long long)pair_len(len1, b, P1) + 1);
+    const size_t r = ((size_t)b * P2 + i) * 3;
+    for (int d = 0; d < 3; ++d) det_convert(grad_p2 + r + d, acc + r + d, e);
+}
+
 // ---------------------------------------------------------------------------------------- host side
 struct NNPlan {
     int R;          // queries per thread
@@ -848,6 +984,79 @@ extern "C" int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t
     PTK_CHECK_LAUNCH();
     launch_pdl(chamfer_bwd_det_convert_kernel, grid, dim3(CD_THREADS), 0, st, (int)P1, (int)P2, len_x, len_y,
                (const unsigned int *)mbits, (const unsigned long long *)acc_x, (const unsigned long long *)acc_y, grad_x, grad_y);
+    PTK_CHECK_LAUNCH();
+    return PTK_OK;
+}
+
+static int knn1_bwd_check(const float *p1, const float *p2, const int32_t *idx, const float *grad_dist, int64_t B,
+                          int64_t P1, int64_t P2) {
+    int rc = check_clouds(p1, p2, B, P1, P2);
+    if (rc) return rc;
+    PTK_REQUIRE(idx && grad_dist, PTK_ERR_SHAPE, "knn1_bwd: null index / grad pointer");
+    return PTK_OK;
+}
+
+extern "C" int ptk_knn1_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
+                                    const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
+                                    float *grad_p1, float *grad_p2, ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_bwd_lengths");
+    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
+    if (rc) return rc;
+    if (!grad_p1 && !grad_p2) return PTK_OK;
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd: batch too large");
+    cudaStream_t st = as_stream(stream);
+    const int64_t Pm = P1 > P2 ? P1 : P2;
+    launch_pdl(knn1_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1, p2,
+               idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, grad_p2);
+    PTK_CHECK_LAUNCH();
+    if (grad_p2) {
+        launch_pdl(knn1_bwd_scatter_kernel, dim3((unsigned)ceil_div(P1, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
+                   p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p2);
+        PTK_CHECK_LAUNCH();
+    }
+    return PTK_OK;
+}
+
+// det workspace: [M_b bits B, padded to 256 bytes][acc_p2 B*P2*3 int64]
+extern "C" size_t ptk_knn1_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
+    if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;
+    return det_align(4 * (size_t)B) + 24 * (size_t)B * P2;
+}
+
+extern "C" int ptk_knn1_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
+                                const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
+                                float *grad_p1, float *grad_p2, void *workspace, size_t workspace_bytes,
+                                ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_bwd_det");
+    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
+    if (rc) return rc;
+    if (!grad_p1 && !grad_p2) return PTK_OK;
+    const size_t need = ptk_knn1_bwd_det_workspace_bytes(B, P1, P2);
+    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "knn1_bwd_det: workspace too small (%zu < %zu)",
+                workspace_bytes, need);
+    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
+                "knn1_bwd_det: workspace must be 16-byte aligned");
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd_det: batch too large");
+    cudaStream_t st = as_stream(stream);
+    const int64_t Pm = P1 > P2 ? P1 : P2;
+    if (!grad_p2) {  // grad_p1 alone: plain stores, nothing to sum
+        launch_pdl(knn1_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
+                   p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, (float *)nullptr);
+        PTK_CHECK_LAUNCH();
+        return PTK_OK;
+    }
+    char *p = reinterpret_cast<char *>(workspace);
+    auto *mbits = reinterpret_cast<unsigned int *>(p);
+    auto *acc = reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B));
+    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
+    launch_pdl(knn1_bwd_det_terms_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
+               p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, grad_p2, acc, mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(knn1_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(P1, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
+               p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p2, acc, (const unsigned int *)mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(knn1_bwd_det_convert_kernel, dim3((unsigned)ceil_div(P2, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st,
+               (int)P1, (int)P2, len1, (const unsigned int *)mbits, (const unsigned long long *)acc, grad_p2);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }

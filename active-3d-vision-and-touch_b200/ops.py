@@ -155,24 +155,53 @@ def chamfer(x, y, x_lengths=None, y_lengths=None, point_reduction="mean"):
     return _Chamfer.apply(x, y, x_lengths, y_lengths, _REDUCTIONS[point_reduction])
 
 
+class _KNN1(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, p1, p2, lengths1, lengths2):
+        _need_cuda(p1, p2)
+        p1, p2 = _f32c(p1), _f32c(p2)
+        if p1.dim() != 3 or p2.dim() != 3 or p1.shape[2] != 3 or p2.shape[2] != 3 or p1.shape[0] != p2.shape[0]:
+            raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(p1.shape)} and {tuple(p2.shape)}")
+        B, P1, _ = p1.shape
+        P2 = p2.shape[1]
+        l1, l2 = _lengths(lengths1, B, p1.device, "lengths1"), _lengths(lengths2, B, p1.device, "lengths2")
+        L = _lib.lib()
+        dist = torch.empty(B, P1, dtype=torch.float32, device=p1.device)
+        idx = torch.empty(B, P1, dtype=torch.int32, device=p1.device)
+        ws = _ws(L.ptk_chamfer_workspace_bytes(B, P1, P2), p1.device)
+        with torch.cuda.device(p1.device):
+            _lib.check(L.ptk_knn1_fwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), B, P1, P2, _p(dist), _p(idx), _p(ws),
+                                              ws.numel(), _stream()), "ptk_knn1_fwd_lengths")
+        ctx.save_for_backward(p1, p2, idx, l1, l2)
+        ctx.mark_non_differentiable(idx)
+        return dist, idx
+
+    @staticmethod
+    def backward(ctx, g, _gi):
+        p1, p2, idx, l1, l2 = ctx.saved_tensors
+        B, P1, _ = p1.shape
+        P2 = p2.shape[1]
+        g = _f32c(g)
+        g1 = torch.empty_like(p1) if ctx.needs_input_grad[0] else None
+        g2 = torch.empty_like(p2) if ctx.needs_input_grad[1] else None
+        L = _lib.lib()
+        with torch.cuda.device(p1.device):
+            if _deterministic():
+                ws = _ws(L.ptk_knn1_bwd_det_workspace_bytes(B, P1, P2), p1.device)
+                _lib.check(L.ptk_knn1_bwd_det(_p(p1), _p(p2), _p(l1), _p(l2), _p(idx), _p(g), B, P1, P2, _p(g1), _p(g2),
+                                              _p(ws), ws.numel(), _stream()), "ptk_knn1_bwd_det")
+            else:
+                _lib.check(L.ptk_knn1_bwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), _p(idx), _p(g), B, P1, P2, _p(g1),
+                                                  _p(g2), _stream()), "ptk_knn1_bwd_lengths")
+        return g1, g2, None, None
+
+
 def knn1(p1, p2, lengths1=None, lengths2=None):
-    """dists (B,P1) f32, idx (B,P1) int32 -- forward only.  lengths1 / lengths2 as in chamfer(): padded queries and
-    queries whose target cloud is empty get dist 0, idx 0."""
-    _need_cuda(p1, p2)
-    p1, p2 = _f32c(p1), _f32c(p2)
-    if p1.dim() != 3 or p2.dim() != 3 or p1.shape[2] != 3 or p2.shape[2] != 3 or p1.shape[0] != p2.shape[0]:
-        raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(p1.shape)} and {tuple(p2.shape)}")
-    B, P1, _ = p1.shape
-    P2 = p2.shape[1]
-    l1, l2 = _lengths(lengths1, B, p1.device, "lengths1"), _lengths(lengths2, B, p1.device, "lengths2")
-    L = _lib.lib()
-    dist = torch.empty(B, P1, dtype=torch.float32, device=p1.device)
-    idx = torch.empty(B, P1, dtype=torch.int32, device=p1.device)
-    ws = _ws(L.ptk_chamfer_workspace_bytes(B, P1, P2), p1.device)
-    with torch.cuda.device(p1.device):
-        _lib.check(L.ptk_knn1_fwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), B, P1, P2, _p(dist), _p(idx), _p(ws),
-                                          ws.numel(), _stream()), "ptk_knn1_fwd_lengths")
-    return dist, idx
+    """dists (B,P1) f32, idx (B,P1) int32.  dists = |p1[b,i] - p2[b,idx]|^2 is differentiable w.r.t. p1 and p2 (the
+    gradient of PyTorch3D's knn_points; deterministic under torch.use_deterministic_algorithms(True)).  lengths1 /
+    lengths2 as in chamfer(): padded queries and queries whose target cloud is empty get dist 0, idx 0 and pass no
+    gradient; padded rows get a zero gradient."""
+    return _KNN1.apply(p1, p2, lengths1, lengths2)
 
 
 # ------------------------------------------------------------------------------------- vertex max-pool

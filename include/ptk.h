@@ -151,6 +151,35 @@ int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t *len_x, co
                         const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1, int64_t P2, int reduction,
                         float *grad_x, float *grad_y, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
 
+/* 1-NN backward: the gradient of dist = ptk_knn1_fwd_lengths(p1, p2, len1, len2) under a per-query upstream gradient
+ * grad_dist (B,P1), with the forward's idx (B,P1).  len1 / len2 as above (NULL: full).  For a valid query i < l1[b]
+ * of a pair with l2[b] > 0 and j = idx[b,i], the term is t = s * (p1[b,i] - p2[b,j]) per component, s = 2 grad_dist[b,i]
+ * (fp32, the operations of PyTorch3D's knn_points_backward for norm 2):
+ *   - grad_p1[b,i] = t (a plain store: a p1 row holds exactly one term);
+ *   - grad_p2[b,j] -= t, summed over every query that chose j;
+ *   - padded queries and queries whose target cloud is empty contribute nothing: their grad_dist is never read, so a
+ *     NaN there does not leak.  Padded rows of both gradients, and every row of a pair with l1 = 0 or l2 = 0, are +0.
+ * grad_p1 / grad_p2 (either may be NULL) are fully overwritten; neither requested: return 0 at once.  PTK_ERR_SHAPE for
+ * a null cloud / idx / grad_dist pointer, an empty or too large shape, B > 65535.  No host synchronisation,
+ * capture-safe.  Replaces pytorch3d.ops.knn_points' backward (_C.knn_points_backward) for K = 1.
+ * ptk_knn1_bwd_lengths: two kernels, grad_p1 and zeroed grad_p2 rows, then a scatter with fp32 atomics (grad_p2's low
+ * bits vary from run to run). */
+int ptk_knn1_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                         const float *grad_dist, int64_t B, int64_t P1, int64_t P2, float *grad_p1, float *grad_p2,
+                         ptk_stream_t stream);
+/* Deterministic form: the scheme of ptk_chamfer_bwd_det per pair b.  grad_p1 is the same plain store, with the same
+ * bits as ptk_knn1_bwd_lengths.  grad_p2: M_b = the largest finite |term| of the pair's valid queries,
+ * e_b = 62 - ceil(log2 M_b) - ceil(log2(l1 + 1)) (a p2 row receives at most l1 terms), exact int64 sums of
+ * round_half_even(term * 2^e_b), grad_p2 = ldexpf((float)sum, -e_b); non-finite terms bypass the integer sum as in
+ * ptk_chamfer_bwd_det.  Bits depend neither on scheduling nor on the batch the pair runs in.  workspace: 16-byte aligned,
+ * ptk_knn1_bwd_det_workspace_bytes(B, P1, P2) = [M_b bits, padded to 256 B][24 B per p2 point] (0 for an empty shape),
+ * also required when only grad_p1 is requested; PTK_ERR_WORKSPACE when missing or too small.  A memset and three
+ * kernels (one kernel without grad_p2). */
+size_t ptk_knn1_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2);
+int ptk_knn1_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                     const float *grad_dist, int64_t B, int64_t P1, int64_t P2, float *grad_p1, float *grad_p2,
+                     void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Area-weighted surface sampling.  Replaces the body of utils.batch_sample
  * (pterotactyl/utility/utils.py:152-187): pytorch3d mesh_face_areas_normals (utils.py:164), the NaN
