@@ -806,16 +806,6 @@ extern "C" int ptk_chamfer_rescued(const void *workspace, int64_t B, int64_t P1,
     return PTK_OK;
 }
 
-static int check_clouds(const void *x, const void *y, int64_t B, int64_t P1, int64_t P2) {
-    PTK_REQUIRE(x && y, PTK_ERR_SHAPE, "chamfer: null cloud pointer");
-    PTK_REQUIRE(B > 0 && P1 > 0 && P2 > 0, PTK_ERR_SHAPE,
-                "chamfer: empty input (B=%lld, P1=%lld, P2=%lld); point clouds must be non-empty",
-                (long long)B, (long long)P1, (long long)P2);
-    PTK_REQUIRE(P1 < (1LL << 31) / 3 && P2 < (1LL << 31) / 3, PTK_ERR_SHAPE,
-                "chamfer: cloud too large for 32-bit indexing");
-    return PTK_OK;
-}
-
 static int knn1_fwd(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, int64_t B, int64_t P1,
                     int64_t P2, float *dist, int32_t *idx, void *workspace, size_t workspace_bytes, ptk_stream_t stream) {
     int rc = check_clouds(p1, p2, B, P1, P2);
@@ -942,7 +932,6 @@ extern "C" int ptk_chamfer_bwd_lengths(const float *x, const float *y, const int
 }
 
 // det workspace: [M_b bits B, padded to 256 bytes][acc_x B*P1*3 int64][acc_y B*P2*3 int64]
-static size_t det_align(size_t b) { return (b + 255) & ~(size_t)255; }
 
 extern "C" size_t ptk_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
     if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;

@@ -23,34 +23,9 @@
 //     thr = +inf (non-finite or extreme input) sends every query down the exact path.
 #pragma once
 #include "chamfer_kernel.cuh"
+#include "nn_common.cuh"
 
 namespace ptk {
-
-typedef unsigned long long u64;
-
-__device__ __forceinline__ u64 pack2(float lo, float hi) {
-    u64 r;
-    asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
-    return r;
-}
-__device__ __forceinline__ void unpack2(u64 v, float &lo, float &hi) {
-    asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v));
-}
-__device__ __forceinline__ u64 fma2(u64 a, u64 b, u64 c) {
-    u64 r;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(a), "l"(b), "l"(c));
-    return r;
-}
-__device__ __forceinline__ u64 sub2(u64 a, u64 b) {
-    u64 r;
-    asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
-__device__ __forceinline__ u64 mul2(u64 a, u64 b) {
-    u64 r;
-    asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
-    return r;
-}
 
 // Per cloud pair: centre c of the joint bounding box and the ambiguity threshold of the filter.
 //
@@ -78,14 +53,6 @@ struct PairAux {
 };
 constexpr float FILTER_THR_BD = 1.9073486e-6f;  // 32 u = 2^-19
 
-// Ragged batches: the points of cloud b that exist, len[b] clamped to [0, P] (P when the caller passed no lengths).
-// Row strides stay those of the padded (B, P, 3) tensor; only the counts of queries and targets become per pair, so
-// padding points are never read into a result, a bound or the filter's certificate.
-__device__ __forceinline__ int pair_len(const int64_t *__restrict__ len, int b, int P) {
-    if (len == nullptr) return P;
-    const long long v = len[b];
-    return v < 0 ? 0 : (v > P ? P : (int)v);
-}
 
 __global__ void __launch_bounds__(1024)
 chamfer_bounds_kernel(const float *__restrict__ x, const float *__restrict__ y, int P1, int P2,

@@ -53,6 +53,9 @@ __device__ __forceinline__ void det_block_max(float m, unsigned int *mbits) {
     }
 }
 
+// workspace sections are aligned to 256 bytes
+inline size_t det_align(size_t b) { return (b + 255) & ~(size_t)255; }
+
 __device__ __forceinline__ float det_abs_finite(float t) { return isfinite(t) ? fabsf(t) : 0.0f; }
 
 // the row's gradient: its output holds the sum of its non-finite terms (0 when there are none)

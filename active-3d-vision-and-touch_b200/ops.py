@@ -204,6 +204,65 @@ def knn1(p1, p2, lengths1=None, lengths2=None):
     return _KNN1.apply(p1, p2, lengths1, lengths2)
 
 
+class _KNN(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, p1, p2, K, lengths1, lengths2):
+        _need_cuda(p1, p2)
+        p1, p2 = _f32c(p1), _f32c(p2)
+        if p1.dim() != 3 or p2.dim() != 3 or p1.shape[2] != 3 or p2.shape[2] != 3 or p1.shape[0] != p2.shape[0]:
+            raise ValueError(f"Expected (B,P,3) point clouds, got {tuple(p1.shape)} and {tuple(p2.shape)}")
+        B, P1, _ = p1.shape
+        P2 = p2.shape[1]
+        l1, l2 = _lengths(lengths1, B, p1.device, "lengths1"), _lengths(lengths2, B, p1.device, "lengths2")
+        L = _lib.lib()
+        dist = torch.empty(B, P1, K, dtype=torch.float32, device=p1.device)
+        idx = torch.empty(B, P1, K, dtype=torch.int32, device=p1.device)
+        ws = _ws(L.ptk_knn_workspace_bytes(B, P1, P2, K), p1.device)
+        with torch.cuda.device(p1.device):
+            _lib.check(L.ptk_knn_fwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), B, P1, P2, K, _p(dist), _p(idx), _p(ws),
+                                             ws.numel(), _stream()), "ptk_knn_fwd_lengths")
+        ctx.save_for_backward(p1, p2, idx, l1, l2)
+        ctx.mark_non_differentiable(idx)
+        return dist, idx
+
+    @staticmethod
+    def backward(ctx, g, _gi):
+        p1, p2, idx, l1, l2 = ctx.saved_tensors
+        B, P1, K = idx.shape
+        P2 = p2.shape[1]
+        g = _f32c(g)
+        g1 = torch.empty_like(p1) if ctx.needs_input_grad[0] else None
+        g2 = torch.empty_like(p2) if ctx.needs_input_grad[1] else None
+        L = _lib.lib()
+        with torch.cuda.device(p1.device):
+            if _deterministic():
+                ws = _ws(L.ptk_knn1_bwd_det_workspace_bytes(B, P1, P2), p1.device)
+                _lib.check(L.ptk_knn_bwd_det(_p(p1), _p(p2), _p(l1), _p(l2), _p(idx), _p(g), B, P1, P2, K, _p(g1),
+                                             _p(g2), _p(ws), ws.numel(), _stream()), "ptk_knn_bwd_det")
+            else:
+                _lib.check(L.ptk_knn_bwd_lengths(_p(p1), _p(p2), _p(l1), _p(l2), _p(idx), _p(g), B, P1, P2, K, _p(g1),
+                                                 _p(g2), _stream()), "ptk_knn_bwd_lengths")
+        return g1, g2, None, None, None
+
+
+def knn(p1, p2, K, lengths1=None, lengths2=None):
+    """dists (B,P1,K) f32, idx (B,P1,K) int32: the K nearest p2 points of every p1 point, ascending distance and the
+    lower index first on equal distances (include/ptk.h), 1 <= K <= 64.  Column 0 is knn1().  dists is differentiable
+    w.r.t. p1 and p2 (deterministic under torch.use_deterministic_algorithms(True)); idx is not.  lengths1 / lengths2
+    as in knn1(): padded queries get (0, 0) in every slot, slots k >= lengths2[b] get (0, 0), and neither passes a
+    gradient.  K = 1 runs knn1()."""
+    if isinstance(K, bool) or not isinstance(K, int):
+        raise ValueError(f"K must be an int, got {K!r}")
+    if K < 1:
+        raise ValueError(f"K must be >= 1, got {K}")
+    if K > _lib.KNN_MAX_K:
+        raise NotImplementedError(f"ptk_b200 knn supports K <= {_lib.KNN_MAX_K}, got K={K}")
+    if K == 1:
+        dist, idx = knn1(p1, p2, lengths1, lengths2)
+        return dist[..., None], idx[..., None]
+    return _KNN.apply(p1, p2, K, lengths1, lengths2)
+
+
 # ------------------------------------------------------------------------------------- vertex max-pool
 class _VertexMax(torch.autograd.Function):
     @staticmethod

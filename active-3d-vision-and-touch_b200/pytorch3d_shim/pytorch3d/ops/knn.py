@@ -1,6 +1,6 @@
-"""pytorch3d.ops.knn_points for K=1 and pytorch3d.ops.knn_gather, on homogeneous or ragged batches (lengths1 /
-lengths2: padded queries and queries whose target cloud is empty get dist 0 and idx 0, as in PyTorch3D).  dists and
-knn are differentiable w.r.t. p1 and p2, as PyTorch3D's are."""
+"""pytorch3d.ops.knn_points for 1 <= K <= 64 and pytorch3d.ops.knn_gather, on homogeneous or ragged batches (lengths1 /
+lengths2: padded queries, queries whose target cloud is empty and slots k >= lengths2 get dist 0 and idx 0, as in
+PyTorch3D).  dists and knn are differentiable w.r.t. p1 and p2, as PyTorch3D's are."""
 from collections import namedtuple
 
 import torch
@@ -11,12 +11,19 @@ _KNN = namedtuple("KNN", "dists idx knn")
 
 
 def knn_points(p1, p2, lengths1=None, lengths2=None, K=1, version=-1, return_nn=False, return_sorted=True):
-    if K != 1:
-        raise NotImplementedError("ptk_b200 knn_points supports K=1")
-    dists, idx = ptk_b200.ops.knn1(p1, p2, lengths1, lengths2)
-    idx = idx.long()[..., None]
+    """`version` is ignored; return_sorted=False returns the sorted order too (a valid unsorted order)."""
+    if K == 1:
+        dists, idx = ptk_b200.ops.knn1(p1, p2, lengths1, lengths2)
+        idx = idx.long()[..., None]
+        knn = knn_gather(p2, idx, lengths2) if return_nn else None
+        return _KNN(dists=dists[..., None], idx=idx, knn=knn)
+    if isinstance(K, int) and K >= 2 and not (p1.is_cuda and p2.is_cuda):
+        raise NotImplementedError(
+            "ptk_b200 ops run on CUDA (sm_100a) tensors only; got a CPU tensor. There is no CPU fallback.")
+    dists, idx = ptk_b200.ops.knn(p1, p2, K, lengths1, lengths2)
+    idx = idx.long()
     knn = knn_gather(p2, idx, lengths2) if return_nn else None
-    return _KNN(dists=dists[..., None], idx=idx, knn=knn)
+    return _KNN(dists=dists, idx=idx, knn=knn)
 
 
 def knn_gather(x, idx, lengths=None):

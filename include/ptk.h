@@ -180,6 +180,55 @@ int ptk_knn1_bwd_det(const float *p1, const float *p2, const int64_t *len1, cons
                      const float *grad_dist, int64_t B, int64_t P1, int64_t P2, float *grad_p1, float *grad_p2,
                      void *workspace, size_t workspace_bytes, ptk_stream_t stream);
 
+/* K nearest neighbours, 1 <= K <= PTK_KNN_MAX_K: pytorch3d.ops.knn_points(p1, p2, lengths1, lengths2, K).
+ * len1 / len2 as for the ragged calls above (device int64, NULL: full, clamped on the device).  For pair b write
+ * l1 = len1[b], l2 = len2[b].  For a valid query i < l1, dist[b,i,:] / idx[b,i,:] (B,P1,K) f32 / int32 are the K
+ * smallest (d, j) over targets j < l2 in lexicographic order: ascending distance, the lower index first on equal
+ * distances.  d is the defining arithmetic of ptk_knn1_fwd (fma(dz,dz, fma(dy,dy, dx*dx)), dx = q.x - t.x).
+ * Operationally: K slots of (+inf, 0); j ascending; (d, j) enters when d < slot[K-1].d (strict: an equal distance
+ * never displaces a lower index, a NaN or +inf distance never enters) and is inserted after every slot whose distance
+ * is <= d.  This is the selection rule of PyTorch3D's knn_cpu.cpp.  Consequences:
+ *   - column 0 is ptk_knn1_fwd_lengths' result bit for bit, for every input (NaN, Inf, ties included);
+ *   - slots that no finite distance fills stay (+inf, 0);
+ *   - zero fill, as PyTorch3D pads: slots k >= l2 are (0, 0), padded queries i >= l1 are (0, 0) in every slot, and
+ *     so is every slot of a pair with l2 = 0.  K > P2 is allowed;
+ *   - the result is a pure function of the pair: it depends neither on the batch nor on how the target range is split.
+ * workspace: 16-byte aligned, ptk_knn_workspace_bytes(B, P1, P2, K) (a function of the shapes only; 0 when the target
+ * range is not split, and then workspace may be NULL).  PTK_ERR_SHAPE for a null cloud / dist / idx pointer, an empty
+ * or too large shape, B > 65535 or K outside [1, PTK_KNN_MAX_K]; PTK_ERR_WORKSPACE for a missing or too small
+ * workspace, PTK_ERR_ALIGN for a misaligned one.  One scan kernel (plus a merge kernel when the target range is
+ * split), PDL-chained, no host synchronisation, capture-safe. */
+#define PTK_KNN_MAX_K 64
+size_t ptk_knn_workspace_bytes(int64_t B, int64_t P1, int64_t P2, int64_t K);
+int ptk_knn_fwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, int64_t B,
+                        int64_t P1, int64_t P2, int64_t K, float *dist, int32_t *idx, void *workspace,
+                        size_t workspace_bytes, ptk_stream_t stream);
+/* K-NN backward: the gradient of dist = ptk_knn_fwd_lengths(...) under the upstream gradient grad_dist (B,P1,K), with
+ * the forward's idx (B,P1,K).  Slot k < min(K, l2) of a valid query i < l1, with j = idx[b,i,k], has the term
+ * t = s * (p1[b,i] - p2[b,j]) per component, s = 2 grad_dist[b,i,k] (fp32: the operations of ptk_knn1_bwd_lengths and
+ * of PyTorch3D's knn_points_backward).  No other slot exists: its grad_dist is never read, so a NaN there does not leak.
+ *   - grad_p1[b,i] = the terms of row i summed in slot order, ((t0 + t1) + t2) + ..., in fp32 (no atomics: the same
+ *     bits in both forms below);
+ *   - grad_p2[b,j] = minus the sum of the terms that chose j;
+ *   - padded rows of both gradients, and every row of a pair with l1 = 0 or l2 = 0, are +0.
+ * grad_p1 / grad_p2 (either may be NULL) are fully overwritten; neither requested: return 0 at once.  PTK_ERR_SHAPE as
+ * for ptk_knn_fwd_lengths and for a null idx / grad_dist pointer.  No host synchronisation, capture-safe.
+ * ptk_knn_bwd_lengths: two kernels, grad_p1 with zeroed grad_p2 rows, then a scatter with fp32 atomics (grad_p2's low
+ * bits vary from run to run). */
+int ptk_knn_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                        const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K, float *grad_p1,
+                        float *grad_p2, ptk_stream_t stream);
+/* Deterministic form: the scheme of ptk_knn1_bwd_det per pair b.  grad_p1 as above.  grad_p2: M_b = the largest finite
+ * |term| of the pair's slots, e_b = 62 - ceil(log2 M_b) - ceil(log2(l1 + 1)) (a query's K indices are distinct, so a p2
+ * row receives at most l1 terms), exact int64 sums of round_half_even(term * 2^e_b), grad_p2 = ldexpf((float)sum,
+ * -e_b); non-finite terms bypass the integer sum.  Bits depend neither on scheduling nor on the batch or the order of
+ * the queries.  workspace: 16-byte aligned, ptk_knn1_bwd_det_workspace_bytes(B, P1, P2) (the same layout), also
+ * required when only grad_p1 is requested; PTK_ERR_WORKSPACE when missing or too small.  A memset and three kernels
+ * (one kernel without grad_p2). */
+int ptk_knn_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                    const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K, float *grad_p1, float *grad_p2,
+                    void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Area-weighted surface sampling.  Replaces the body of utils.batch_sample
  * (pterotactyl/utility/utils.py:152-187): pytorch3d mesh_face_areas_normals (utils.py:164), the NaN
