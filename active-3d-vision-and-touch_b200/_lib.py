@@ -43,7 +43,13 @@ SIGNATURES = {
     "ptk_knn1_fwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_chamfer_bwd_det_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "ptk_chamfer_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _sz, _vp]),
-    "ptk_knn1_bwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp]),
+    "ptk_chamfer_normals_workspace_bytes": (_sz, [_i64, _i64, _i64]),
+    "ptk_chamfer_normals_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _sz,
+                                          _vp]),
+    "ptk_chamfer_normals_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp]),
+    "ptk_chamfer_normals_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp,
+                                              _sz, _vp]),
+    "ptk_knn1_bwd_lengths":(C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp]),
     "ptk_knn1_bwd_det_workspace_bytes": (_sz, [_i64, _i64, _i64]),
     "ptk_knn1_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_knn_workspace_bytes": (_sz, [_i64, _i64, _i64, _i64]),

@@ -134,17 +134,6 @@ static ChamferWs carve(void *workspace, int64_t B, int64_t P1, int64_t P2) {
 // does not depend on the batch it is computed in.  In a ragged batch each pair is sliced by fin_splits of its OWN lengths
 // (CTAs past that count only zero-fill padding), so its value is also that of a homogeneous call on the sliced pair.
 // Padded queries (i >= len) and queries whose target cloud is empty get dist = 0, idx = 0 (PyTorch3D's zero fill).
-constexpr int FIN_SLICE = 16384;
-__host__ __device__ inline int fin_splits(int64_t P1, int64_t P2) {
-    const int64_t n = ceil_div(P1 > P2 ? P1 : P2, (int64_t)FIN_SLICE);
-    return (int)(n < 1 ? 1 : (n > 64 ? 64 : n));
-}
-
-// cham[b] from the two sums: mean = sum_x / max(lx, 1) + sum_y / max(ly, 1), sum = sum_x + sum_y
-__device__ __forceinline__ float chamfer_reduce(float sx, float sy, int L1, int L2, int mean) {
-    return mean ? sx / (float)max(L1, 1) + sy / (float)max(L2, 1) : sx + sy;
-}
-
 __global__ void __launch_bounds__(512)
 chamfer_finalize_kernel(const unsigned long long *__restrict__ keys_x,
                         const unsigned long long *__restrict__ keys_y, int P1, int P2,

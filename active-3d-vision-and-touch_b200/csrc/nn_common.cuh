@@ -40,6 +40,20 @@ __device__ __forceinline__ int pair_len(const int64_t *__restrict__ len, int b, 
     return v < 0 ? 0 : (v > P ? P : (int)v);
 }
 
+// Fixed-order per-pair reductions (chamfer_finalize_kernel, the Chamfer normal term): a pair's queries are cut into
+// fin_splits(l1, l2) slices of its OWN lengths, one CTA per slice, and the slice partials are added in slice order, so
+// a pair's value depends neither on the batch nor on the padding it is computed in.  1 slice up to 16k points.
+constexpr int FIN_SLICE = 16384;
+__host__ __device__ inline int fin_splits(int64_t P1, int64_t P2) {
+    const int64_t n = ceil_div(P1 > P2 ? P1 : P2, (int64_t)FIN_SLICE);
+    return (int)(n < 1 ? 1 : (n > 64 ? 64 : n));
+}
+
+// cham[b] from the two sums: mean = sum_x / max(lx, 1) + sum_y / max(ly, 1), sum = sum_x + sum_y
+__device__ __forceinline__ float chamfer_reduce(float sx, float sy, int L1, int L2, int mean) {
+    return mean ? sx / (float)max(L1, 1) + sy / (float)max(L2, 1) : sx + sy;
+}
+
 // host-side validation of a cloud pair shared by the Chamfer and K-NN entry points
 static inline int check_clouds(const void *x, const void *y, int64_t B, int64_t P1, int64_t P2) {
     PTK_REQUIRE(x && y, PTK_ERR_SHAPE, "chamfer: null cloud pointer");

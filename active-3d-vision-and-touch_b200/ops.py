@@ -155,6 +155,69 @@ def chamfer(x, y, x_lengths=None, y_lengths=None, point_reduction="mean"):
     return _Chamfer.apply(x, y, x_lengths, y_lengths, _REDUCTIONS[point_reduction])
 
 
+class _ChamferNormals(torch.autograd.Function):
+    """cham_normals (B,) from the normals and the nearest-neighbour indices of one _Chamfer call; differentiable w.r.t.
+    the normals only."""
+
+    @staticmethod
+    def forward(ctx, xn, yn, lx, ly, idx_x, idx_y, reduction):
+        B, P1, _ = xn.shape
+        P2 = yn.shape[1]
+        L = _lib.lib()
+        cham_n = torch.empty(B, dtype=torch.float32, device=xn.device)
+        ws = _ws(L.ptk_chamfer_normals_workspace_bytes(B, P1, P2), xn.device)
+        with torch.cuda.device(xn.device):
+            _lib.check(L.ptk_chamfer_normals_fwd(_p(xn), _p(yn), _p(lx), _p(ly), _p(idx_x), _p(idx_y), B, P1, P2, reduction,
+                                                 None, None, _p(cham_n), _p(ws), ws.numel(), _stream()),
+                       "ptk_chamfer_normals_fwd")
+        ctx.save_for_backward(xn, yn, lx, ly, idx_x, idx_y)
+        ctx.reduction = reduction
+        return cham_n
+
+    @staticmethod
+    def backward(ctx, g):
+        xn, yn, lx, ly, idx_x, idx_y = ctx.saved_tensors
+        B, P1, _ = xn.shape
+        P2 = yn.shape[1]
+        g = _f32c(g)
+        gx = torch.empty_like(xn) if ctx.needs_input_grad[0] else None
+        gy = torch.empty_like(yn) if ctx.needs_input_grad[1] else None
+        L = _lib.lib()
+        with torch.cuda.device(xn.device):
+            if _deterministic():
+                ws = _ws(L.ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2), xn.device)
+                _lib.check(L.ptk_chamfer_normals_bwd_det(_p(xn), _p(yn), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B,
+                                                         P1, P2, ctx.reduction, _p(gx), _p(gy), _p(ws), ws.numel(),
+                                                         _stream()), "ptk_chamfer_normals_bwd_det")
+            else:
+                _lib.check(L.ptk_chamfer_normals_bwd(_p(xn), _p(yn), _p(lx), _p(ly), _p(idx_x), _p(idx_y), _p(g), B, P1,
+                                                     P2, ctx.reduction, _p(gx), _p(gy), _stream()),
+                           "ptk_chamfer_normals_bwd")
+        return gx, gy, None, None, None, None, None
+
+
+def chamfer_normals(x, y, x_normals, y_normals, x_lengths=None, y_lengths=None, point_reduction="mean"):
+    """(cham, cham_normals, idx_x, idx_y): chamfer() and PyTorch3D 0.5.0's normal term on that call's nearest
+    neighbours.  x_normals (B,P1,3) and y_normals (B,P2,3) have their clouds' shapes.  cham_normals[b] sums
+    1 - |cos(n_i, n_nearest)| over the valid queries of both directions (F.cosine_similarity with eps=1e-6; a query whose
+    target cloud is empty counts 1), divided by max(length, 1) per direction for "mean" (include/ptk.h).  cham is
+    bit-identical to chamfer()'s and differentiable w.r.t. x and y; cham_normals is differentiable w.r.t. the normals
+    only (deterministic under torch.use_deterministic_algorithms(True))."""
+    if point_reduction not in _REDUCTIONS:
+        raise ValueError('point_reduction must be one of ["mean", "sum"]')
+    for name, n, cloud in (("x_normals", x_normals, x), ("y_normals", y_normals, y)):
+        if not torch.is_tensor(n) or n.shape != cloud.shape:
+            raise ValueError(f"{name} must have the shape of its cloud {tuple(cloud.shape)}, "
+                             f"got {tuple(n.shape) if torch.is_tensor(n) else type(n).__name__}")
+    _need_cuda(x, y, x_normals, y_normals)
+    reduction = _REDUCTIONS[point_reduction]
+    cham, idx_x, idx_y = _Chamfer.apply(x, y, x_lengths, y_lengths, reduction)
+    B = x.shape[0]
+    lx, ly = _lengths(x_lengths, B, x.device, "x_lengths"), _lengths(y_lengths, B, x.device, "y_lengths")
+    cham_n = _ChamferNormals.apply(_f32c(x_normals), _f32c(y_normals), lx, ly, idx_x, idx_y, reduction)
+    return cham, cham_n, idx_x, idx_y
+
+
 class _KNN1(torch.autograd.Function):
     @staticmethod
     def forward(ctx, p1, p2, lengths1, lengths2):

@@ -151,6 +151,55 @@ int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t *len_x, co
                         const int32_t *idx_y, const float *grad_cham, int64_t B, int64_t P1, int64_t P2, int reduction,
                         float *grad_x, float *grad_y, void *workspace, size_t workspace_bytes, ptk_stream_t stream);
 
+/* Chamfer normal term: the cham_normals of pytorch3d.loss.chamfer_distance(x, y, x_lengths, y_lengths, x_normals,
+ * y_normals, point_reduction=...) of PyTorch3D 0.5.0, on the idx_x / idx_y of ptk_chamfer_fwd_lengths (cham itself is
+ * that call's, unchanged).  x_normals (B,P1,3), y_normals (B,P2,3); len_x / len_y as for the ragged calls above.  For
+ * pair b write lx = len_x[b], ly = len_y[b] (clamped to [0, P]).  For a valid query x_i (i < lx) with ly > 0 and
+ * j = idx_x[b,i], a = x_normals[b,i], n = y_normals[b,j]:
+ *     c_i = sum_k (a_k / max(|a|, 1e-6)) * (n_k / max(|n|, 1e-6))     (torch's F.cosine_similarity, eps = 1e-6: each
+ *     term_x[b,i] = 1 - |c_i|                                          norm clamped on its own)
+ *   - a valid query whose target cloud is empty (ly = 0) reads PyTorch3D's zero-filled gathered normal: c = 0 and the
+ *     term is 1 (NaN for a non-finite a, as there);
+ *   - padded queries (i >= lx) have term 0; the y direction is the same with idx_y and the roles swapped;
+ *   - PTK_REDUCE_MEAN: cham_normals[b] = sum term_x / max(lx, 1) + sum term_y / max(ly, 1) (the divisors of cham);
+ *     PTK_REDUCE_SUM: the plain sum.  The sum of a pair is a fixed-order function of the pair alone: its bits depend
+ *     neither on the batch nor on the padding it is computed in;
+ *   - term_x (B,P1) / term_y (B,P2) (either may be NULL) receive the per-query terms, 0 at padded entries.
+ * Padding (normals and idx of padded rows) is never read.  workspace: ptk_chamfer_normals_workspace_bytes(B, P1, P2)
+ * of 16-byte aligned slice partials, 0 (workspace may be NULL) up to 16384 points per cloud.  PTK_ERR_SHAPE for a null
+ * normals / idx / cham_normals pointer, an unknown reduction, an empty or too large shape or B > 65535;
+ * PTK_ERR_WORKSPACE / PTK_ERR_ALIGN for a missing, too small or misaligned workspace.  One kernel (two when the clouds
+ * are sliced), PDL-chained, no host synchronisation, capture-safe. */
+size_t ptk_chamfer_normals_workspace_bytes(int64_t B, int64_t P1, int64_t P2);
+int ptk_chamfer_normals_fwd(const float *x_normals, const float *y_normals, const int64_t *len_x, const int64_t *len_y,
+                            const int32_t *idx_x, const int32_t *idx_y, int64_t B, int64_t P1, int64_t P2, int reduction,
+                            float *term_x, float *term_y, float *cham_normals, void *workspace, size_t workspace_bytes,
+                            ptk_stream_t stream);
+/* Gradient of cham_normals under grad_cham_normals (B) w.r.t. the normals only (the points get none: idx is piecewise
+ * constant).  It is torch's autograd of the formula above: d|c|/dc = sign(c) with sign(0) = 0, and
+ * dc/da = (n / |n|_c - c * a / |a|) / |a|_c, |.|_c the clamped norm, a / |a| = 0 at a = 0.  Each valid query with a
+ * non-empty target cloud has an own part, -s sign(c) dc/da onto its normal row, and a near part, -s sign(c) dc/dn onto
+ * the gathered row j (s = g[b] / lq for mean, g[b] for sum).  Padded rows, and every row of a pair with lx = 0 or
+ * ly = 0 in the direction that has no target, get +0.  grad_xn (B,P1,3) / grad_yn (B,P2,3) (either may be NULL) are
+ * fully overwritten; neither requested: return 0 at once.  PTK_ERR_SHAPE as for the forward and for a null
+ * grad_cham_normals pointer.  No host synchronisation, capture-safe.
+ * ptk_chamfer_normals_bwd: two kernels, the own parts as plain stores, then the near parts with fp32 atomics (their
+ * rows' low bits vary from run to run).
+ * ptk_chamfer_normals_bwd_det: the scheme of ptk_chamfer_bwd_det per pair: M_b = the largest finite |part| of both
+ * directions, e_b = 62 - ceil(log2 M_b) - ceil(log2(max(lx, ly) + 1)) (a row holds one own part and at most l_other
+ * near parts), exact int64 sums of round_half_even(part * 2^e_b), grad = ldexpf((float)sum, -e_b), non-finite parts
+ * outside the integer sum.  Bits depend neither on scheduling nor on the batch or the order of the queries.  workspace:
+ * ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2) (the same layout), 16-byte aligned; PTK_ERR_WORKSPACE when missing or
+ * too small.  A memset and three kernels. */
+int ptk_chamfer_normals_bwd(const float *x_normals, const float *y_normals, const int64_t *len_x, const int64_t *len_y,
+                            const int32_t *idx_x, const int32_t *idx_y, const float *grad_cham_normals, int64_t B,
+                            int64_t P1, int64_t P2, int reduction, float *grad_xn, float *grad_yn, ptk_stream_t stream);
+int ptk_chamfer_normals_bwd_det(const float *x_normals, const float *y_normals, const int64_t *len_x,
+                                const int64_t *len_y, const int32_t *idx_x, const int32_t *idx_y,
+                                const float *grad_cham_normals, int64_t B, int64_t P1, int64_t P2, int reduction,
+                                float *grad_xn, float *grad_yn, void *workspace, size_t workspace_bytes,
+                                ptk_stream_t stream);
+
 /* 1-NN backward: the gradient of dist = ptk_knn1_fwd_lengths(p1, p2, len1, len2) under a per-query upstream gradient
  * grad_dist (B,P1), with the forward's idx (B,P1).  len1 / len2 as above (NULL: full).  For a valid query i < l1[b]
  * of a pair with l2[b] > 0 and j = idx[b,i], the term is t = s * (p1[b,i] - p2[b,j]) per component, s = 2 grad_dist[b,i]
