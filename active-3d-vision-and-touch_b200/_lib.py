@@ -56,6 +56,10 @@ SIGNATURES = {
     "ptk_knn_fwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_knn_bwd_lengths": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp]),
     "ptk_knn_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp, _vp, _sz, _vp]),
+    "ptk_point_frames_fwd": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp]),
+    "ptk_point_frames_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp]),
+    "ptk_point_frames_bwd_det": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, C.c_int, _vp, _vp, _vp, _vp, _vp, _sz,
+                                           _vp]),
     "ptk_sample_workspace_bytes": (_sz, [_i64, _i64]),
     "ptk_sample_fwd": (C.c_int, [_vp, _i64, _i64, _vp, _i64, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ptk_sample_bwd": (C.c_int, [_vp, _vp, _vp, _vp, _i64, _i64, _i64, _i64, _vp, _vp]),

@@ -308,22 +308,98 @@ class _KNN(torch.autograd.Function):
         return g1, g2, None, None, None
 
 
-def knn(p1, p2, K, lengths1=None, lengths2=None):
-    """dists (B,P1,K) f32, idx (B,P1,K) int32: the K nearest p2 points of every p1 point, ascending distance and the
-    lower index first on equal distances (include/ptk.h), 1 <= K <= 64.  Column 0 is knn1().  dists is differentiable
-    w.r.t. p1 and p2 (deterministic under torch.use_deterministic_algorithms(True)); idx is not.  lengths1 / lengths2
-    as in knn1(): padded queries get (0, 0) in every slot, slots k >= lengths2[b] get (0, 0), and neither passes a
-    gradient.  K = 1 runs knn1()."""
+def _check_knn_k(K):
     if isinstance(K, bool) or not isinstance(K, int):
         raise ValueError(f"K must be an int, got {K!r}")
     if K < 1:
         raise ValueError(f"K must be >= 1, got {K}")
     if K > _lib.KNN_MAX_K:
         raise NotImplementedError(f"ptk_b200 knn supports K <= {_lib.KNN_MAX_K}, got K={K}")
+
+
+def knn(p1, p2, K, lengths1=None, lengths2=None):
+    """dists (B,P1,K) f32, idx (B,P1,K) int32: the K nearest p2 points of every p1 point, ascending distance and the
+    lower index first on equal distances (include/ptk.h), 1 <= K <= 64.  Column 0 is knn1().  dists is differentiable
+    w.r.t. p1 and p2 (deterministic under torch.use_deterministic_algorithms(True)); idx is not.  lengths1 / lengths2
+    as in knn1(): padded queries get (0, 0) in every slot, slots k >= lengths2[b] get (0, 0), and neither passes a
+    gradient.  K = 1 runs knn1()."""
+    _check_knn_k(K)
     if K == 1:
         dist, idx = knn1(p1, p2, lengths1, lengths2)
         return dist[..., None], idx[..., None]
     return _KNN.apply(p1, p2, K, lengths1, lengths2)
+
+
+class _PointFrames(torch.autograd.Function):
+    """normals (frames=False) or (curvatures, frames) of estimate_normals / estimate_local_frames, differentiable w.r.t.
+    the points.  The K-NN runs on the detached points: idx is piecewise constant and the backward differentiates the
+    covariance of the neighbourhood it selects."""
+
+    @staticmethod
+    def forward(ctx, points, lengths, K, disambiguate, frames):
+        B, P, _ = points.shape
+        pts = points.detach()
+        dist, idx = knn(pts, pts, K, lengths, lengths)
+        normals = curv = fr = None
+        if frames:
+            curv = torch.empty(B, P, 3, dtype=torch.float32, device=points.device)
+            fr = torch.empty(B, P, 3, 3, dtype=torch.float32, device=points.device)
+        else:
+            normals = torch.empty(B, P, 3, dtype=torch.float32, device=points.device)
+        with torch.cuda.device(points.device):
+            _lib.check(_lib.lib().ptk_point_frames_fwd(_p(pts), _p(lengths), _p(idx), _p(dist), B, P, K,
+                                                       int(disambiguate), _p(normals), _p(curv), _p(fr), _stream()),
+                       "ptk_point_frames_fwd")
+        ctx.save_for_backward(pts, lengths, idx, dist)
+        ctx.K, ctx.disambiguate, ctx.frames = K, int(disambiguate), frames
+        ctx.set_materialize_grads(False)
+        return (curv, fr) if frames else normals
+
+    @staticmethod
+    def backward(ctx, *grads):
+        pts, lengths, idx, dist = ctx.saved_tensors
+        if not ctx.needs_input_grad[0] or all(g is None for g in grads):
+            return None, None, None, None, None
+        gn, gc, gf = (None,) + tuple(grads) if ctx.frames else (grads[0], None, None)
+        gn, gc, gf = (_f32c(g) if g is not None else None for g in (gn, gc, gf))
+        B, P, _ = pts.shape
+        gp = torch.empty_like(pts)
+        L = _lib.lib()
+        args = (_p(pts), _p(lengths), _p(idx), _p(dist), B, P, ctx.K, ctx.disambiguate, _p(gn), _p(gc), _p(gf), _p(gp))
+        with torch.cuda.device(pts.device):
+            if _deterministic():
+                ws = _ws(L.ptk_knn1_bwd_det_workspace_bytes(B, P, P), pts.device)
+                _lib.check(L.ptk_point_frames_bwd_det(*args, _p(ws), ws.numel(), _stream()), "ptk_point_frames_bwd_det")
+            else:
+                _lib.check(L.ptk_point_frames_bwd(*args, _stream()), "ptk_point_frames_bwd")
+        return gp, None, None, None, None
+
+
+def _point_frames(points, lengths, neighborhood_size, disambiguate_directions, frames):
+    _check_knn_k(neighborhood_size)
+    if not torch.is_tensor(points) or points.dim() != 3 or points.shape[2] != 3:
+        raise ValueError(f"points must be a (B,P,3) tensor, got {getattr(points, 'shape', type(points).__name__)}")
+    _need_cuda(points)
+    lengths = _lengths(lengths, points.shape[0], points.device, "lengths")
+    return _PointFrames.apply(_f32c(points), lengths, neighborhood_size, bool(disambiguate_directions), frames)
+
+
+def estimate_normals(points, lengths=None, neighborhood_size=50, disambiguate_directions=True):
+    """normals (B,P,3) f32: PyTorch3D 0.5.0's estimate_pointcloud_normals on a (B,P,3) cloud (include/ptk.h:
+    ptk_point_frames_fwd).  Each point's unit normal is the eigenvector of the smallest eigenvalue of the covariance of
+    its min(neighborhood_size, lengths[b]) nearest neighbours (itself included), signed so that at least half of the
+    neighbours lie on its positive side when disambiguate_directions.  lengths (B,) as in knn(): padded points get 0;
+    a point whose neighbourhood has a non-finite distance gets NaN.  1 <= neighborhood_size <= 64.  Differentiable
+    w.r.t. points (deterministic under torch.use_deterministic_algorithms(True))."""
+    return _point_frames(points, lengths, neighborhood_size, disambiguate_directions, False)
+
+
+def estimate_local_frames(points, lengths=None, neighborhood_size=50, disambiguate_directions=True):
+    """(curvatures (B,P,3), frames (B,P,3,3)): PyTorch3D 0.5.0's estimate_pointcloud_local_coord_frames.  curvatures
+    are the ascending eigenvalues of each point's neighbourhood covariance; frames[b,i] has the columns (normal, y, z)
+    with y = normal x z (disambiguated) or the three eigenvectors (not), and frames[..., 0] equals estimate_normals()
+    bit for bit.  Arguments, padding and NaN as in estimate_normals(); both outputs are differentiable w.r.t. points."""
+    return _point_frames(points, lengths, neighborhood_size, disambiguate_directions, True)
 
 
 # ------------------------------------------------------------------------------------- vertex max-pool

@@ -278,6 +278,61 @@ int ptk_knn_bwd_det(const float *p1, const float *p2, const int64_t *len1, const
                     const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K, float *grad_p1, float *grad_p2,
                     void *workspace, size_t workspace_bytes, ptk_stream_t stream);
 
+/* Point-cloud normals and local coordinate frames: pytorch3d.ops.estimate_pointcloud_normals and
+ * estimate_pointcloud_local_coord_frames of PyTorch3D 0.5.0 (points_normals.py), on idx / dist (B,P,K) of
+ * ptk_knn_fwd_lengths(points, points, lengths, lengths, K).  points (B,P,3); lengths as for the ragged calls above.
+ * For cloud b write l = lengths[b] and K' = min(K, l).  For a valid query i < l, with q_k = points[b, idx[b,i,k]]:
+ *     d_k = q_k - p_i,  m = (1/K') sum_{k<K'} d_k,  C = (1/K') sum_{k<K'} (d_k - m)(d_k - m)^T
+ * (the covariance of the neighbours about their mean, computed relative to the query: C is translation invariant).
+ * The eigenpairs (lam_m, v_m) of C, lam_0 <= lam_1 <= lam_2, come from a cyclic Jacobi solver with a fixed number of
+ * sweeps (so NaN input cannot make it loop); v_0 is normalised, v_2 orthogonalised against it and normalised, and
+ * v_1 = v_2 x v_0.  curvatures[b,i] = (lam_0, lam_1, lam_2).
+ *   - disambiguate != 0 (PyTorch3D's default): for v in {v_0, v_2}, n_pos = #{k < K' : v . d_k > 0}; v is negated when
+ *     n_pos < 0.5 K'.  This gives n (from v_0) and z (from v_2); y = n x z and frames[b,i] has the columns (n, y, z).
+ *   - disambiguate == 0: frames[b,i] has the columns (v_0, v_1, v_2) with the solver's signs.
+ *   - normals[b,i] = frames[b,i][:, 0], bit for bit; frames[b,i,r,c] is component r of column c.
+ *   - repeated eigenvalues (C = 0 at K' = 1, exactly planar or collinear neighbourhoods): any orthonormal basis of the
+ *     eigenspace; the result is still finite, unit-length, orthonormal and a deterministic function of the input.
+ *   - padded queries (i >= l): every output is 0.
+ *   - a query with a slot k < K' whose distance is not finite (a NaN / Inf point, or a slot left at (+inf, 0) by the
+ *     K-NN) gets NaN in every output.  A NaN point never enters another query's neighbourhood, so it changes nothing
+ *     else.  l <= K is not an error (K' handles it) and needs no host synchronisation.
+ * ptk_point_frames_fwd writes normals (may be NULL) and / or curvatures (B,P,3) with frames (B,P,3,3) (both NULL or
+ * both given); at least one output.  One kernel, one thread per query, PDL-chained, capture-safe.
+ * PTK_ERR_SHAPE for a null points / idx / dist / output pointer, an empty or too large shape, B > 65535 or K outside
+ * [1, PTK_KNN_MAX_K]. */
+int ptk_point_frames_fwd(const float *points, const int64_t *lengths, const int32_t *idx, const float *dist, int64_t B,
+                         int64_t P, int64_t K, int disambiguate, float *normals, float *curvatures, float *frames,
+                         ptk_stream_t stream);
+/* Gradient of the outputs above w.r.t. points under grad_normals (B,P,3), grad_curvatures (B,P,3) and grad_frames
+ * (B,P,3,3), any of which may be NULL (zero).  The eigensystem is recomputed with the forward's arithmetic; nothing but
+ * the inputs is saved.  Per valid query, gV folds the upstream gradients into the eigenvectors: with disambiguate,
+ * g_n += z x g_y and g_z += g_y x n (y = n x z), then g_v0 = s_0 g_n and g_v2 = s_2 g_z (s = the signs applied);
+ * without it g_v0 / g_v1 / g_v2 are the frame columns' gradients.  Normals add to g_n (resp. g_v0).  Then, as
+ * torch.linalg.eigh's backward,
+ *     G = V (diag(g_lam) + F o (V^T gV)) V^T,  F_mn = 1 / (lam_n - lam_m) for m != n, 0 on the diagonal,
+ * where F_mn is taken as 0 when lam_n == lam_m in fp32 (a repeated eigenspace has no defined gradient), and slot k adds
+ *     (1/K') (G + G^T) (q_k - mean of the q)
+ * to the gradient of point idx[b,i,k].  Terms that are zero analytically are left out: those through the mean (the
+ * centred neighbours sum to zero), through the query's own p_i (C is translation invariant) and through the sign rule
+ * (a step function).  Padded queries and queries with NaN outputs pass no gradient.  grad_points (B,P,3) is fully
+ * overwritten; padded rows are +0.  PTK_ERR_SHAPE as for the forward and for a null grad_points pointer.  No host
+ * synchronisation, capture-safe.
+ * ptk_point_frames_bwd: a memset and one kernel, the terms added with fp32 atomics (low bits vary from run to run).
+ * ptk_point_frames_bwd_det: the scheme of ptk_knn_bwd_det per cloud b: M_b = the largest finite |term|,
+ * e_b = 62 - ceil(log2 M_b) - ceil(log2(l + 1)) (a query's K' indices are distinct, so a point receives at most l
+ * terms), exact int64 sums of round_half_even(term * 2^e_b), grad = ldexpf((float)sum, -e_b); non-finite terms bypass
+ * the integer sum.  Bits depend neither on scheduling nor on the batch or the order of the points.  workspace:
+ * 16-byte aligned, ptk_knn1_bwd_det_workspace_bytes(B, P, P) (the same layout); PTK_ERR_WORKSPACE when missing or too
+ * small, PTK_ERR_ALIGN when misaligned.  A memset and three kernels. */
+int ptk_point_frames_bwd(const float *points, const int64_t *lengths, const int32_t *idx, const float *dist, int64_t B,
+                         int64_t P, int64_t K, int disambiguate, const float *grad_normals, const float *grad_curvatures,
+                         const float *grad_frames, float *grad_points, ptk_stream_t stream);
+int ptk_point_frames_bwd_det(const float *points, const int64_t *lengths, const int32_t *idx, const float *dist,
+                             int64_t B, int64_t P, int64_t K, int disambiguate, const float *grad_normals,
+                             const float *grad_curvatures, const float *grad_frames, float *grad_points,
+                             void *workspace, size_t workspace_bytes, ptk_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Area-weighted surface sampling.  Replaces the body of utils.batch_sample
  * (pterotactyl/utility/utils.py:152-187): pytorch3d mesh_face_areas_normals (utils.py:164), the NaN
