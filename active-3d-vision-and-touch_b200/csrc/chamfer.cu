@@ -38,7 +38,7 @@
 
 #include "chamfer_kernel2.cuh"
 #include "chamfer_pruned.cuh"
-#include "det_accum.cuh"
+#include "pair_bwd.cuh"
 
 namespace ptk {
 
@@ -211,329 +211,21 @@ chamfer_finalize_sum_kernel(const float *__restrict__ partial, int B, int nsp, i
     cham[b] = chamfer_reduce(sx, sy, L1, L2, mean);
 }
 
-// Backward, phase A (plain stores): the "own point" terms, s_x = 2 g[b] / max(lx, 1) (mean) or 2 g[b] (sum).
-//   grad_x[b,i] = s_x * (x_i - y[idx_x[i]]);  grad_y[b,j] = s_y * (y_j - x[idx_y[j]])
-// Padded points (i >= len) and points whose target cloud is empty get 0: every row is written.
-__global__ void chamfer_bwd_direct_kernel(const float *__restrict__ x, const float *__restrict__ y,
-                                          const int32_t *__restrict__ idx_x,
-                                          const int32_t *__restrict__ idx_y,
-                                          const float *__restrict__ grad_cham, int P1, int P2,
-                                          const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
-                                          float *__restrict__ grad_x, float *__restrict__ grad_y) {
-    pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const float g = grad_cham[b];
-    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    if (grad_x && i < P1) {
-        float *o = grad_x + ((size_t)b * P1 + i) * 3;
-        if (i < L1 && L2 > 0) {
-            const int j = idx_x[(size_t)b * P1 + i];
-            const float s = mean ? 2.0f * (g / (float)L1) : 2.0f * g;
-            o[0] = s * (xb[i * 3 + 0] - yb[j * 3 + 0]);
-            o[1] = s * (xb[i * 3 + 1] - yb[j * 3 + 1]);
-            o[2] = s * (xb[i * 3 + 2] - yb[j * 3 + 2]);
-        } else {
-            o[0] = o[1] = o[2] = 0.f;
-        }
-    }
-    if (grad_y && i < P2) {
-        float *o = grad_y + ((size_t)b * P2 + i) * 3;
-        if (i < L2 && L1 > 0) {
-            const int j = idx_y[(size_t)b * P2 + i];
-            const float s = mean ? 2.0f * (g / (float)L2) : 2.0f * g;
-            o[0] = s * (yb[i * 3 + 0] - xb[j * 3 + 0]);
-            o[1] = s * (yb[i * 3 + 1] - xb[j * 3 + 1]);
-            o[2] = s * (yb[i * 3 + 2] - xb[j * 3 + 2]);
-        } else {
-            o[0] = o[1] = o[2] = 0.f;
-        }
-    }
-}
-
-// Backward, phase B (scatter): the "I am somebody's nearest neighbour" terms, RED.ADD.F32, from valid queries with a
-// non-empty target cloud only.
-//   grad_y[b, idx_x[i]] -= s_x (x_i - y[idx_x[i]]);  grad_x[b, idx_y[j]] -= s_y (y_j - x[idx_y[j]])
-__global__ void chamfer_bwd_scatter_kernel(const float *__restrict__ x, const float *__restrict__ y,
-                                           const int32_t *__restrict__ idx_x,
-                                           const int32_t *__restrict__ idx_y,
-                                           const float *__restrict__ grad_cham, int P1, int P2,
-                                           const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
-                                           float *__restrict__ grad_x, float *__restrict__ grad_y) {
-    pdl_wait();  // launched with programmatic stream serialization (ptk_common.cuh)
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const float g = grad_cham[b];
-    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    if (grad_y && i < L1 && L2 > 0) {
-        const int j = idx_x[(size_t)b * P1 + i];
-        const float s = mean ? 2.0f * (g / (float)L1) : 2.0f * g;
-        float *o = grad_y + ((size_t)b * P2 + j) * 3;
-        atomicAdd(o + 0, -(s * (xb[i * 3 + 0] - yb[j * 3 + 0])));
-        atomicAdd(o + 1, -(s * (xb[i * 3 + 1] - yb[j * 3 + 1])));
-        atomicAdd(o + 2, -(s * (xb[i * 3 + 2] - yb[j * 3 + 2])));
-    }
-    if (grad_x && i < L2 && L1 > 0) {
-        const int j = idx_y[(size_t)b * P2 + i];
-        const float s = mean ? 2.0f * (g / (float)L2) : 2.0f * g;
-        float *o = grad_x + ((size_t)b * P1 + j) * 3;
-        atomicAdd(o + 0, -(s * (yb[i * 3 + 0] - xb[j * 3 + 0])));
-        atomicAdd(o + 1, -(s * (yb[i * 3 + 1] - xb[j * 3 + 1])));
-        atomicAdd(o + 2, -(s * (yb[i * 3 + 2] - xb[j * 3 + 2])));
-    }
-}
-
-// Deterministic backward (ptk_chamfer_bwd_det, scheme in det_accum.cuh): three kernels, grid = (ceil(max(P1,P2) / 256), B).
-// Thread i owns x-query i and y-query i.  A valid query's own term is s * (q - t[idx]) per component, with s and the
-// arithmetic of chamfer_bwd_direct_kernel; it goes to the query's row and, negated, to its nearest neighbour's row.
-// M_b and the scatter into one cloud always take the terms of both directions, so each gradient has the same bits
-// whether or not the other one is requested.  A row of x receives at most ly + 1 terms, a row of y lx + 1.
-constexpr int CD_THREADS = 256;
-
-// the three components of query i's own term (dir 0: x-query against y, dir 1: y-query against x); false: no term
+// Backward (pair_bwd.cuh): a valid query's own term is s * (q - t[idx]) per component, s = 2 g[b] / max(lq, 1) (mean) or
+// 2 g[b] (sum); it goes to the query's row and, negated, to its nearest neighbour's row.  Padded points and points
+// whose target cloud is empty have no term.
 __device__ __forceinline__ bool chamfer_own_term(const float *__restrict__ qb, const float *__restrict__ tb,
                                                  const int32_t *__restrict__ idx, float g, int i, int Lq, int Lt,
-                                                 int mean, int &j, float t[3]) {
+                                                 int mean, int &j, float own[3], float near[3]) {
     if (i >= Lq || Lt <= 0) return false;
     j = idx[i];
     const float s = mean ? 2.0f * (g / (float)Lq) : 2.0f * g;
-    t[0] = s * (qb[i * 3 + 0] - tb[j * 3 + 0]);
-    t[1] = s * (qb[i * 3 + 1] - tb[j * 3 + 1]);
-    t[2] = s * (qb[i * 3 + 2] - tb[j * 3 + 2]);
-    return true;
-}
-
-// phase 1: M_b (atomicMax into mbits[b], zeroed by the caller); zero the accumulators and the outputs of every row
-__global__ void __launch_bounds__(CD_THREADS)
-chamfer_bwd_det_terms_kernel(const float *__restrict__ x, const float *__restrict__ y, const int32_t *__restrict__ idx_x,
-                             const int32_t *__restrict__ idx_y, const float *__restrict__ grad_cham, int P1, int P2,
-                             const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
-                             float *__restrict__ grad_x, float *__restrict__ grad_y, unsigned long long *__restrict__ acc_x,
-                             unsigned long long *__restrict__ acc_y, unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const float g = grad_cham[b];
-    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    float m = 0.0f, t[3];
-    int j;
-    if (chamfer_own_term(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, t))
-        m = fmaxf(m, fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2]))));
-    if (chamfer_own_term(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, t))
-        m = fmaxf(m, fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2]))));
-    if (grad_x && i < P1) {
-        const size_t r = ((size_t)b * P1 + i) * 3;
-        acc_x[r + 0] = acc_x[r + 1] = acc_x[r + 2] = 0ull;
-        grad_x[r + 0] = grad_x[r + 1] = grad_x[r + 2] = 0.0f;
-    }
-    if (grad_y && i < P2) {
-        const size_t r = ((size_t)b * P2 + i) * 3;
-        acc_y[r + 0] = acc_y[r + 1] = acc_y[r + 2] = 0ull;
-        grad_y[r + 0] = grad_y[r + 1] = grad_y[r + 2] = 0.0f;
-    }
-    det_block_max<CD_THREADS>(m, mbits + b);
-}
-
-// the own term of one query into its row (acc_q / out_q) and, negated, into its neighbour's row (acc_t / out_t)
-__device__ __forceinline__ void chamfer_det_add(const float t[3], double scale, unsigned long long *acc_q, float *out_q,
-                                                unsigned long long *acc_t, float *out_t) {
 #pragma unroll
     for (int d = 0; d < 3; ++d) {
-        if (isfinite(t[d])) {
-            const unsigned long long q = det_quantise(t[d], scale);
-            if (acc_q) atomicAdd(acc_q + d, q);
-            if (acc_t) atomicAdd(acc_t + d, 0ull - q);
-        } else {
-            if (out_q) atomicAdd(out_q + d, t[d]);
-            if (out_t) atomicAdd(out_t + d, -t[d]);
-        }
+        own[d] = s * (qb[i * 3 + d] - tb[j * 3 + d]);
+        near[d] = -own[d];
     }
-}
-
-// phase 2: quantise and add (64-bit reductions; non-finite terms into the outputs)
-__global__ void __launch_bounds__(CD_THREADS)
-chamfer_bwd_det_reduce_kernel(const float *__restrict__ x, const float *__restrict__ y, const int32_t *__restrict__ idx_x,
-                              const int32_t *__restrict__ idx_y, const float *__restrict__ grad_cham, int P1, int P2,
-                              const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y, int mean,
-                              float *__restrict__ grad_x, float *__restrict__ grad_y,
-                              unsigned long long *__restrict__ acc_x, unsigned long long *__restrict__ acc_y,
-                              const unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const float g = grad_cham[b];
-    const float *xb = x + (size_t)b * P1 * 3, *yb = y + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)max(L1, L2) + 1));
-    const size_t bx = (size_t)b * P1 * 3, by = (size_t)b * P2 * 3;
-    float t[3];
-    int j;
-    if (chamfer_own_term(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, t))
-        chamfer_det_add(t, scale, acc_x ? acc_x + bx + (size_t)i * 3 : nullptr, grad_x ? grad_x + bx + (size_t)i * 3 : nullptr,
-                        acc_y ? acc_y + by + (size_t)j * 3 : nullptr, grad_y ? grad_y + by + (size_t)j * 3 : nullptr);
-    if (chamfer_own_term(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, t))
-        chamfer_det_add(t, scale, acc_y ? acc_y + by + (size_t)i * 3 : nullptr, grad_y ? grad_y + by + (size_t)i * 3 : nullptr,
-                        acc_x ? acc_x + bx + (size_t)j * 3 : nullptr, grad_x ? grad_x + bx + (size_t)j * 3 : nullptr);
-}
-
-// phase 3: grad = fp32(acc) * 2^-e_b, unless the row's output already holds a non-finite sum
-__global__ void __launch_bounds__(CD_THREADS)
-chamfer_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len_x, const int64_t *__restrict__ len_y,
-                               const unsigned int *__restrict__ mbits, const unsigned long long *__restrict__ acc_x,
-                               const unsigned long long *__restrict__ acc_y, float *__restrict__ grad_x,
-                               float *__restrict__ grad_y) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    const int e = det_exponent(mbits[b], (long long)max(L1, L2) + 1);
-    if (grad_x && i < P1) {
-        const size_t r = ((size_t)b * P1 + i) * 3;
-        for (int d = 0; d < 3; ++d) det_convert(grad_x + r + d, acc_x + r + d, e);
-    }
-    if (grad_y && i < P2) {
-        const size_t r = ((size_t)b * P2 + i) * 3;
-        for (int d = 0; d < 3; ++d) det_convert(grad_y + r + d, acc_y + r + d, e);
-    }
-}
-
-// 1-NN backward (ptk_knn1_bwd_lengths, ptk_knn1_bwd_det): the gradient of dist[b,i] = |p1_i - p2_j|^2, j = idx[b,i],
-// under a per-query upstream gradient g[b,i].  A valid query's term is s * (p1_i - p2_j) per component, s = 2 g[b,i]
-// (the fp32 operations of PyTorch3D's knn_points_backward and of chamfer_own_term); it is the whole gradient of p1 row i
-// and goes, negated, to p2 row j.  Padded queries and queries with an empty target cloud have no term (g is not read).
-__device__ __forceinline__ bool knn1_term(const float *__restrict__ p1b, const float *__restrict__ p2b,
-                                          const int32_t *__restrict__ idx, const float *__restrict__ g, int i, int L1,
-                                          int L2, int &j, float t[3]) {
-    if (i >= L1 || L2 <= 0) return false;
-    j = idx[i];
-    const float s = 2.0f * g[i];
-    t[0] = s * (p1b[i * 3 + 0] - p2b[j * 3 + 0]);
-    t[1] = s * (p1b[i * 3 + 1] - p2b[j * 3 + 1]);
-    t[2] = s * (p1b[i * 3 + 2] - p2b[j * 3 + 2]);
     return true;
-}
-
-// phase A, grid = (ceil(max(P1,P2) / 256), B): grad_p1 rows (the term, or 0), grad_p2 rows zeroed for phase B
-__global__ void __launch_bounds__(CD_THREADS)
-knn1_bwd_direct_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
-                       const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
-                       const int64_t *__restrict__ len2, float *__restrict__ grad_p1, float *__restrict__ grad_p2) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
-    if (grad_p1 && i < P1) {
-        float *o = grad_p1 + ((size_t)b * P1 + i) * 3;
-        float t[3];
-        int j;
-        if (knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i,
-                      L1, L2, j, t)) {
-            o[0] = t[0];
-            o[1] = t[1];
-            o[2] = t[2];
-        } else {
-            o[0] = o[1] = o[2] = 0.0f;
-        }
-    }
-    if (grad_p2 && i < P2) {
-        float *o = grad_p2 + ((size_t)b * P2 + i) * 3;
-        o[0] = o[1] = o[2] = 0.0f;
-    }
-}
-
-// phase B, grid = (ceil(P1 / 256), B): grad_p2[b, j] -= term, RED.ADD.F32
-__global__ void __launch_bounds__(CD_THREADS)
-knn1_bwd_scatter_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
-                        const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
-                        const int64_t *__restrict__ len2, float *__restrict__ grad_p2) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
-    float t[3];
-    int j;
-    if (knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i, L1,
-                  L2, j, t)) {
-        float *o = grad_p2 + ((size_t)b * P2 + j) * 3;
-        atomicAdd(o + 0, -t[0]);
-        atomicAdd(o + 1, -t[1]);
-        atomicAdd(o + 2, -t[2]);
-    }
-}
-
-// Deterministic form (scheme in det_accum.cuh): a p1 row holds one term, so grad_p1 is phase A's plain store; only
-// grad_p2 goes through the integer sum.  M_b = the largest finite |term| of pair b, e_b from n = l1 + 1 (a p2 row
-// receives at most l1 terms).
-// phase 1, grid = (ceil(max(P1,P2) / 256), B): M_b (atomicMax into mbits[b], zeroed by the caller), grad_p1 as in phase A,
-// accumulators and outputs of every p2 row zeroed
-__global__ void __launch_bounds__(CD_THREADS)
-knn1_bwd_det_terms_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
-                          const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
-                          const int64_t *__restrict__ len2, float *__restrict__ grad_p1, float *__restrict__ grad_p2,
-                          unsigned long long *__restrict__ acc, unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
-    float m = 0.0f, t[3];
-    int j;
-    const bool term = knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1,
-                                grad_dist + (size_t)b * P1, i, L1, L2, j, t);
-    if (term) m = fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2])));
-    if (grad_p1 && i < P1) {
-        float *o = grad_p1 + ((size_t)b * P1 + i) * 3;
-        o[0] = term ? t[0] : 0.0f;
-        o[1] = term ? t[1] : 0.0f;
-        o[2] = term ? t[2] : 0.0f;
-    }
-    if (i < P2) {
-        const size_t r = ((size_t)b * P2 + i) * 3;
-        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
-        grad_p2[r + 0] = grad_p2[r + 1] = grad_p2[r + 2] = 0.0f;
-    }
-    det_block_max<CD_THREADS>(m, mbits + b);
-}
-
-// phase 2, grid = (ceil(P1 / 256), B): quantise and add into the neighbour's row (non-finite terms into grad_p2)
-__global__ void __launch_bounds__(CD_THREADS)
-knn1_bwd_det_reduce_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
-                           const float *__restrict__ grad_dist, int P1, int P2, const int64_t *__restrict__ len1,
-                           const int64_t *__restrict__ len2, float *__restrict__ grad_p2,
-                           unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    const int L1 = pair_len(len1, b, P1), L2 = pair_len(len2, b, P2);
-    float t[3];
-    int j;
-    if (!knn1_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1, grad_dist + (size_t)b * P1, i,
-                   L1, L2, j, t))
-        return;
-    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)L1 + 1));
-    const size_t r = ((size_t)b * P2 + j) * 3;
-#pragma unroll
-    for (int d = 0; d < 3; ++d) {
-        if (isfinite(t[d]))
-            atomicAdd(acc + r + d, 0ull - det_quantise(t[d], scale));
-        else
-            atomicAdd(grad_p2 + r + d, -t[d]);
-    }
-}
-
-// phase 3, grid = (ceil(P2 / 256), B): grad_p2 = fp32(acc) * 2^-e_b, unless the row already holds a non-finite sum
-__global__ void __launch_bounds__(CD_THREADS)
-knn1_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len1, const unsigned int *__restrict__ mbits,
-                            const unsigned long long *__restrict__ acc, float *__restrict__ grad_p2) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CD_THREADS + threadIdx.x;
-    if (i >= P2) return;
-    const int e = det_exponent(mbits[b], (long long)pair_len(len1, b, P1) + 1);
-    const size_t r = ((size_t)b * P2 + i) * 3;
-    for (int d = 0; d < 3; ++d) det_convert(grad_p2 + r + d, acc + r + d, e);
 }
 
 // ---------------------------------------------------------------------------------------- host side
@@ -891,18 +583,9 @@ static int chamfer_bwd(const float *x, const float *y, const int64_t *len_x, con
     if (rc) return rc;
     PTK_REQUIRE(idx_x && idx_y && grad_cham, PTK_ERR_SHAPE, "chamfer_bwd: null index / grad pointer");
     if (!grad_x && !grad_y) return PTK_OK;
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    dim3 grid((unsigned)ceil_div(Pm, 256), (unsigned)B);
     PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "chamfer_bwd: batch too large");
-    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
-    launch_pdl(chamfer_bwd_direct_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, len_x, len_y,
-               mean, grad_x, grad_y);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_bwd_scatter_kernel, grid, dim3(256), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2, len_x, len_y,
-               mean, grad_x, grad_y);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
+    return pair_bwd<chamfer_own_term>(x, y, len_x, len_y, idx_x, idx_y, grad_cham, B, P1, P2,
+                                  reduction == PTK_REDUCE_MEAN ? 1 : 0, grad_x, grad_y, as_stream(stream));
 }
 
 extern "C" int ptk_chamfer_bwd(const float *x, const float *y, const int32_t *idx_x,
@@ -920,11 +603,9 @@ extern "C" int ptk_chamfer_bwd_lengths(const float *x, const float *y, const int
     return chamfer_bwd(x, y, len_x, len_y, idx_x, idx_y, grad_cham, B, P1, P2, reduction, grad_x, grad_y, stream);
 }
 
-// det workspace: [M_b bits B, padded to 256 bytes][acc_x B*P1*3 int64][acc_y B*P2*3 int64]
-
 extern "C" size_t ptk_chamfer_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
     if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;
-    return det_align(4 * (size_t)B) + det_align(24 * (size_t)B * P1) + 24 * (size_t)B * P2;
+    return det_workspace_bytes(B, P1, P2);
 }
 
 extern "C" int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t *len_x, const int64_t *len_y,
@@ -938,103 +619,9 @@ extern "C" int ptk_chamfer_bwd_det(const float *x, const float *y, const int64_t
     if (rc) return rc;
     PTK_REQUIRE(idx_x && idx_y && grad_cham, PTK_ERR_SHAPE, "chamfer_bwd_det: null index / grad pointer");
     if (!grad_x && !grad_y) return PTK_OK;
-    const size_t need = ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "chamfer_bwd_det: workspace too small (%zu < %zu)",
-                workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "chamfer_bwd_det: workspace must be 16-byte aligned");
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2), "chamfer_bwd_det");
+    if (rc) return rc;
     PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "chamfer_bwd_det: batch too large");
-    char *p = reinterpret_cast<char *>(workspace);
-    auto *mbits = reinterpret_cast<unsigned int *>(p);
-    auto *acc_x = grad_x ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B)) : nullptr;
-    auto *acc_y = grad_y ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B) + det_align(24 * (size_t)B * P1))
-                         : nullptr;
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    const dim3 grid((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B);
-    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
-    launch_pdl(chamfer_bwd_det_terms_kernel, grid, dim3(CD_THREADS), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2,
-               len_x, len_y, mean, grad_x, grad_y, acc_x, acc_y, mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_bwd_det_reduce_kernel, grid, dim3(CD_THREADS), 0, st, x, y, idx_x, idx_y, grad_cham, (int)P1, (int)P2,
-               len_x, len_y, mean, grad_x, grad_y, acc_x, acc_y, (const unsigned int *)mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_bwd_det_convert_kernel, grid, dim3(CD_THREADS), 0, st, (int)P1, (int)P2, len_x, len_y,
-               (const unsigned int *)mbits, (const unsigned long long *)acc_x, (const unsigned long long *)acc_y, grad_x, grad_y);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
-}
-
-static int knn1_bwd_check(const float *p1, const float *p2, const int32_t *idx, const float *grad_dist, int64_t B,
-                          int64_t P1, int64_t P2) {
-    int rc = check_clouds(p1, p2, B, P1, P2);
-    if (rc) return rc;
-    PTK_REQUIRE(idx && grad_dist, PTK_ERR_SHAPE, "knn1_bwd: null index / grad pointer");
-    return PTK_OK;
-}
-
-extern "C" int ptk_knn1_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
-                                    const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
-                                    float *grad_p1, float *grad_p2, ptk_stream_t stream) {
-    PTK_NVTX("ptk_knn1_bwd_lengths");
-    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
-    if (rc) return rc;
-    if (!grad_p1 && !grad_p2) return PTK_OK;
-    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd: batch too large");
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    launch_pdl(knn1_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1, p2,
-               idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, grad_p2);
-    PTK_CHECK_LAUNCH();
-    if (grad_p2) {
-        launch_pdl(knn1_bwd_scatter_kernel, dim3((unsigned)ceil_div(P1, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
-                   p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p2);
-        PTK_CHECK_LAUNCH();
-    }
-    return PTK_OK;
-}
-
-// det workspace: [M_b bits B, padded to 256 bytes][acc_p2 B*P2*3 int64]
-extern "C" size_t ptk_knn1_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
-    if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;
-    return det_align(4 * (size_t)B) + 24 * (size_t)B * P2;
-}
-
-extern "C" int ptk_knn1_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
-                                const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
-                                float *grad_p1, float *grad_p2, void *workspace, size_t workspace_bytes,
-                                ptk_stream_t stream) {
-    PTK_NVTX("ptk_knn1_bwd_det");
-    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
-    if (rc) return rc;
-    if (!grad_p1 && !grad_p2) return PTK_OK;
-    const size_t need = ptk_knn1_bwd_det_workspace_bytes(B, P1, P2);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "knn1_bwd_det: workspace too small (%zu < %zu)",
-                workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "knn1_bwd_det: workspace must be 16-byte aligned");
-    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd_det: batch too large");
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    if (!grad_p2) {  // grad_p1 alone: plain stores, nothing to sum
-        launch_pdl(knn1_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
-                   p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, (float *)nullptr);
-        PTK_CHECK_LAUNCH();
-        return PTK_OK;
-    }
-    char *p = reinterpret_cast<char *>(workspace);
-    auto *mbits = reinterpret_cast<unsigned int *>(p);
-    auto *acc = reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B));
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
-    launch_pdl(knn1_bwd_det_terms_kernel, dim3((unsigned)ceil_div(Pm, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
-               p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p1, grad_p2, acc, mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(knn1_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(P1, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st, p1,
-               p2, idx, grad_dist, (int)P1, (int)P2, len1, len2, grad_p2, acc, (const unsigned int *)mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(knn1_bwd_det_convert_kernel, dim3((unsigned)ceil_div(P2, CD_THREADS), (unsigned)B), dim3(CD_THREADS), 0, st,
-               (int)P1, (int)P2, len1, (const unsigned int *)mbits, (const unsigned long long *)acc, grad_p2);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
+    return pair_bwd_det<chamfer_own_term>(x, y, len_x, len_y, idx_x, idx_y, grad_cham, B, P1, P2,
+                                      reduction == PTK_REDUCE_MEAN ? 1 : 0, grad_x, grad_y, workspace, as_stream(stream));
 }

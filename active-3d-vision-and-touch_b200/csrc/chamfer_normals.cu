@@ -10,13 +10,11 @@
 // and reduces each pair in the fixed order of chamfer_finalize_kernel (fin_splits of the pair's own lengths, slice
 // partials added in slice order).  The backward splits a term's gradient into an "own" part on the query's normal row
 // and a "near" part on the gathered normal's row, recomputing c from the normals.
-#include "det_accum.cuh"
-#include "nn_common.cuh"
+#include "pair_bwd.cuh"
 
 namespace ptk {
 
 constexpr float CN_EPS = 1e-6f;  // F.cosine_similarity's default eps, clamped per norm
-constexpr int CN_THREADS = 256;  // backward kernels: thread i owns x-query i and y-query i
 
 __device__ __forceinline__ void load_normal(const float *__restrict__ p, int i, float v[3]) {
     v[0] = p[i * 3 + 0];
@@ -149,168 +147,6 @@ __device__ __forceinline__ bool normal_parts(const float *__restrict__ qn, const
     return true;
 }
 
-// Default backward, phase A, grid = (ceil(max(P1,P2) / 256), B): every row of the requested gradients gets its own
-// part (a plain store: one per row) or 0
-__global__ void __launch_bounds__(CN_THREADS)
-chamfer_normals_bwd_own_kernel(const float *__restrict__ xn, const float *__restrict__ yn,
-                               const int32_t *__restrict__ idx_x, const int32_t *__restrict__ idx_y,
-                               const float *__restrict__ grad_cn, int P1, int P2, const int64_t *__restrict__ len_x,
-                               const int64_t *__restrict__ len_y, int mean, float *__restrict__ grad_xn,
-                               float *__restrict__ grad_yn) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CN_THREADS + threadIdx.x;
-    const float g = grad_cn[b];
-    const float *xb = xn + (size_t)b * P1 * 3, *yb = yn + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    float own[3], near[3];
-    int j;
-    if (grad_xn && i < P1) {
-        float *o = grad_xn + ((size_t)b * P1 + i) * 3;
-        const bool t = normal_parts(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, own, near);
-        o[0] = t ? own[0] : 0.0f;
-        o[1] = t ? own[1] : 0.0f;
-        o[2] = t ? own[2] : 0.0f;
-    }
-    if (grad_yn && i < P2) {
-        float *o = grad_yn + ((size_t)b * P2 + i) * 3;
-        const bool t = normal_parts(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, own, near);
-        o[0] = t ? own[0] : 0.0f;
-        o[1] = t ? own[1] : 0.0f;
-        o[2] = t ? own[2] : 0.0f;
-    }
-}
-
-// phase B, same grid: the near parts, RED.ADD.F32 into the gathered rows (x-queries into grad_yn, y-queries into
-// grad_xn)
-__global__ void __launch_bounds__(CN_THREADS)
-chamfer_normals_bwd_near_kernel(const float *__restrict__ xn, const float *__restrict__ yn,
-                                const int32_t *__restrict__ idx_x, const int32_t *__restrict__ idx_y,
-                                const float *__restrict__ grad_cn, int P1, int P2, const int64_t *__restrict__ len_x,
-                                const int64_t *__restrict__ len_y, int mean, float *__restrict__ grad_xn,
-                                float *__restrict__ grad_yn) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CN_THREADS + threadIdx.x;
-    const float g = grad_cn[b];
-    const float *xb = xn + (size_t)b * P1 * 3, *yb = yn + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    float own[3], near[3];
-    int j;
-    if (grad_yn && normal_parts(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, own, near)) {
-        float *o = grad_yn + ((size_t)b * P2 + j) * 3;
-        atomicAdd(o + 0, near[0]);
-        atomicAdd(o + 1, near[1]);
-        atomicAdd(o + 2, near[2]);
-    }
-    if (grad_xn && normal_parts(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, own, near)) {
-        float *o = grad_xn + ((size_t)b * P1 + j) * 3;
-        atomicAdd(o + 0, near[0]);
-        atomicAdd(o + 1, near[1]);
-        atomicAdd(o + 2, near[2]);
-    }
-}
-
-// Deterministic backward (scheme in det_accum.cuh, workspace of ptk_chamfer_bwd_det): M_b = the largest finite |part|
-// of both directions, so each gradient has the same bits whether or not the other one is requested; a row receives
-// its own part and at most l_other near parts, e_b from n = max(lx, ly) + 1.
-// phase 1, grid = (ceil(max(P1,P2) / 256), B): M_b (atomicMax into mbits[b], zeroed by the caller); accumulators and
-// outputs of every row zeroed
-__global__ void __launch_bounds__(CN_THREADS)
-chamfer_normals_bwd_det_max_kernel(const float *__restrict__ xn, const float *__restrict__ yn,
-                                   const int32_t *__restrict__ idx_x, const int32_t *__restrict__ idx_y,
-                                   const float *__restrict__ grad_cn, int P1, int P2, const int64_t *__restrict__ len_x,
-                                   const int64_t *__restrict__ len_y, int mean, float *__restrict__ grad_xn,
-                                   float *__restrict__ grad_yn, unsigned long long *__restrict__ acc_x,
-                                   unsigned long long *__restrict__ acc_y, unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CN_THREADS + threadIdx.x;
-    const float g = grad_cn[b];
-    const float *xb = xn + (size_t)b * P1 * 3, *yb = yn + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    float m = 0.0f, own[3], near[3];
-    int j;
-    if (normal_parts(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, own, near))
-#pragma unroll
-        for (int d = 0; d < 3; ++d) m = fmaxf(m, fmaxf(det_abs_finite(own[d]), det_abs_finite(near[d])));
-    if (normal_parts(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, own, near))
-#pragma unroll
-        for (int d = 0; d < 3; ++d) m = fmaxf(m, fmaxf(det_abs_finite(own[d]), det_abs_finite(near[d])));
-    if (grad_xn && i < P1) {
-        const size_t r = ((size_t)b * P1 + i) * 3;
-        acc_x[r + 0] = acc_x[r + 1] = acc_x[r + 2] = 0ull;
-        grad_xn[r + 0] = grad_xn[r + 1] = grad_xn[r + 2] = 0.0f;
-    }
-    if (grad_yn && i < P2) {
-        const size_t r = ((size_t)b * P2 + i) * 3;
-        acc_y[r + 0] = acc_y[r + 1] = acc_y[r + 2] = 0ull;
-        grad_yn[r + 0] = grad_yn[r + 1] = grad_yn[r + 2] = 0.0f;
-    }
-    det_block_max<CN_THREADS>(m, mbits + b);
-}
-
-// one part into one row: quantised into its accumulator, or (non-finite) added to its output
-__device__ __forceinline__ void normals_det_add(const float t[3], double scale, unsigned long long *acc, float *out) {
-#pragma unroll
-    for (int d = 0; d < 3; ++d) {
-        if (isfinite(t[d]))
-            atomicAdd(acc + d, det_quantise(t[d], scale));
-        else
-            atomicAdd(out + d, t[d]);
-    }
-}
-
-// phase 2, same grid: quantise and add both parts of x-query i and of y-query i
-__global__ void __launch_bounds__(CN_THREADS)
-chamfer_normals_bwd_det_add_kernel(const float *__restrict__ xn, const float *__restrict__ yn,
-                                   const int32_t *__restrict__ idx_x, const int32_t *__restrict__ idx_y,
-                                   const float *__restrict__ grad_cn, int P1, int P2, const int64_t *__restrict__ len_x,
-                                   const int64_t *__restrict__ len_y, int mean, float *__restrict__ grad_xn,
-                                   float *__restrict__ grad_yn, unsigned long long *__restrict__ acc_x,
-                                   unsigned long long *__restrict__ acc_y, const unsigned int *__restrict__ mbits) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CN_THREADS + threadIdx.x;
-    const float g = grad_cn[b];
-    const float *xb = xn + (size_t)b * P1 * 3, *yb = yn + (size_t)b * P2 * 3;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)max(L1, L2) + 1));
-    const size_t bx = (size_t)b * P1 * 3, by = (size_t)b * P2 * 3;
-    float own[3], near[3];
-    int j;
-    if (normal_parts(xb, yb, idx_x + (size_t)b * P1, g, i, L1, L2, mean, j, own, near)) {
-        if (grad_xn) normals_det_add(own, scale, acc_x + bx + (size_t)i * 3, grad_xn + bx + (size_t)i * 3);
-        if (grad_yn) normals_det_add(near, scale, acc_y + by + (size_t)j * 3, grad_yn + by + (size_t)j * 3);
-    }
-    if (normal_parts(yb, xb, idx_y + (size_t)b * P2, g, i, L2, L1, mean, j, own, near)) {
-        if (grad_yn) normals_det_add(own, scale, acc_y + by + (size_t)i * 3, grad_yn + by + (size_t)i * 3);
-        if (grad_xn) normals_det_add(near, scale, acc_x + bx + (size_t)j * 3, grad_xn + bx + (size_t)j * 3);
-    }
-}
-
-// phase 3, same grid: grad = fp32(acc) * 2^-e_b, unless the row's output already holds a non-finite sum
-__global__ void __launch_bounds__(CN_THREADS)
-chamfer_normals_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len_x,
-                                       const int64_t *__restrict__ len_y, const unsigned int *__restrict__ mbits,
-                                       const unsigned long long *__restrict__ acc_x,
-                                       const unsigned long long *__restrict__ acc_y, float *__restrict__ grad_xn,
-                                       float *__restrict__ grad_yn) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * CN_THREADS + threadIdx.x;
-    const int L1 = pair_len(len_x, b, P1), L2 = pair_len(len_y, b, P2);
-    const int e = det_exponent(mbits[b], (long long)max(L1, L2) + 1);
-    if (grad_xn && i < P1) {
-        const size_t r = ((size_t)b * P1 + i) * 3;
-        for (int d = 0; d < 3; ++d) det_convert(grad_xn + r + d, acc_x + r + d, e);
-    }
-    if (grad_yn && i < P2) {
-        const size_t r = ((size_t)b * P2 + i) * 3;
-        for (int d = 0; d < 3; ++d) det_convert(grad_yn + r + d, acc_y + r + d, e);
-    }
-}
-
 // host-side checks shared by the three entry points
 static int normals_check(const float *xn, const float *yn, const int32_t *idx_x, const int32_t *idx_y, int64_t B,
                          int64_t P1, int64_t P2, int reduction, const char *what) {
@@ -371,16 +207,8 @@ extern "C" int ptk_chamfer_normals_bwd(const float *x_normals, const float *y_no
     if (rc) return rc;
     PTK_REQUIRE(grad_cham_normals, PTK_ERR_SHAPE, "chamfer_normals_bwd: null grad_cham_normals pointer");
     if (!grad_xn && !grad_yn) return PTK_OK;
-    cudaStream_t st = as_stream(stream);
-    const dim3 grid((unsigned)ceil_div(P1 > P2 ? P1 : P2, CN_THREADS), (unsigned)B);
-    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
-    launch_pdl(chamfer_normals_bwd_own_kernel, grid, dim3(CN_THREADS), 0, st, x_normals, y_normals, idx_x, idx_y,
-               grad_cham_normals, (int)P1, (int)P2, len_x, len_y, mean, grad_xn, grad_yn);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_normals_bwd_near_kernel, grid, dim3(CN_THREADS), 0, st, x_normals, y_normals, idx_x, idx_y,
-               grad_cham_normals, (int)P1, (int)P2, len_x, len_y, mean, grad_xn, grad_yn);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
+    return pair_bwd<normal_parts>(x_normals, y_normals, len_x, len_y, idx_x, idx_y, grad_cham_normals, B, P1, P2,
+                                 reduction == PTK_REDUCE_MEAN ? 1 : 0, grad_xn, grad_yn, as_stream(stream));
 }
 
 extern "C" int ptk_chamfer_normals_bwd_det(const float *x_normals, const float *y_normals, const int64_t *len_x,
@@ -393,31 +221,9 @@ extern "C" int ptk_chamfer_normals_bwd_det(const float *x_normals, const float *
     if (rc) return rc;
     PTK_REQUIRE(grad_cham_normals, PTK_ERR_SHAPE, "chamfer_normals_bwd_det: null grad_cham_normals pointer");
     if (!grad_xn && !grad_yn) return PTK_OK;
-    const size_t need = ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE,
-                "chamfer_normals_bwd_det: workspace too small (%zu < %zu)", workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "chamfer_normals_bwd_det: workspace must be 16-byte aligned");
-    // the layout of ptk_chamfer_bwd_det's workspace: [M_b bits B, padded to 256 bytes][acc_x B*P1*3][acc_y B*P2*3] int64
-    char *p = reinterpret_cast<char *>(workspace);
-    auto *mbits = reinterpret_cast<unsigned int *>(p);
-    auto *acc_x = grad_xn ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B)) : nullptr;
-    auto *acc_y = grad_yn ? reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B) + det_align(24 * (size_t)B * P1))
-                          : nullptr;
-    cudaStream_t st = as_stream(stream);
-    const dim3 grid((unsigned)ceil_div(P1 > P2 ? P1 : P2, CN_THREADS), (unsigned)B);
-    const int mean = reduction == PTK_REDUCE_MEAN ? 1 : 0;
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
-    launch_pdl(chamfer_normals_bwd_det_max_kernel, grid, dim3(CN_THREADS), 0, st, x_normals, y_normals, idx_x, idx_y,
-               grad_cham_normals, (int)P1, (int)P2, len_x, len_y, mean, grad_xn, grad_yn, acc_x, acc_y, mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_normals_bwd_det_add_kernel, grid, dim3(CN_THREADS), 0, st, x_normals, y_normals, idx_x, idx_y,
-               grad_cham_normals, (int)P1, (int)P2, len_x, len_y, mean, grad_xn, grad_yn, acc_x, acc_y,
-               (const unsigned int *)mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(chamfer_normals_bwd_det_convert_kernel, grid, dim3(CN_THREADS), 0, st, (int)P1, (int)P2, len_x, len_y,
-               (const unsigned int *)mbits, (const unsigned long long *)acc_x, (const unsigned long long *)acc_y, grad_xn,
-               grad_yn);
-    PTK_CHECK_LAUNCH();
-    return PTK_OK;
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_chamfer_bwd_det_workspace_bytes(B, P1, P2),
+                             "chamfer_normals_bwd_det");
+    if (rc) return rc;
+    return pair_bwd_det<normal_parts>(x_normals, y_normals, len_x, len_y, idx_x, idx_y, grad_cham_normals, B, P1, P2,
+                                     reduction == PTK_REDUCE_MEAN ? 1 : 0, grad_xn, grad_yn, workspace, as_stream(stream));
 }

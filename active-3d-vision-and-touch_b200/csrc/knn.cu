@@ -280,8 +280,9 @@ knn_merge_kernel(const uint2 *__restrict__ part, const int64_t *__restrict__ len
 
 // ---------------------------------------------------------------------------------------- backward
 // The gradient of dist[b,i,k] = |p1_i - p2_j|^2, j = idx[b,i,k], under the upstream gradient g[b,i,k].  A slot
-// k < min(K, l2) of a valid query i < l1 has the term s * (p1_i - p2_j) per component, s = 2 g[b,i,k] (knn1_term's fp32
-// operations, PyTorch3D's knn_points_backward); no other slot exists and its g is never read.
+// k < min(K, l2) of a valid query i < l1 has the term s * (p1_i - p2_j) per component, s = 2 g[b,i,k] (PyTorch3D's
+// knn_points_backward); no other slot exists and its g is never read.  The 1-NN backward (ptk_knn1_bwd_*) is this code
+// at K = 1.
 __device__ __forceinline__ bool knn_term(const float *__restrict__ p1b, const float *__restrict__ p2b,
                                          const int32_t *__restrict__ idx, const float *__restrict__ g, int i, int k,
                                          int K, int L1, int L2, int &j, float t[3]) {
@@ -356,9 +357,9 @@ knn_bwd_scatter_kernel(const float *__restrict__ p1, const float *__restrict__ p
     }
 }
 
-// Deterministic form (det_accum.cuh), as ptk_knn1_bwd_det: grad_p1 is phase A's slot-order sum; grad_p2 goes through
-// the integer sum with M_b = the largest finite |term| of pair b and e_b from n = l1 + 1 (a query's K indices are
-// distinct, so a p2 row receives at most l1 terms).
+// Deterministic form (det_accum.cuh): grad_p1 is phase A's slot-order sum; grad_p2 goes through the integer sum with
+// M_b = the largest finite |term| of pair b and n = l1 + 1 (a query's K indices are distinct, so a p2 row receives at
+// most l1 terms).
 // phase 1, grid = (ceil(max(P1 * K, P2) / 256), B): M_b over the slots (atomicMax into mbits[b], zeroed by the
 // caller), grad_p1 rows as in phase A, accumulators and outputs of every p2 row zeroed
 __global__ void __launch_bounds__(256)
@@ -378,11 +379,7 @@ knn_bwd_det_terms_kernel(const float *__restrict__ p1, const float *__restrict__
     if (e < P1 * K && knn_term(p1b, p2b, ib, gb, e / K, e % K, K, L1, L2, j, t))
         m = fmaxf(det_abs_finite(t[0]), fmaxf(det_abs_finite(t[1]), det_abs_finite(t[2])));
     if (grad_p1 && e < P1) knn_grad_p1_row(p1b, p2b, ib, gb, e, K, L1, L2, grad_p1 + ((size_t)b * P1 + e) * 3);
-    if (e < P2) {
-        const size_t r = ((size_t)b * P2 + e) * 3;
-        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
-        grad_p2[r + 0] = grad_p2[r + 1] = grad_p2[r + 2] = 0.0f;
-    }
+    if (e < P2) det_zero_row(acc, grad_p2, (size_t)b * P2 + e);
     det_block_max<256>(m, mbits + b);
 }
 
@@ -391,7 +388,7 @@ __global__ void __launch_bounds__(256)
 knn_bwd_det_reduce_kernel(const float *__restrict__ p1, const float *__restrict__ p2, const int32_t *__restrict__ idx,
                           const float *__restrict__ grad_dist, int P1, int P2, int K, const int64_t *__restrict__ len1,
                           const int64_t *__restrict__ len2, float *__restrict__ grad_p2,
-                          unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
+                          unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits, DetBound nb) {
     pdl_wait();
     const int b = blockIdx.y;
     const int e = blockIdx.x * 256 + threadIdx.x;
@@ -402,28 +399,10 @@ knn_bwd_det_reduce_kernel(const float *__restrict__ p1, const float *__restrict_
     if (!knn_term(p1 + (size_t)b * P1 * 3, p2 + (size_t)b * P2 * 3, idx + (size_t)b * P1 * K,
                   grad_dist + (size_t)b * P1 * K, e / K, e % K, K, L1, L2, j, t))
         return;
-    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)L1 + 1));
+    const double scale = det_scale(mbits, nb, b);
     const size_t r = ((size_t)b * P2 + j) * 3;
 #pragma unroll
-    for (int d = 0; d < 3; ++d) {
-        if (isfinite(t[d]))
-            atomicAdd(acc + r + d, 0ull - det_quantise(t[d], scale));
-        else
-            atomicAdd(grad_p2 + r + d, -t[d]);
-    }
-}
-
-// phase 3, grid = (ceil(P2 / 256), B): grad_p2 = fp32(acc) * 2^-e_b, unless the row already holds a non-finite sum
-__global__ void __launch_bounds__(256)
-knn_bwd_det_convert_kernel(int P1, int P2, const int64_t *__restrict__ len1, const unsigned int *__restrict__ mbits,
-                           const unsigned long long *__restrict__ acc, float *__restrict__ grad_p2) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * 256 + threadIdx.x;
-    if (i >= P2) return;
-    const int e = det_exponent(mbits[b], (long long)pair_len(len1, b, P1) + 1);
-    const size_t r = ((size_t)b * P2 + i) * 3;
-    for (int d = 0; d < 3; ++d) det_convert(grad_p2 + r + d, acc + r + d, e);
+    for (int d = 0; d < 3; ++d) det_add(acc + r + d, grad_p2 + r + d, -t[d], scale);
 }
 
 // ---------------------------------------------------------------------------------------- host side
@@ -505,22 +484,11 @@ extern "C" int ptk_knn_fwd_lengths(const float *p1, const float *p2, const int64
     return PTK_OK;
 }
 
-static int knn_bwd_check(const float *p1, const float *p2, const int32_t *idx, const float *grad_dist, int64_t B,
-                         int64_t P1, int64_t P2, int64_t K) {
-    int rc = check_knn(p1, p2, B, P1, P2, K);
-    if (rc) return rc;
-    PTK_REQUIRE(idx && grad_dist, PTK_ERR_SHAPE, "knn_bwd: null index / grad pointer");
-    return PTK_OK;
-}
-
-extern "C" int ptk_knn_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
-                                   const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
-                                   int64_t K, float *grad_p1, float *grad_p2, ptk_stream_t stream) {
-    PTK_NVTX("ptk_knn_bwd_lengths");
-    int rc = knn_bwd_check(p1, p2, idx, grad_dist, B, P1, P2, K);
-    if (rc) return rc;
-    if (!grad_p1 && !grad_p2) return PTK_OK;
-    cudaStream_t st = as_stream(stream);
+// The backward bodies behind ptk_knn_bwd_* and ptk_knn1_bwd_* (K = 1); the caller has checked the arguments and that
+// a gradient is requested.
+static int knn_bwd(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                   const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K, float *grad_p1, float *grad_p2,
+                   cudaStream_t st) {
     const int64_t Pm = P1 > P2 ? P1 : P2;
     launch_pdl(knn_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, 256), (unsigned)B), dim3(256), 0, st, p1, p2, idx,
                grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p1, grad_p2);
@@ -533,6 +501,53 @@ extern "C" int ptk_knn_bwd_lengths(const float *p1, const float *p2, const int64
     return PTK_OK;
 }
 
+// workspace: det_workspace_bytes(B, P2), checked by the caller
+static int knn_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2, const int32_t *idx,
+                       const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K, float *grad_p1,
+                       float *grad_p2, void *workspace, cudaStream_t st) {
+    if (!grad_p2) return knn_bwd(p1, p2, len1, len2, idx, grad_dist, B, P1, P2, K, grad_p1, nullptr, st);  // plain stores
+    DetWs w;
+    PTK_CHECK_CUDA(det_begin(workspace, B, P2, st, w));
+    const DetBound nb = det_bound_len(len1, P1);
+    const int64_t PK = P1 * K > P2 ? P1 * K : P2;
+    launch_pdl(knn_bwd_det_terms_kernel, dim3((unsigned)ceil_div(PK, 256), (unsigned)B), dim3(256), 0, st, p1, p2, idx,
+               grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p1, grad_p2, w.acc_a, w.mbits);
+    PTK_CHECK_LAUNCH();
+    launch_pdl(knn_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(P1 * K, 256), (unsigned)B), dim3(256), 0, st, p1, p2,
+               idx, grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p2, w.acc_a, (const unsigned int *)w.mbits, nb);
+    PTK_CHECK_LAUNCH();
+    det_launch_convert<256>(w, nb, B, grad_p2, P2, nullptr, 0, st);
+    PTK_CHECK_LAUNCH();
+    return PTK_OK;
+}
+
+static int knn_bwd_check(const float *p1, const float *p2, const int32_t *idx, const float *grad_dist, int64_t B,
+                         int64_t P1, int64_t P2, int64_t K) {
+    int rc = check_knn(p1, p2, B, P1, P2, K);
+    if (rc) return rc;
+    PTK_REQUIRE(idx && grad_dist, PTK_ERR_SHAPE, "knn_bwd: null index / grad pointer");
+    return PTK_OK;
+}
+
+}  // namespace ptk
+
+using namespace ptk;
+
+extern "C" int ptk_knn_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
+                                   const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
+                                   int64_t K, float *grad_p1, float *grad_p2, ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn_bwd_lengths");
+    int rc = knn_bwd_check(p1, p2, idx, grad_dist, B, P1, P2, K);
+    if (rc) return rc;
+    if (!grad_p1 && !grad_p2) return PTK_OK;
+    return knn_bwd(p1, p2, len1, len2, idx, grad_dist, B, P1, P2, K, grad_p1, grad_p2, as_stream(stream));
+}
+
+extern "C" size_t ptk_knn1_bwd_det_workspace_bytes(int64_t B, int64_t P1, int64_t P2) {
+    if (B <= 0 || P1 <= 0 || P2 <= 0) return 0;
+    return det_workspace_bytes(B, P2);
+}
+
 extern "C" int ptk_knn_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
                                const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2, int64_t K,
                                float *grad_p1, float *grad_p2, void *workspace, size_t workspace_bytes,
@@ -541,35 +556,40 @@ extern "C" int ptk_knn_bwd_det(const float *p1, const float *p2, const int64_t *
     int rc = knn_bwd_check(p1, p2, idx, grad_dist, B, P1, P2, K);
     if (rc) return rc;
     if (!grad_p1 && !grad_p2) return PTK_OK;
-    const size_t need = ptk_knn1_bwd_det_workspace_bytes(B, P1, P2);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "knn_bwd_det: workspace too small (%zu < %zu)",
-                workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "knn_bwd_det: workspace must be 16-byte aligned");
-    cudaStream_t st = as_stream(stream);
-    const int64_t Pm = P1 > P2 ? P1 : P2;
-    if (!grad_p2) {  // grad_p1 alone: plain stores, nothing to sum
-        launch_pdl(knn_bwd_direct_kernel, dim3((unsigned)ceil_div(Pm, 256), (unsigned)B), dim3(256), 0, st, p1, p2, idx,
-                   grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p1, (float *)nullptr);
-        PTK_CHECK_LAUNCH();
-        return PTK_OK;
-    }
-    // the layout of ptk_knn1_bwd_det's workspace: [M_b bits B, padded to 256 bytes][acc_p2 B*P2*3 int64]
-    char *p = reinterpret_cast<char *>(workspace);
-    auto *mbits = reinterpret_cast<unsigned int *>(p);
-    auto *acc = reinterpret_cast<unsigned long long *>(p + det_align(4 * (size_t)B));
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
-    const int64_t PK = P1 * K > P2 ? P1 * K : P2;
-    launch_pdl(knn_bwd_det_terms_kernel, dim3((unsigned)ceil_div(PK, 256), (unsigned)B), dim3(256), 0, st, p1, p2, idx,
-               grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p1, grad_p2, acc, mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(knn_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(P1 * K, 256), (unsigned)B), dim3(256), 0, st, p1, p2,
-               idx, grad_dist, (int)P1, (int)P2, (int)K, len1, len2, grad_p2, acc, (const unsigned int *)mbits);
-    PTK_CHECK_LAUNCH();
-    launch_pdl(knn_bwd_det_convert_kernel, dim3((unsigned)ceil_div(P2, 256), (unsigned)B), dim3(256), 0, st, (int)P1,
-               (int)P2, len1, (const unsigned int *)mbits, (const unsigned long long *)acc, grad_p2);
-    PTK_CHECK_LAUNCH();
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_knn1_bwd_det_workspace_bytes(B, P1, P2), "knn_bwd_det");
+    if (rc) return rc;
+    return knn_bwd_det(p1, p2, len1, len2, idx, grad_dist, B, P1, P2, K, grad_p1, grad_p2, workspace, as_stream(stream));
+}
+
+static int knn1_bwd_check(const float *p1, const float *p2, const int32_t *idx, const float *grad_dist, int64_t B,
+                          int64_t P1, int64_t P2) {
+    int rc = check_clouds(p1, p2, B, P1, P2);
+    if (rc) return rc;
+    PTK_REQUIRE(idx && grad_dist, PTK_ERR_SHAPE, "knn1_bwd: null index / grad pointer");
     return PTK_OK;
 }
 
-}  // namespace ptk
+extern "C" int ptk_knn1_bwd_lengths(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
+                                    const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
+                                    float *grad_p1, float *grad_p2, ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_bwd_lengths");
+    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
+    if (rc) return rc;
+    if (!grad_p1 && !grad_p2) return PTK_OK;
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd: batch too large");
+    return knn_bwd(p1, p2, len1, len2, idx, grad_dist, B, P1, P2, 1, grad_p1, grad_p2, as_stream(stream));
+}
+
+extern "C" int ptk_knn1_bwd_det(const float *p1, const float *p2, const int64_t *len1, const int64_t *len2,
+                                const int32_t *idx, const float *grad_dist, int64_t B, int64_t P1, int64_t P2,
+                                float *grad_p1, float *grad_p2, void *workspace, size_t workspace_bytes,
+                                ptk_stream_t stream) {
+    PTK_NVTX("ptk_knn1_bwd_det");
+    int rc = knn1_bwd_check(p1, p2, idx, grad_dist, B, P1, P2);
+    if (rc) return rc;
+    if (!grad_p1 && !grad_p2) return PTK_OK;
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_knn1_bwd_det_workspace_bytes(B, P1, P2), "knn1_bwd_det");
+    if (rc) return rc;
+    PTK_REQUIRE(B <= 65535, PTK_ERR_SHAPE, "knn1_bwd_det: batch too large");
+    return knn_bwd_det(p1, p2, len1, len2, idx, grad_dist, B, P1, P2, 1, grad_p1, grad_p2, workspace, as_stream(stream));
+}

@@ -343,8 +343,8 @@ point_frames_bwd_kernel(const float *__restrict__ points, const int64_t *__restr
     }
 }
 
-// Deterministic form (det_accum.cuh), as ptk_knn_bwd_det: M_b over the finite terms of cloud b, n = l + 1 (a query's
-// K' neighbours are distinct, so a row receives at most l terms).
+// Deterministic form (det_accum.cuh): M_b over the finite terms of cloud b, n = l + 1 (a query's K' neighbours are
+// distinct, so a row receives at most l terms).
 // phase 1, grid = (ceil(P / PN_THREADS), B): M_b (atomicMax into mbits[b], zeroed by the caller), accumulators and
 // grad_points rows zeroed
 __global__ void __launch_bounds__(PN_THREADS)
@@ -359,9 +359,7 @@ point_frames_bwd_det_max_kernel(const float *__restrict__ points, const int64_t 
     const int i = blockIdx.x * PN_THREADS + threadIdx.x;
     float m = 0.0f;
     if (i < P) {
-        const size_t r = ((size_t)b * P + i) * 3;
-        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
-        grad_points[r + 0] = grad_points[r + 1] = grad_points[r + 2] = 0.0f;
+        det_zero_row(acc, grad_points, (size_t)b * P + i);
         int Kp;
         PnFrame f;
         float S[3][3], t[3];
@@ -386,7 +384,7 @@ point_frames_bwd_det_add_kernel(const float *__restrict__ points, const int64_t 
                                 int disambiguate, const float *__restrict__ grad_normals,
                                 const float *__restrict__ grad_curvatures, const float *__restrict__ grad_frames,
                                 float *__restrict__ grad_points, unsigned long long *__restrict__ acc,
-                                const unsigned int *__restrict__ mbits) {
+                                const unsigned int *__restrict__ mbits, DetBound nb) {
     pdl_wait();
     const int b = blockIdx.y;
     const int i = blockIdx.x * PN_THREADS + threadIdx.x;
@@ -397,32 +395,14 @@ point_frames_bwd_det_add_kernel(const float *__restrict__ points, const int64_t 
     if (!pn_query_grad(points, lengths, idx, dist, b, i, P, K, disambiguate, grad_normals, grad_curvatures, grad_frames,
                        Kp, f, S))
         return;
-    const double scale = ldexp(1.0, det_exponent(mbits[b], (long long)pair_len(lengths, b, P) + 1));
+    const double scale = det_scale(mbits, nb, b);
     const float *pb = points + (size_t)b * P * 3;
     const int32_t *ir = idx + ((size_t)b * P + i) * K;
     for (int k = 0; k < Kp; ++k) {
         const size_t r = ((size_t)b * P + pn_term(f, S, pb, ir, k, t)) * 3;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            if (isfinite(t[c]))
-                atomicAdd(acc + r + c, det_quantise(t[c], scale));
-            else
-                atomicAdd(grad_points + r + c, t[c]);
-        }
+        for (int c = 0; c < 3; ++c) det_add(acc + r + c, grad_points + r + c, t[c], scale);
     }
-}
-
-// phase 3, grid = (ceil(P / PN_THREADS), B): grad_points = fp32(acc) * 2^-e_b, unless the row holds a non-finite sum
-__global__ void __launch_bounds__(PN_THREADS)
-point_frames_bwd_det_convert_kernel(int P, const int64_t *__restrict__ lengths, const unsigned int *__restrict__ mbits,
-                                    const unsigned long long *__restrict__ acc, float *__restrict__ grad_points) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * PN_THREADS + threadIdx.x;
-    if (i >= P) return;
-    const int e = det_exponent(mbits[b], (long long)pair_len(lengths, b, P) + 1);
-    const size_t r = ((size_t)b * P + i) * 3;
-    for (int c = 0; c < 3; ++c) det_convert(grad_points + r + c, acc + r + c, e);
 }
 
 // ---------------------------------------------------------------------------------------- host side
@@ -483,29 +463,25 @@ extern "C" int ptk_point_frames_bwd_det(const float *points, const int64_t *leng
     int rc = pn_check(points, idx, dist, B, P, K, "point_frames_bwd_det");
     if (rc) return rc;
     PTK_REQUIRE(grad_points, PTK_ERR_SHAPE, "point_frames_bwd_det: null grad_points pointer");
-    const size_t need = ptk_knn1_bwd_det_workspace_bytes(B, P, P);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE,
-                "point_frames_bwd_det: workspace too small (%zu < %zu)", workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "point_frames_bwd_det: workspace must be 16-byte aligned");
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_knn1_bwd_det_workspace_bytes(B, P, P),
+                             "point_frames_bwd_det");
+    if (rc) return rc;
     cudaStream_t st = as_stream(stream);
     if (!grad_normals && !grad_curvatures && !grad_frames) {
         PTK_CHECK_CUDA(cudaMemsetAsync(grad_points, 0, sizeof(float) * (size_t)B * P * 3, st));
         return PTK_OK;
     }
-    // the layout of ptk_knn1_bwd_det's workspace: [M_b bits B, padded to 256 bytes][acc B*P*3 int64]
-    auto *mbits = reinterpret_cast<unsigned int *>(workspace);
-    auto *acc = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(workspace) + det_align(4 * (size_t)B));
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
+    DetWs w;
+    PTK_CHECK_CUDA(det_begin(workspace, B, P, st, w));
+    const DetBound nb = det_bound_len(lengths, P);
     launch_pdl(point_frames_bwd_det_max_kernel, pn_grid(B, P), dim3(PN_THREADS), 0, st, points, lengths, idx, dist,
-               (int)P, (int)K, disambiguate, grad_normals, grad_curvatures, grad_frames, grad_points, acc, mbits);
+               (int)P, (int)K, disambiguate, grad_normals, grad_curvatures, grad_frames, grad_points, w.acc_a, w.mbits);
     PTK_CHECK_LAUNCH();
     launch_pdl(point_frames_bwd_det_add_kernel, pn_grid(B, P), dim3(PN_THREADS), 0, st, points, lengths, idx, dist,
-               (int)P, (int)K, disambiguate, grad_normals, grad_curvatures, grad_frames, grad_points, acc,
-               (const unsigned int *)mbits);
+               (int)P, (int)K, disambiguate, grad_normals, grad_curvatures, grad_frames, grad_points, w.acc_a,
+               (const unsigned int *)w.mbits, nb);
     PTK_CHECK_LAUNCH();
-    launch_pdl(point_frames_bwd_det_convert_kernel, pn_grid(B, P), dim3(PN_THREADS), 0, st, (int)P, lengths,
-               (const unsigned int *)mbits, (const unsigned long long *)acc, grad_points);
+    det_launch_convert<PN_THREADS>(w, nb, B, grad_points, P, nullptr, 0, st);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }

@@ -181,24 +181,8 @@ sample_normals_bwd_det_max_kernel(const float *__restrict__ verts, const int32_t
 #pragma unroll
             for (int d = 0; d < 3; ++d) m = fmaxf(m, fmaxf(det_abs_finite(pt[k][d]), det_abs_finite(nt[k][d])));
     }
-    if (i < V) {
-        const size_t r = ((size_t)b * V + i) * 3;
-        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
-        grad_verts[r + 0] = grad_verts[r + 1] = grad_verts[r + 2] = 0.0f;
-    }
+    if (i < V) det_zero_row(acc, grad_verts, (size_t)b * V + i);
     det_block_max<SN_THREADS>(m, mbits + b);
-}
-
-// one term into vertex component k: quantised into the accumulator (shared or global), or (non-finite) added to the
-// output
-__device__ __forceinline__ void sn_det_add(float t, double scale, bool in_smem, unsigned long long *s_acc,
-                                           unsigned long long *av, float *gv, size_t k) {
-    if (!isfinite(t))
-        atomicAdd(&gv[k], t);
-    else if (in_smem)
-        atomicAdd(&s_acc[k], det_quantise(t, scale));
-    else
-        atomicAdd(&av[k], det_quantise(t, scale));
 }
 
 // phase 2, grid = (ceil(S / SN_PER_CTA), B): quantise and add both terms.  Meshes of up to SND_SMEM_VERTS vertices are
@@ -208,7 +192,8 @@ sample_normals_bwd_det_add_kernel(const float *__restrict__ verts, const int32_t
                                   const int32_t *__restrict__ face_idx, const float *__restrict__ uu,
                                   const float *__restrict__ vv, const float *__restrict__ grad_pts,
                                   const float *__restrict__ grad_n, int V, int F, int S, float *__restrict__ grad_verts,
-                                  unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
+                                  unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits,
+                                  DetBound nb) {
     pdl_wait();
     const int b = blockIdx.y;
     const int tid = threadIdx.x;
@@ -218,7 +203,7 @@ sample_normals_bwd_det_add_kernel(const float *__restrict__ verts, const int32_t
         for (int k = tid; k < V * 3; k += SN_THREADS) s_acc[k] = 0ull;
         __syncthreads();
     }
-    const double scale = ldexp(1.0, det_exponent(mbits[b], 6LL * S + 1));
+    const double scale = det_scale(mbits, nb, b);
     const float *vb = verts + (size_t)b * V * 3;
     float *gv = grad_verts + (size_t)b * V * 3;
     unsigned long long *av = acc + (size_t)b * V * 3;
@@ -233,8 +218,13 @@ sample_normals_bwd_det_add_kernel(const float *__restrict__ verts, const int32_t
 #pragma unroll
             for (int d = 0; d < 3; ++d) {
                 const size_t e = (size_t)vi[k] * 3 + d;
-                sn_det_add(pt[k][d], scale, in_smem, s_acc, av, gv, e);
-                sn_det_add(nt[k][d], scale, in_smem, s_acc, av, gv, e);
+                if (in_smem) {
+                    det_add(&s_acc[e], &gv[e], pt[k][d], scale);
+                    det_add(&s_acc[e], &gv[e], nt[k][d], scale);
+                } else {
+                    det_add(&av[e], &gv[e], pt[k][d], scale);
+                    det_add(&av[e], &gv[e], nt[k][d], scale);
+                }
             }
     }
     if (in_smem) {
@@ -244,19 +234,6 @@ sample_normals_bwd_det_add_kernel(const float *__restrict__ verts, const int32_t
             if (a != 0ull) atomicAdd(&av[k], a);
         }
     }
-}
-
-// phase 3, grid = (ceil(V / SN_THREADS), B)
-__global__ void __launch_bounds__(SN_THREADS)
-sample_normals_bwd_det_convert_kernel(int V, int S, const unsigned int *__restrict__ mbits,
-                                      const unsigned long long *__restrict__ acc, float *__restrict__ grad_verts) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * SN_THREADS + threadIdx.x;
-    if (i >= V) return;
-    const int e = det_exponent(mbits[b], 6LL * S + 1);
-    const size_t r = ((size_t)b * V + i) * 3;
-    for (int d = 0; d < 3; ++d) det_convert(grad_verts + r + d, acc + r + d, e);
 }
 
 // host-side checks shared by the backward entry points
@@ -301,10 +278,9 @@ extern "C" int ptk_sample_normals_bwd(const float *verts, const int32_t *faces, 
     return PTK_OK;
 }
 
-// det workspace: [M_b bits B, padded to 256 bytes][acc B*V*3 int64] (the layout of ptk_sample_bwd_det's)
 extern "C" size_t ptk_sample_normals_bwd_det_workspace_bytes(int64_t B, int64_t V) {
     if (B <= 0 || V <= 0) return 0;
-    return det_align(4 * (size_t)B) + 24 * (size_t)B * (size_t)V;
+    return det_workspace_bytes(B, V);
 }
 
 extern "C" int ptk_sample_normals_bwd_det(const float *verts, const int32_t *faces, const int32_t *face_idx,
@@ -314,27 +290,23 @@ extern "C" int ptk_sample_normals_bwd_det(const float *verts, const int32_t *fac
     PTK_NVTX("ptk_sample_normals_bwd_det");
     int rc = sn_bwd_check(verts, faces, face_idx, uv, grad_normals, grad_verts, B, V, F, S, "sample_normals_bwd_det");
     if (rc) return rc;
-    const size_t need = ptk_sample_normals_bwd_det_workspace_bytes(B, V);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE,
-                "sample_normals_bwd_det: workspace too small (%zu < %zu)", workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "sample_normals_bwd_det: workspace must be 16-byte aligned");
-    auto *mbits = reinterpret_cast<unsigned int *>(workspace);
-    auto *acc = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(workspace) + det_align(4 * (size_t)B));
+    rc = det_check_workspace(workspace, workspace_bytes, ptk_sample_normals_bwd_det_workspace_bytes(B, V),
+                             "sample_normals_bwd_det");
+    if (rc) return rc;
     cudaStream_t st = as_stream(stream);
+    DetWs w;
+    PTK_CHECK_CUDA(det_begin(workspace, B, V, st, w));
+    const DetBound nb = det_bound_const(6LL * S + 1);
     const float *uu = uv, *vv = uv + (size_t)B * S;
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
     launch_pdl(sample_normals_bwd_det_max_kernel, dim3((unsigned)ceil_div(S > V ? S : V, SN_THREADS), (unsigned)B),
                dim3(SN_THREADS), 0, st, verts, faces, face_idx, uu, vv, grad_pts, grad_normals, (int)V, (int)F, (int)S,
-               grad_verts, acc, mbits);
+               grad_verts, w.acc_a, w.mbits);
     PTK_CHECK_LAUNCH();
     launch_pdl(sample_normals_bwd_det_add_kernel, dim3((unsigned)ceil_div(S, SN_PER_CTA), (unsigned)B), dim3(SN_THREADS),
-               0, st, verts, faces, face_idx, uu, vv, grad_pts, grad_normals, (int)V, (int)F, (int)S, grad_verts, acc,
-               (const unsigned int *)mbits);
+               0, st, verts, faces, face_idx, uu, vv, grad_pts, grad_normals, (int)V, (int)F, (int)S, grad_verts, w.acc_a,
+               (const unsigned int *)w.mbits, nb);
     PTK_CHECK_LAUNCH();
-    launch_pdl(sample_normals_bwd_det_convert_kernel, dim3((unsigned)ceil_div(V, SN_THREADS), (unsigned)B),
-               dim3(SN_THREADS), 0, st, (int)V, (int)S, (const unsigned int *)mbits, (const unsigned long long *)acc,
-               grad_verts);
+    det_launch_convert<SN_THREADS>(w, nb, B, grad_verts, V, nullptr, 0, st);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }

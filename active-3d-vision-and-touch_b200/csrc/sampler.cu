@@ -237,11 +237,7 @@ sample_bwd_det_terms_kernel(const float *__restrict__ grad_pts, const float *__r
 #pragma unroll
             for (int d = 0; d < 3; ++d) m = fmaxf(m, det_abs_finite(__fmul_rn(w[k], grad_pts[o * 3 + d])));
     }
-    if (i < V) {
-        const size_t r = ((size_t)b * V + i) * 3;
-        acc[r + 0] = acc[r + 1] = acc[r + 2] = 0ull;
-        grad_verts[r + 0] = grad_verts[r + 1] = grad_verts[r + 2] = 0.0f;
-    }
+    if (i < V) det_zero_row(acc, grad_verts, (size_t)b * V + i);
     det_block_max<SP_THREADS>(m, mbits + b);
 }
 
@@ -253,7 +249,7 @@ __global__ void __launch_bounds__(SP_THREADS)
 sample_bwd_det_reduce_kernel(const float *__restrict__ grad_pts, const int32_t *__restrict__ face_idx,
                              const float *__restrict__ uu, const float *__restrict__ vv, const int32_t *__restrict__ faces,
                              int V, int S, int samples_per_cta, float *__restrict__ grad_verts,
-                             unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits) {
+                             unsigned long long *__restrict__ acc, const unsigned int *__restrict__ mbits, DetBound nb) {
     pdl_wait();
     const int b = blockIdx.y;
     const int tid = threadIdx.x;
@@ -263,7 +259,7 @@ sample_bwd_det_reduce_kernel(const float *__restrict__ grad_pts, const int32_t *
         for (int k = tid; k < V * 3; k += SP_THREADS) s_acc[k] = 0ull;
         __syncthreads();
     }
-    const double scale = ldexp(1.0, det_exponent(mbits[b], 3LL * S + 1));
+    const double scale = det_scale(mbits, nb, b);
     float *gv = grad_verts + (size_t)b * V * 3;
     unsigned long long *av = acc + (size_t)b * V * 3;
     const int s_begin = blockIdx.x * samples_per_cta;
@@ -280,12 +276,10 @@ sample_bwd_det_reduce_kernel(const float *__restrict__ grad_pts, const int32_t *
 #pragma unroll
             for (int d = 0; d < 3; ++d) {
                 const float c = __fmul_rn(w[k], g[d]);
-                if (!isfinite(c))
-                    atomicAdd(&gv[(size_t)vi * 3 + d], c);
-                else if (in_smem)
-                    atomicAdd(&s_acc[vi * 3 + d], det_quantise(c, scale));
+                if (in_smem)
+                    det_add(&s_acc[vi * 3 + d], &gv[(size_t)vi * 3 + d], c, scale);
                 else
-                    atomicAdd(&av[(size_t)vi * 3 + d], det_quantise(c, scale));
+                    det_add(&av[(size_t)vi * 3 + d], &gv[(size_t)vi * 3 + d], c, scale);
             }
         }
     }
@@ -296,19 +290,6 @@ sample_bwd_det_reduce_kernel(const float *__restrict__ grad_pts, const int32_t *
             if (a != 0ull) atomicAdd(&av[k], a);
         }
     }
-}
-
-// phase 3, grid = (ceil(V / SP_THREADS), B)
-__global__ void __launch_bounds__(SP_THREADS)
-sample_bwd_det_convert_kernel(int V, int S, const unsigned int *__restrict__ mbits,
-                              const unsigned long long *__restrict__ acc, float *__restrict__ grad_verts) {
-    pdl_wait();
-    const int b = blockIdx.y;
-    const int i = blockIdx.x * SP_THREADS + threadIdx.x;
-    if (i >= V) return;
-    const int e = det_exponent(mbits[b], 3LL * S + 1);
-    const size_t r = ((size_t)b * V + i) * 3;
-    for (int d = 0; d < 3; ++d) det_convert(grad_verts + r + d, acc + r + d, e);
 }
 
 // pytorch3d.ops.mesh_face_areas_normals drop-in (packed verts (V,3), int64 faces (F,3)): areas (F) and
@@ -422,12 +403,9 @@ extern "C" int ptk_sample_bwd(const float *grad_pts, const int32_t *face_idx, co
     return PTK_OK;
 }
 
-// det workspace: [M_b bits B, padded to 256 bytes][acc B*V*3 int64]
-static size_t sbd_mbits_bytes(int64_t B) { return (4 * (size_t)B + 255) & ~(size_t)255; }
-
 extern "C" size_t ptk_sample_bwd_det_workspace_bytes(int64_t B, int64_t V) {
     if (B <= 0 || V <= 0) return 0;
-    return sbd_mbits_bytes(B) + 24 * (size_t)B * (size_t)V;
+    return det_workspace_bytes(B, V);
 }
 
 extern "C" int ptk_sample_bwd_det(const float *grad_pts, const int32_t *face_idx, const float *uv, const int32_t *faces,
@@ -437,25 +415,22 @@ extern "C" int ptk_sample_bwd_det(const float *grad_pts, const int32_t *face_idx
     PTK_REQUIRE(grad_pts && face_idx && uv && faces && grad_verts, PTK_ERR_SHAPE, "sample_bwd_det: null pointer");
     PTK_REQUIRE(B > 0 && V > 0 && F > 0 && S > 0 && B <= 65535 && V < (1 << 28) && S < (1 << 28), PTK_ERR_SHAPE,
                 "sample_bwd_det: bad sizes");
-    const size_t need = ptk_sample_bwd_det_workspace_bytes(B, V);
-    PTK_REQUIRE(workspace && workspace_bytes >= need, PTK_ERR_WORKSPACE, "sample_bwd_det: workspace too small (%zu < %zu)",
-                workspace_bytes, need);
-    PTK_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, PTK_ERR_ALIGN,
-                "sample_bwd_det: workspace must be 16-byte aligned");
-    auto *mbits = reinterpret_cast<unsigned int *>(workspace);
-    auto *acc = reinterpret_cast<unsigned long long *>(reinterpret_cast<char *>(workspace) + sbd_mbits_bytes(B));
+    int rc = det_check_workspace(workspace, workspace_bytes, ptk_sample_bwd_det_workspace_bytes(B, V), "sample_bwd_det");
+    if (rc) return rc;
     cudaStream_t st = as_stream(stream);
+    DetWs w;
+    PTK_CHECK_CUDA(det_begin(workspace, B, V, st, w));
+    const DetBound nb = det_bound_const(3LL * S + 1);
     const float *uu = uv, *vv = uv + (size_t)B * S;
-    PTK_CHECK_CUDA(cudaMemsetAsync(mbits, 0, sizeof(unsigned int) * (size_t)B, st));
     launch_pdl(sample_bwd_det_terms_kernel, dim3((unsigned)ceil_div(S > V ? S : V, SP_THREADS), (unsigned)B), dim3(SP_THREADS),
-               0, st, grad_pts, uu, vv, (int)V, (int)S, grad_verts, acc, mbits);
+               0, st, grad_pts, uu, vv, (int)V, (int)S, grad_verts, w.acc_a, w.mbits);
     PTK_CHECK_LAUNCH();
     const int per_cta = 2048;
     launch_pdl(sample_bwd_det_reduce_kernel, dim3((unsigned)ceil_div(S, per_cta), (unsigned)B), dim3(SP_THREADS), 0, st,
-               grad_pts, face_idx, uu, vv, faces, (int)V, (int)S, per_cta, grad_verts, acc, (const unsigned int *)mbits);
+               grad_pts, face_idx, uu, vv, faces, (int)V, (int)S, per_cta, grad_verts, w.acc_a, (const unsigned int *)w.mbits,
+               nb);
     PTK_CHECK_LAUNCH();
-    launch_pdl(sample_bwd_det_convert_kernel, dim3((unsigned)ceil_div(V, SP_THREADS), (unsigned)B), dim3(SP_THREADS), 0, st,
-               (int)V, (int)S, (const unsigned int *)mbits, (const unsigned long long *)acc, grad_verts);
+    det_launch_convert<SP_THREADS>(w, nb, B, grad_verts, V, nullptr, 0, st);
     PTK_CHECK_LAUNCH();
     return PTK_OK;
 }

@@ -60,12 +60,16 @@ def test_det_workspace_sizes():
     # [M_b bits, padded to 256 B][24 B per x point][24 B per y point]
     assert L.ptk_chamfer_bwd_det_workspace_bytes(2, 100, 50) == 256 + 4864 + 2400
     assert L.ptk_sample_bwd_det_workspace_bytes(2, 10) == 256 + 480
+    assert L.ptk_sample_normals_bwd_det_workspace_bytes(2, 10) == 256 + 480
+    assert L.ptk_sample_normals_bwd_det_workspace_bytes(65, 3000) == 512 + 65 * 3000 * 24
     # the default workspace of the fused backward, then the two above (each padded to 256 B)
     assert L.ptk_mesh_chamfer_bwd_det_workspace_bytes(2, 10, 4, 100, 50) == \
         L.ptk_mesh_chamfer_workspace_bytes(2, 10, 4, 100, 50) + 256 + 4864 + 2560 + 768
     for shape in ((0, 10, 10), (1, 0, 10), (1, 10, 0), (-1, 10, 10)):
         assert L.ptk_chamfer_bwd_det_workspace_bytes(*shape) == 0
     assert L.ptk_sample_bwd_det_workspace_bytes(0, 10) == 0 and L.ptk_sample_bwd_det_workspace_bytes(3, 0) == 0
+    assert L.ptk_sample_normals_bwd_det_workspace_bytes(0, 10) == 0
+    assert L.ptk_sample_normals_bwd_det_workspace_bytes(3, 0) == 0
     for shape in ((0, 10, 4, 100, 50), (2, 0, 4, 100, 50), (2, 10, 0, 100, 50), (2, 10, 4, 0, 50), (2, 10, 4, 100, 0)):
         assert L.ptk_mesh_chamfer_bwd_det_workspace_bytes(*shape) == 0
 

@@ -53,6 +53,9 @@ def test_knn1_bwd_det_rejects_missing_or_small_workspace():
 def test_knn1_bwd_without_requested_gradients_is_a_no_op():
     assert _bwd(g1=None, g2=None) == 0
     assert _det(g1=None, g2=None, ws=None, nbytes=0) == 0
+    # the no-op comes before the batch-size check (which ptk_knn_bwd_* makes first)
+    assert _bwd(B=70000, g1=None, g2=None) == 0
+    assert _det(B=70000, g1=None, g2=None, ws=None, nbytes=0) == 0
 
 
 def test_knn1_bwd_det_workspace_sizes():

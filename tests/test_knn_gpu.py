@@ -206,7 +206,7 @@ def test_a_pair_alone_equals_the_pair_in_a_batch_of_256(K):
 
 # ------------------------------------------------------------------------------------- 4. backward
 def _terms(x, y, idx, g, l1, l2):
-    """(B,P1,K,3) terms 2 g (p1_i - p2_j) with knn1_term's fp32 operations, and the slot mask."""
+    """(B,P1,K,3) terms 2 g (p1_i - p2_j) with knn_term's fp32 operations, and the slot mask."""
     B, P1, K = idx.shape
     P2 = y.shape[1]
     l1 = torch.full((B,), P1, device="cuda") if l1 is None else l1.clamp(0, P1)
