@@ -24,7 +24,7 @@
 //   * a second small kernel unpacks the keys and does the fused mean reduction in a fixed order
 //     (deterministic, no float atomics).
 //   * default algorithm (PTK_CHAMFER_FILTER): the scan above is run on the 3-FFMA expansion
-//     |t|^2 - 2 q.t with packed FFMA2 instructions as a FILTER (chamfer_kernel2.cuh).  Its target tiles
+//     |t|^2 - 2 q.t with packed FFMA2 instructions as a FILTER (chamfer_scan.cuh).  Its target tiles
 //     are TMA-staged (cp.async.bulk + mbarrier, double buffered) from padded SoA arrays a small
 //     pre-pass writes (chamfer_prep_kernel).  The chunk the filter records is re-evaluated with the
 //     defining arithmetic, and the few queries whose runner-up chunk is within the proven error bound
@@ -36,13 +36,12 @@
 //     device-side lengths (pair_len(), NULL = full) and keeps the padded strides; the homogeneous calls pass NULL.
 #include <atomic>
 
-#include "chamfer_kernel2.cuh"
 #include "chamfer_pruned.cuh"
 #include "pair_bwd.cuh"
 
 namespace ptk {
 
-// library configuration of the kernel template (tuned with tools/chamfer_tune.cu)
+// library configuration of the scan templates
 constexpr int CH_THREADS = 128;
 constexpr int CH_CHUNK = 16;   // exact scan; filter scan on clouds the recheck cannot read with vector loads
 constexpr int CH_CHUNK_F = 64; // filter scan: one bookkeeping step per 64 targets (DESIGN.md K1)
@@ -331,20 +330,10 @@ static int launch_nn_pruned(const float *x, const float *y, const int64_t *lx, c
     PTK_CHECK_LAUNCH();
     u64 *keys_x = dir_only == 1 ? nullptr : w.keys_x;
     u64 *keys_y = dir_only == 0 ? nullptr : w.keys_y;
-    // One query per lane.  Two per lane (R = 2) halve the leaf loads per query -- the kernel is bound by the L1 return
-    // path -- but the wider query box costs as many extra scans and 72 registers: measured 891 vs 870 us at 256 x 10k,
-    // 422 vs 413 us at 16 x 50k.  Kept selectable for development (PTK_PR_R=2, read per call).
-    int R = 1;
-    if (getenv("PTK_PR_R")) R = atoi(getenv("PTK_PR_R")) == 2 ? 2 : 1;
-    dim3 qgrid((unsigned)ceil_div(Pq, (int64_t)PR_QUERY_WARPS * 32 * R), (unsigned)(B * ndir));
-    if (R == 2)
-        launch_pdl(chamfer_pruned_query_kernel<2>, qgrid, dim3(PR_QUERY_WARPS * 32), 0, st, (const float *)w.soa_x,
-                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, lx, ly, keys_x,
-                   keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
-    else
-        launch_pdl(chamfer_pruned_query_kernel<1>, qgrid, dim3(PR_QUERY_WARPS * 32), 0, st, (const float *)w.soa_x,
-                   (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, lx, ly, keys_x,
-                   keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
+    dim3 qgrid((unsigned)ceil_div(Pq, (int64_t)PR_QUERY_WARPS * 32), (unsigned)(B * ndir));
+    launch_pdl(chamfer_pruned_query_kernel, qgrid, dim3(PR_QUERY_WARPS * 32), 0, st, (const float *)w.soa_x,
+               (const float *)w.soa_y, (const PrBox *)w.box_x, (const PrBox *)w.box_y, (const int *)w.bad, iP1, iP2, lx, ly, keys_x,
+               keys_y, dir_only, w.rescue_x, w.rescue_y, w.count);
     PTK_CHECK_LAUNCH();
     const NNPlan p = plan_nn(B, Pq, Pt, ndir, CH_MINB, CH_CHUNK);
     dim3 rgrid((unsigned)ceil_div(Pq, (int64_t)CH_THREADS * 8), (unsigned)p.n_split, (unsigned)(B * ndir));

@@ -28,7 +28,7 @@
 // filter path does with its ambiguous queries.  The order of points inside a cell depends on the scheduling of
 // shared-memory atomics; results do not (a (distance, lowest original index) minimum is order-free).
 #pragma once
-#include "chamfer_kernel2.cuh"
+#include "chamfer_scan.cuh"
 
 namespace ptk {
 
@@ -627,10 +627,9 @@ __device__ __forceinline__ float pr_unord(unsigned k) {
     return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k);
 }
 
-// grid (ceil(max queries / (32 R x warps per CTA)), B * ndir), block = 128: a warp owns 32 R consecutive sorted queries,
-// R per lane (positions base + lane, base + 32 + lane, ...).  R = 1 is what runs; R = 2 halves the loads per (query, leaf)
-// pair -- the kernel is bound by the L1 return path, DESIGN.md K1b -- but its wider query box costs as much (chamfer.cu).
-template <int R>
+// grid (ceil(max queries / (32 x warps per CTA)), B * ndir), block = 128: a warp owns 32 consecutive sorted queries,
+// one per lane.  (Two per lane halve the loads per (query, leaf) pair -- the kernel is bound by the L1 return path --
+// but the wider query box costs as many extra scans: measured slower, DESIGN.md K1b.)
 __global__ void __launch_bounds__(PR_QUERY_WARPS * 32)
 chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__restrict__ soa_y,
                             const PrBox *__restrict__ box_x, const PrBox *__restrict__ box_y,
@@ -647,7 +646,7 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
     const int NQ = pair_len(dir == 0 ? len_x : len_y, b, dir == 0 ? P1 : P2);
     const int NT = pair_len(dir == 0 ? len_y : len_x, b, dir == 0 ? P2 : P1);
     const int lane = threadIdx.x & 31;
-    const int base = (blockIdx.x * PR_QUERY_WARPS + (threadIdx.x >> 5)) * 32 * R;  // first sorted position of the warp
+    const int base = (blockIdx.x * PR_QUERY_WARPS + (threadIdx.x >> 5)) * 32;  // first sorted position of the warp
     if (base >= NQ || NT == 0) return;  // whole warp (no target: chamfer_finalize_kernel writes the zero result)
     const int P1p = soa_padded(P1), P2p = soa_padded(P2);
     const int NQp = dir == 0 ? P1p : P2p;
@@ -661,43 +660,37 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
     int *__restrict__ list = dir == 0 ? rescue_x + (size_t)b * P1 : rescue_y + (size_t)b * P2;
     const float INF = __int_as_float(0x7f800000);
 
-    bool valid[R];  // positions NQ .. padded end hold +inf padding (inert); beyond the padded end: clamped, inert
-    float qx[R], qy[R], qz[R], best[R];
-    int qorig[R], barg[R];  // (best, barg): smallest distance so far and the lowest ORIGINAL index that attains it
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-        const int p = base + r * 32 + lane;
-        valid[r] = p < NQ;
-        const int pc = min(p, NQp - 1);
-        const float *qp = QS + (size_t)(pc >> 4) * 64 + (pc & 15);
-        qx[r] = qp[0], qy[r] = qp[16], qz[r] = qp[32];
-        qorig[r] = __float_as_int(qp[48]);
-        best[r] = valid[r] ? INF : -INF;
-        barg[r] = 0x7fffffff;
-    }
+    // positions NQ .. padded end hold +inf padding (inert); beyond the padded end: clamped, inert
+    const int p = base + lane;
+    const bool valid = p < NQ;
+    const int pc = min(p, NQp - 1);
+    const float *qp = QS + (size_t)(pc >> 4) * 64 + (pc & 15);
+    const float qx = qp[0], qy = qp[16], qz = qp[32];
+    const int qorig = __float_as_int(qp[48]);
+    float best = valid ? INF : -INF;  // (best, barg): smallest distance so far and the lowest ORIGINAL index attaining it
+    int barg = 0x7fffffff;
     bool rescue = (bad_flags[2 * b] | bad_flags[2 * b + 1]) != 0;  // non-finite input: everything takes the exact scan
     if (!rescue) {
         // the warp's query box
         unsigned olx = SENT, oly = SENT, olz = SENT, ohx = 0u, ohy = 0u, ohz = 0u;
-#pragma unroll
-        for (int r = 0; r < R; ++r)
-            if (valid[r]) {
-                olx = min(olx, pr_ord(qx[r])), oly = min(oly, pr_ord(qy[r])), olz = min(olz, pr_ord(qz[r]));
-                ohx = max(ohx, pr_ord(qx[r])), ohy = max(ohy, pr_ord(qy[r])), ohz = max(ohz, pr_ord(qz[r]));
-            }
+        if (valid) {
+            olx = pr_ord(qx), oly = pr_ord(qy), olz = pr_ord(qz);
+            ohx = pr_ord(qx), ohy = pr_ord(qy), ohz = pr_ord(qz);
+        }
         const float wlx = pr_unord(__reduce_min_sync(FULL, olx)), wly = pr_unord(__reduce_min_sync(FULL, oly));
         const float wlz = pr_unord(__reduce_min_sync(FULL, olz)), whx = pr_unord(__reduce_max_sync(FULL, ohx));
         const float why = pr_unord(__reduce_max_sync(FULL, ohy)), whz = pr_unord(__reduce_max_sync(FULL, ohz));
-        u64 qx2[R], qy2[R], qz2[R];
-#pragma unroll
-        for (int r = 0; r < R; ++r) qx2[r] = pack2(qx[r], qx[r]), qy2[r] = pack2(qy[r], qy[r]), qz2[r] = pack2(qz[r], qz[r]);
+        const u64 qx2 = pack2(qx, qx), qy2 = pack2(qy, qy), qz2 = pack2(qz, qz);
         unsigned wbest = 0x7f800000u;  // bit pattern of the largest `best` among the warp's live queries
         int scans = 0;
         const int scan_cap = max(64, pr_nb0(NT) >> 3);
         bool bail = false;
 
-        int st1 = 0, st2 = 0, st3 = 0, stA = 0, stB = 0, stL = 0;
-        (void)st1, (void)st2, (void)st3, (void)stA, (void)stB, (void)stL;
+        int st1 = 0, st2 = 0, st3 = 0;  // PTK_PR_STATS counters
+        (void)st1, (void)st2, (void)st3;
+#ifdef PTK_PR_STATS
+        int stA = 0, stB = 0, stL = 0;
+#endif
         unsigned k2 = SENT;
         if (lane < nb2) k2 = __float_as_uint(pr_lb(b2[lane].lo, b2[lane].hi, wlx, wly, wlz, whx, why, whz));
         while (!bail) {
@@ -727,10 +720,7 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
                     ++st3;
                     const int c = node1 * PR_FAN + l0;
                     const float4 blo = b0[c].lo, bhi = b0[c].hi;
-                    bool want = false;
-#pragma unroll
-                    for (int r = 0; r < R; ++r)
-                        want |= pr_lb(blo, bhi, qx[r], qy[r], qz[r], qx[r], qy[r], qz[r]) <= best[r];
+                    const bool want = pr_lb(blo, bhi, qx, qy, qz, qx, qy, qz) <= best;
 #ifdef PTK_PR_STATS
                     {
                         const unsigned wb = __ballot_sync(FULL, want);
@@ -746,60 +736,33 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
                     }
                     // scan the leaf: 16 targets, uniform addresses, the defining arithmetic on packed pairs
                     const float *__restrict__ cp = TS + (size_t)c * 64;
-                    float m[R], d[R][PR_CHUNK];
-#pragma unroll
-                    for (int r = 0; r < R; ++r) m[r] = INF;
+                    float m = INF, d[PR_CHUNK];
 #pragma unroll
                     for (int g = 0; g < PR_CHUNK / 4; ++g) {
                         const ulonglong2 tx = *reinterpret_cast<const ulonglong2 *>(cp + g * 4);
                         const ulonglong2 ty = *reinterpret_cast<const ulonglong2 *>(cp + 16 + g * 4);
                         const ulonglong2 tz = *reinterpret_cast<const ulonglong2 *>(cp + 32 + g * 4);
-#pragma unroll
-                        for (int r = 0; r < R; ++r) {
-                            const u64 dxa = sub2(qx2[r], tx.x), dxb = sub2(qx2[r], tx.y);
-                            const u64 dya = sub2(qy2[r], ty.x), dyb = sub2(qy2[r], ty.y);
-                            const u64 dza = sub2(qz2[r], tz.x), dzb = sub2(qz2[r], tz.y);
-                            u64 da = mul2(dxa, dxa), db = mul2(dxb, dxb);
-                            da = fma2(dya, dya, da);
-                            db = fma2(dyb, dyb, db);
-                            da = fma2(dza, dza, da);
-                            db = fma2(dzb, dzb, db);
-                            unpack2(da, d[r][4 * g], d[r][4 * g + 1]);
-                            unpack2(db, d[r][4 * g + 2], d[r][4 * g + 3]);
-                            m[r] = min3f(m[r], d[r][4 * g], d[r][4 * g + 1]);
-                            m[r] = min3f(m[r], d[r][4 * g + 2], d[r][4 * g + 3]);
-                        }
+                        sqdist4(qx2, qy2, qz2, tx, ty, tz, d[4 * g], d[4 * g + 1], d[4 * g + 2], d[4 * g + 3]);
+                        m = min3f(m, d[4 * g], d[4 * g + 1]);
+                        m = min3f(m, d[4 * g + 2], d[4 * g + 3]);
                     }
-                    bool touch = false;
-#pragma unroll
-                    for (int r = 0; r < R; ++r) touch |= m[r] <= best[r];
-                    if (__any_sync(FULL, touch)) {
+                    if (__any_sync(FULL, m <= best)) {
                         // some query improves or ties: lowest original index among this leaf's exact minima
-                        int a[R];
-#pragma unroll
-                        for (int r = 0; r < R; ++r) a[r] = 0x7fffffff;
+                        int a = 0x7fffffff;
 #pragma unroll
                         for (int g = 0; g < PR_CHUNK / 4; ++g) {
                             const int4 id = *reinterpret_cast<const int4 *>(cp + 48 + g * 4);
-#pragma unroll
-                            for (int r = 0; r < R; ++r) {
-                                a[r] = d[r][4 * g] == m[r] ? min(a[r], id.x) : a[r];
-                                a[r] = d[r][4 * g + 1] == m[r] ? min(a[r], id.y) : a[r];
-                                a[r] = d[r][4 * g + 2] == m[r] ? min(a[r], id.z) : a[r];
-                                a[r] = d[r][4 * g + 3] == m[r] ? min(a[r], id.w) : a[r];
-                            }
+                            a = min(a, d[4 * g] == m ? id.x : 0x7fffffff);
+                            a = min(a, d[4 * g + 1] == m ? id.y : 0x7fffffff);
+                            a = min(a, d[4 * g + 2] == m ? id.z : 0x7fffffff);
+                            a = min(a, d[4 * g + 3] == m ? id.w : 0x7fffffff);
                         }
-#pragma unroll
-                        for (int r = 0; r < R; ++r)
-                            if (m[r] < best[r] || (m[r] == best[r] && a[r] < barg[r])) {
-                                best[r] = m[r];
-                                barg[r] = a[r];
-                            }
+                        if (m < best || (m == best && a < barg)) {
+                            best = m;
+                            barg = a;
+                        }
                     }
-                    unsigned mine = 0u;
-#pragma unroll
-                    for (int r = 0; r < R; ++r) mine = max(mine, valid[r] ? __float_as_uint(best[r]) : 0u);
-                    wbest = __reduce_max_sync(FULL, mine);
+                    wbest = __reduce_max_sync(FULL, valid ? __float_as_uint(best) : 0u);
                 }
             }
         }
@@ -813,16 +776,13 @@ chamfer_pruned_query_kernel(const float *__restrict__ soa_x, const float *__rest
         PR_STAT(6, max(stA, stB));  // leaf scans if each 16-query half walked its own leaves
         PR_STAT(7, stL);            // (lane, leaf) pairs that wanted the scan
     }
-#pragma unroll
-    for (int r = 0; r < R; ++r) {
-        if (!valid[r]) continue;
-        if (rescue || !(best[r] < INF)) {
-            keys[qorig[r]] = ~0ull;  // the rescue scan merges with a 64-bit atomicMin
-            const unsigned int pos = atomicAdd(&rescue_count[2 * b + dir], 1u);
-            list[pos] = qorig[r];
-        } else {
-            keys[qorig[r]] = ((u64)__float_as_uint(best[r]) << 32) | (unsigned int)barg[r];
-        }
+    if (!valid) return;
+    if (rescue || !(best < INF)) {
+        keys[qorig] = ~0ull;  // the rescue scan merges with a 64-bit atomicMin
+        const unsigned int pos = atomicAdd(&rescue_count[2 * b + dir], 1u);
+        list[pos] = qorig;
+    } else {
+        keys[qorig] = ((u64)__float_as_uint(best) << 32) | (unsigned int)barg;
     }
 }
 

@@ -5,7 +5,6 @@
 // per query and drained per warp, target-range splits merged lexicographically for small batches.
 #include <algorithm>
 
-#include "chamfer_kernel.cuh"
 #include "nn_common.cuh"
 #include "det_accum.cuh"
 
@@ -117,29 +116,8 @@ knn_scan_kernel(const float *__restrict__ p1, const float *__restrict__ p2, cons
     for (int tile = t_begin; tile < t_end; tile += CH_TT) {
         const int n = min(CH_TT, t_end - tile);
         __syncthreads();
-        // global (n,3) packed floats -> shared SoA, padded to a whole chunk with +inf (never enters: d is +inf or NaN)
-        const int npad = ((n + KNN_CHUNK - 1) / KNN_CHUNK) * KNN_CHUNK;
-        const float *__restrict__ src = T + (size_t)tile * 3;
-        for (int e0 = 0; e0 < npad * 3; e0 += KNN_THREADS * 8) {
-            float v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int e = e0 + u * KNN_THREADS + tid;
-                v[u] = e < n * 3 ? src[e] : INF;
-            }
-#pragma unroll
-            for (int u = 0; u < 8; ++u) {
-                const int e = e0 + u * KNN_THREADS + tid;
-                if (e < npad * 3) {
-                    const int p = e / 3;
-                    const int c = e - p * 3;
-                    float *dst = c == 0 ? sx : (c == 1 ? sy : sz);
-                    dst[p] = v[u];
-                }
-            }
-        }
+        const int nchunks = stage_tile_soa<KNN_THREADS, KNN_CHUNK>(T + (size_t)tile * 3, n, sx, sy, sz);
         __syncthreads();
-        const int nchunks = npad / KNN_CHUNK;
         for (int ch = 0; ch < nchunks; ++ch) {
             float m[R];
 #pragma unroll
@@ -151,17 +129,8 @@ knn_scan_kernel(const float *__restrict__ p1, const float *__restrict__ p2, cons
                 const ulonglong2 tz = *reinterpret_cast<const ulonglong2 *>(&sz[ch * KNN_CHUNK + g * 4]);
 #pragma unroll
                 for (int r = 0; r < R; ++r) {
-                    const u64 dxa = sub2(qx[r], tx.x), dxb = sub2(qx[r], tx.y);
-                    const u64 dya = sub2(qy[r], ty.x), dyb = sub2(qy[r], ty.y);
-                    const u64 dza = sub2(qz[r], tz.x), dzb = sub2(qz[r], tz.y);
-                    u64 da = mul2(dxa, dxa), db = mul2(dxb, dxb);
-                    da = fma2(dya, dya, da);
-                    db = fma2(dyb, dyb, db);
-                    da = fma2(dza, dza, da);
-                    db = fma2(dzb, dzb, db);
                     float d0, d1, d2, d3;
-                    unpack2(da, d0, d1);
-                    unpack2(db, d2, d3);
+                    sqdist4(qx[r], qy[r], qz[r], tx, ty, tz, d0, d1, d2, d3);
                     m[r] = min3f(m[r], d0, d1);
                     m[r] = min3f(m[r], d2, d3);
                 }

@@ -88,7 +88,7 @@ def test_duplicate_points_and_grid_ties(oracle, algo):
 
 
 def _clouds(kind, rng, B, P1, P2):
-    """Adversarial inputs for the expansion filter (chamfer_kernel2.cuh)."""
+    """Adversarial inputs for the expansion filter (chamfer_scan.cuh)."""
     if kind == "far_from_origin":      # translation to the box centre must absorb the offset
         c = np.array([1000.0, -250.0, 40.0], np.float32)
         return (c + 0.01 * rng.standard_normal((B, P1, 3))).astype(np.float32), \
